@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (driver contract; torchrun for N > 1)
     python bench.py --impl reference ...                      (the reference's own CPU chain, same workload)
+    python bench.py ... --dump-outputs DIR                    (also writes the last timed step's audio and the RDS groups to DIR)
 
 Workload (BASELINE.json configs[3], the one the metric is quoted on; fits one GPU): a batch of 4096 independent
 synthetic 2.4 MS/s u8 IQ streams (stereo + RDS stations), full chain.  One step = one 65472-sample block of every
@@ -290,6 +291,35 @@ def c5_leg(torch, rfm, rank, world, local, barrier, max_over_ranks, steps=12, wa
     return out
 
 
+DUMP_BYTES = 64 << 20
+NPY_HEADER = 128   # bytes of an .npy header for arrays of up to two dimensions
+
+
+def dump_outputs(out_dir, audio, groups, first_stream, rank, world):
+    """What the device-resident path delivered by the end of the timed steps, as float32 / float64 .npy files:
+      audio.npy             [streams, floats] float32, the audio of the last timed block (interleaved L, R);
+      rds_groups.npy        [groups, 4] float64, the RDS groups decoded so far (rfm_decoder_rds_take_groups), the
+                            streams' one after another;
+      rds_group_counts.npy  [streams] float64, how many of them belong to each stream;
+      stream_ids.npy        [streams] float64, the global stream id of each row (first_stream + index in the batch).
+    With several GPUs each rank writes <name>_rank<r>.npy.  Where the batch exceeds the rank's share of DUMP_BYTES, a
+    fixed seeded sample of its streams is written."""
+    sfx = "" if world == 1 else f"_rank{rank}"
+    os.makedirs(out_dir, exist_ok=True)
+    n = audio.shape[0]
+    budget = DUMP_BYTES // world - 4 * NPY_HEADER - sum(g.shape[0] for g in groups) * 4 * 8
+    rows = max(0, budget) // (audio[0].nbytes + 16)
+    idx = np.arange(n)
+    if rows < n:
+        idx = np.sort(np.random.default_rng(0).choice(n, rows, replace=False))
+    picked = [np.asarray(groups[i], dtype=np.float64).reshape(-1, 4) for i in idx]
+    out = {"audio": audio[idx], "rds_groups": np.concatenate(picked) if picked else np.zeros((0, 4)),
+           "rds_group_counts": np.array([g.shape[0] for g in picked], dtype=np.float64),
+           "stream_ids": (first_stream + idx).astype(np.float64)}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}{sfx}.npy"), a)
+
+
 # --------------------------------------------------------------------------------------------------------------
 def run_b200(args):
     import torch
@@ -368,6 +398,10 @@ def run_b200(args):
     t1 = time.perf_counter()
     clk = clocks.stop(t0, t1)
     launches = rfm.launch_count() - launches0
+    if args.dump_outputs:
+        # pass 2 below rewrites the same audio buffer: take the metric pass's last block now
+        dump_outputs(args.dump_outputs, audio[:, :nfl].cpu().numpy(), [dec.take_groups(s) for s in range(S)], rank * S,
+                     rank, world)
     # pass 2 (the roofline leg): the same K steps again with every kernel launch bracketed by CUDA events on the
     # stream it is launched on; ~50 extra event records per step cost 3-4 %, which is why it is not the metric pass
     prof, ms_prof = {}, None
@@ -617,7 +651,12 @@ def main():
     ap.add_argument("--lanes-sms", type=int, default=0, help="rfm_config::lanes_sms (0 = automatic, 1 = no SM partition)")
     ap.add_argument("--fir-fused", type=int, default=0, help="rfm_config::fir_fused for the main legs (1 = tolerance mode; the "
                                                              "headline is the default 0)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the audio of the last timed step and the RDS groups "
+                                                          "decoded by then as DIR/*.npy (at most 64 MB; see dump_outputs), "
+                                                          "to compare two builds output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -5,6 +5,9 @@ from __future__ import annotations
 import json
 import os
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -45,3 +48,66 @@ def test_reference_arm_line():
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert d["cpu_baseline"]["value"] == d["value"] and d["cpu_baseline"]["kind"] == "reference"
     assert d["gpu_launches"] == 0
+
+
+def test_dump_outputs_fits_the_budget(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: the whole batch where it fits, else the same seeded sample of streams on every run,
+    within the rank's share of the byte budget, .npy headers included; rows carry their global stream ids."""
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 20)
+    rng = np.random.default_rng(0)
+    a = rng.standard_normal((64, 1000)).astype(np.float32)
+    ga = [rng.integers(0, 65536, (k % 3, 4)).astype(np.uint16) for k in range(64)]
+    bench.dump_outputs(str(tmp_path / "a"), a, ga, 0, 0, 1)
+    assert sorted(os.listdir(tmp_path / "a")) == ["audio.npy", "rds_group_counts.npy", "rds_groups.npy", "stream_ids.npy"]
+    assert np.array_equal(np.load(tmp_path / "a" / "audio.npy"), a)
+    assert np.array_equal(np.load(tmp_path / "a" / "rds_groups.npy"), np.concatenate(ga).astype(np.float64))
+    assert np.array_equal(np.load(tmp_path / "a" / "rds_group_counts.npy"), [len(g) for g in ga])
+    assert np.array_equal(np.load(tmp_path / "a" / "stream_ids.npy"), np.arange(64))
+    # the largest audio that fills one rank's share (1 MB / 2) to the byte once the headers are counted
+    share = (1 << 20) // 2
+    rows = 300
+    width = ((share - 4 * bench.NPY_HEADER) // rows - 16) // 4
+    b = rng.standard_normal((1024, width)).astype(np.float32)
+    gb = [np.zeros((0, 4), np.uint16)] * 1024
+    for d in ("b1", "b2"):
+        bench.dump_outputs(str(tmp_path / d), b, gb, 1024, 1, 2)
+    files = sorted(os.listdir(tmp_path / "b1"))
+    assert files == ["audio_rank1.npy", "rds_group_counts_rank1.npy", "rds_groups_rank1.npy", "stream_ids_rank1.npy"]
+    assert sum(os.path.getsize(tmp_path / "b1" / f) for f in files) <= share
+    ids, got = np.load(tmp_path / "b1" / "stream_ids_rank1.npy"), np.load(tmp_path / "b1" / "audio_rank1.npy")
+    assert ids.dtype == np.float64 and got.dtype == np.float32 and ids.size == rows
+    assert np.all(np.diff(ids) > 0) and ids.min() >= 1024 and ids.max() < 2048
+    assert np.array_equal(got, b[ids.astype(np.int64) - 1024])
+    for f in files:
+        assert np.array_equal(np.load(tmp_path / "b1" / f), np.load(tmp_path / "b2" / f))
+
+
+@pytest.mark.gpu
+def test_dump_outputs_is_the_last_timed_block(tmp_path, rfm):
+    """bench.py --dump-outputs end to end: the dumped audio is what the decoder returns for the last timed block of the
+    seeded batch (after the warm-up and the timed blocks before it), the groups what it decoded by then."""
+    import importlib
+    import subprocess
+    import sys
+    import torch
+    import bench
+    S, K, W = 8, 8, 3
+    out = tmp_path / "d"
+    subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(K), "--warmup", str(W), "--streams",
+                    str(S), "--no-extras", "--no-cpu", "--no-e2e", "--no-prof", "--dump-outputs", str(out)],
+                   check=True, cwd=str(tmp_path), capture_output=True)
+    synth_device = importlib.import_module("radiofm_b200.synth_device")
+    nres = min(K + W, 12)   # bench.py --resident-blocks default
+    iq = synth_device.make_batch_u8(torch, S, bench.FS, nres * bench.BLK, torch.device("cuda", 0)).cpu().numpy()
+    d = rfm.FmDecoderBatch(bench.FS, -0.15 * bench.FS, downsample=bench.DS, n_streams=S, max_block_len=bench.BLK, device=0)
+    for i in range(W + K):
+        b = i % nres
+        a = d.process_u8(iq[:, b * bench.BLK:(b + 1) * bench.BLK])
+    got = np.load(out / "audio.npy")
+    assert got.dtype == np.float32 and got.shape == a.shape and np.array_equal(got.view(np.uint32), a.view(np.uint32))
+    groups = [d.take_groups(s) for s in range(S)]
+    assert sum(len(g) for g in groups) > 0
+    assert np.array_equal(np.load(out / "rds_group_counts.npy"), [len(g) for g in groups])
+    assert np.array_equal(np.load(out / "rds_groups.npy"), np.concatenate(groups).astype(np.float64))
+    assert np.array_equal(np.load(out / "stream_ids.npy"), np.arange(S))

@@ -12,6 +12,7 @@ box the unmodified reference is checked as well.
 """
 import hashlib
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -20,6 +21,7 @@ from conftest import RATES, ROOT, bits_equal, station
 
 pytestmark = pytest.mark.gpu
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+sys.path.insert(0, GOLDEN)
 GPU_TAPS = ["demod_in", "baseband", "rawstereo", "mono_rs", "stereo_rs", "lp_stereo", "lp_mono", "rds_dec",
             "rds_lp", "rds_pll", "rds_mf"]
 
@@ -87,6 +89,19 @@ def test_against_unmodified_reference(rfm, ref):
         tolerances(a_d, a_r)
         assert bits_equal(a_d, a_r)
     assert np.array_equal(r.take_bits(), d.take_bits()) and np.array_equal(r.take_groups(), d.take_groups())
+
+
+def test_against_unmodified_reference_golden(rfm):
+    """test_against_unmodified_reference's 11 blocks against the audio digests, bits and groups stored for them in
+    tests/golden/ref_cases.npz (tests/golden/make_golden_ref_cases.py, checked against the original where it is built)."""
+    from make_golden_ref_cases import sha
+    g = np.load(os.path.join(GOLDEN, "ref_cases.npz"))
+    fs, ds, blk = RATES["1.2M"]
+    iq, _ = station("1.2M", 11)
+    d = rfm.FmDecoderBatch(fs, -0.15 * fs, downsample=ds, max_block_len=blk)
+    for b in range(11):
+        assert sha(d.process_u8(iq[None, b * blk:(b + 1) * blk])[0]) == g["ref12_sha"][b], b
+    assert np.array_equal(d.take_bits(), g["ref12_bits"]) and np.array_equal(d.take_groups(), g["ref12_groups"])
 
 
 @pytest.mark.parametrize("rate", ["1.0M", "1.2M", "2.4M", "390k"])
@@ -300,34 +315,42 @@ def test_ragged_block_lengths_and_edges(rfm, port):
     assert rc == -5  # RFM_ERR_OVERFLOW
 
 
-def test_default_rtlsdr_block_at_1200k_and_odd_short_blocks(rfm, port, ref):
+def test_default_rtlsdr_block_at_1200k_and_odd_short_blocks(rfm, port):
     """Any block length yields audio, and the RDS branch follows the reference through the counts its half-band
     stages were not written for (DownConvert.cpp:498-550).  cRtlSdrSource's default block of 65536 samples at
     1.2 MS/s / 5 leaves 13107 or 13108 baseband samples: odd counts make (m + 1) / 2 outputs per stage and restart the
     decimation phase every block; blocks so short that a stage gets fewer samples than taps pass through unfiltered.
-    Checked against the UNMODIFIED reference where oracle/_ref travelled (and always against the oracle port)."""
+    Checked against the UNMODIFIED reference where oracle/_ref was built, and always against the oracle port and the
+    per-block audio digests, bits and groups stored for these sizes in tests/golden/ref_cases.npz."""
+    from make_golden_ref_cases import ODD_SIZES, sha
+    from oracle import ref
+    g = np.load(os.path.join(GOLDEN, "ref_cases.npz"))
     fs, ds = 1.2e6, 5
     blk = 65536
     iq, _ = station("1.2M", 12)
     d = rfm.FmDecoderBatch(fs, -0.15 * fs, downsample=ds, n_streams=2, max_block_len=blk)
     o = port.OracleFmDecoder(fs, -0.15 * fs, downsample=ds)
-    r = ref.RefFmDecoder(fs, -0.15 * fs, downsample=ds)
+    r = ref.RefFmDecoder(fs, -0.15 * fs, downsample=ds) if ref.available() else None
     pos = 0
     sizes = [blk] * 9 + [100, 333, 1000, 47, 4096, 65521, 777, 20000, 41, 65535, 4097]
-    for n in sizes:
+    assert sizes == ODD_SIZES
+    for i, n in enumerate(sizes):
         x = iq[pos:pos + n]
         pos += n
         a = d.process_u8(np.stack([x, x]))
         a_o = o.process_u8(x)
-        a_r, _ = r.process_staged(ref.u8_to_cf32(x), want=())
-        assert bits_equal(a_o, a_r), n
+        assert sha(a_o) == g["odd_sha"][i], n
+        if r is not None:
+            a_r, _ = r.process_staged(ref.u8_to_cf32(x), want=())
+            assert bits_equal(a_o, a_r), n
         assert bits_equal(a[0], a_o) and bits_equal(a[1], a_o), n
         assert bits_equal(d.tap("rds_dec"), o.tap("rds_dec")) and bits_equal(d.tap("rds_mf"), o.tap("rds_mf")), n
     bo = o.take_bits()
-    assert bo.size > 700 and np.array_equal(bo, r.take_bits())
+    assert bo.size > 700 and np.array_equal(bo, g["odd_bits"]) and (r is None or np.array_equal(bo, r.take_bits()))
     assert np.array_equal(d.take_bits(0), bo) and np.array_equal(d.take_bits(1), bo)
     go = o.take_groups()
-    assert len(go) >= 5 and np.array_equal(go, r.take_groups()) and np.array_equal(d.take_groups(1), go)
+    assert len(go) >= 5 and np.array_equal(go, g["odd_groups"]) and (r is None or np.array_equal(go, r.take_groups()))
+    assert np.array_equal(d.take_groups(1), go)
 
 
 @pytest.mark.parametrize("rate,n", [("2.4M", 65536), ("2.4M", 20000), ("1.2M", 4096), ("390k", 16004)])

@@ -6,8 +6,10 @@
 The reference ships no tests or golden vectors (SURVEY.md section 4).  CPU only.
 """
 import ctypes as C
+import functools
 import hashlib
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -280,3 +282,59 @@ def test_rdsdc_port_vs_ref_every_stage_kind(port, ref, in_rate, max_bw, wfm, fre
         assert kp == kr and bits_equal(yp[:kp], yr[:kr])
     LP.rfo_rdsdc_destroy(hp)
     LR.ref_rdsdc_destroy(hr)
+
+
+# ---------------------------------------------------------------------------------------------------
+# (3) the cases of (1) against tests/golden/ref_cases.npz (tests/golden/make_golden_ref_cases.py): the same
+#     comparisons where the original is not built
+# ---------------------------------------------------------------------------------------------------
+GOLD_REF = np.load(os.path.join(GOLDEN, "ref_cases.npz"))
+
+
+@functools.lru_cache(maxsize=None)
+def ref_cases(use_ref: bool) -> dict:
+    sys.path.insert(0, GOLDEN)
+    import make_golden_ref_cases as mr
+    return mr.make(use_ref)
+
+
+def same_as_golden(prefix: str):
+    got = ref_cases(False)
+    keys = [k for k in GOLD_REF.files if k.startswith(prefix)]
+    assert keys
+    for k in keys:
+        assert np.array_equal(got[k], GOLD_REF[k]), k
+
+
+@pytest.mark.parametrize("rate", ["1.0M", "1.2M", "2.4M", "390k"])
+def test_port_matches_golden_every_stage(port, rate):
+    same_as_golden(f"stage_{rate}_")
+
+
+def test_port_reset_matches_golden(port):
+    same_as_golden("reset_")
+
+
+def test_port_noisy_and_mono_match_golden(port):
+    same_as_golden("noisy_")
+
+
+@pytest.mark.parametrize("j", range(4))
+def test_rdsdc_port_matches_golden_every_stage_kind(port, j):
+    same_as_golden(f"rdsdc{j}_")
+
+
+def test_demux_port_packets_match_golden(port):
+    """the restatement of cRadioReceiver::DemuxRead against the add-on's packets (test_ref_addon.py)"""
+    same_as_golden("demux_")
+
+
+def test_ref_cases_golden_is_what_the_reference_produces(port):
+    sys.path.insert(0, GOLDEN)
+    import make_golden_ref_cases as mr
+    if not mr.reference_available():
+        pytest.skip("oracle/_ref/ not built (see oracle/Makefile)")
+    got = ref_cases(True)
+    for k in GOLD_REF.files:
+        if k != "source":
+            assert np.array_equal(got[k], GOLD_REF[k]), k

@@ -171,6 +171,22 @@ def test_against_compiled_reference_random_streams():
         assert frames == want and nm == wn
 
 
+def test_random_streams_match_golden():
+    """the streams of test_against_compiled_reference_random_streams through the port and the product, against the
+    frames and names stored for them in tests/golden/ref_cases.npz (checked against the original where it is built)"""
+    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+    import make_golden_uecp as mg
+    import make_golden_ref_cases as mr
+    want = np.load(os.path.join(ROOT, "tests", "golden", "ref_cases.npz"))["uecp_sha"]
+    for k, seed in enumerate((1, 2, 3)):
+        rng = np.random.default_rng(seed)
+        g = np.concatenate([mg.fuzz(rng, 3000), mg.scripted(rng), mg.fuzz(rng, 3000)])
+        o = uecp_port.OracleGroupDecoder()
+        assert mr.frames_sha(o.decode(g), o.names) == want[k]
+        _, frames, nm = product_frames(g)
+        assert mr.frames_sha(frames, nm) == want[k]
+
+
 @pytest.mark.skipif(not ref_uecp.available(), reason="compiled reference group decoder not present (oracle/_ref)")
 def test_golden_is_what_the_reference_produces():
     for case in ("scripted", "fuzz"):
