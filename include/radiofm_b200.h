@@ -463,6 +463,57 @@ RFM_API const char* rfm_rtlsdr_error(const rfm_rtlsdr* s);    /* error() */
 /* GetSignalStatus(float&, float&, bool&), RadioReceiver.cpp:544-556: levels in dB */
 RFM_API int rfm_demux_signal_status(rfm_demux* m, float* interface_level_db, float* audio_level_db, int* stereo);
 
+/* ------------------------------------------------------------------------------------------------
+ * Band scan of one wideband capture: the add-on's tuner auto-scan (ChannelSettings.cpp:96-147: retune one frequency,
+ * wait, check cFmDecoder::StereoDetected) generalised to every channel of a capture in one pass.
+ *   spectrum   Welch average over N = 4096 periodic-Hann segments, hop N/2, of x = float(u / 127.5 - 1)
+ *              (RTL_SDR_Source.cpp:207-211): P[k] = sum_s |X_s[k]|^2 / (S N sum w^2), so sum_k P is the mean power of
+ *              the windowed signal (a complex tone of modulus 1 is 0 dBFS).  Centred: index k <-> (k - N/2) Fs / N Hz.
+ *              Independent of the device, its SM count and any SM partition (fixed work split, no atomics).
+ *   channels   raster point f_j = raster_first + j raster_step owns the bins with f_j - step/2 <= f < f_j + step/2;
+ *              C_j = sum of its bins' P in double, in bin order.  floor = the sorted C at index (count - 1) / 4.
+ *   candidate  C_j >= floor * 10^(min_snr_db / 10), C_j > C_{j-1} (when j-1 exists), C_j >= C_{j+1} (when j+1 exists).
+ *   stations   every candidate confirmed with the reference's receiver over every whole call of the capture: rows of
+ *              rfm_downconvert (CRDSDownConvert::SetFrequency(-f_j) + SetWfmDataRate(Fs, 100 kHz)) into one
+ *              rfm_decoder (cFmDecoder(rate, 0, 48000, 15000, 1)); one call = 16000 baseband samples
+ *              (16000 << stages capture samples).  PS is what cRDSGroupDecoder hands to SetChannelName for the groups.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct rfm_scan rfm_scan;
+typedef struct rfm_scan_config
+{
+  double sample_rate;                 /* capture rate, Hz */
+  double raster_first, raster_step;   /* Hz from the capture centre; step >= 4 Fs / 4096 */
+  uint32_t raster_count;              /* 1 .. 4096; every |f_j| + 100 kHz <= Fs / 2 */
+  double min_snr_db;                  /* default 10 */
+  int32_t device;                     /* -1 = current */
+} rfm_scan_config;
+typedef struct rfm_scan_station
+{
+  double freq;                        /* raster frequency, Hz from the capture centre */
+  float power_dbfs, snr_db;           /* 10 log10 C_j, 10 log10 (C_j / floor) */
+  int32_t stereo_detected;            /* rfm_stream_status after the last call */
+  float pilot_level, interface_level, baseband_level;
+  uint32_t rds_groups;                /* groups delivered by the block synchroniser */
+  int32_t pi;                         /* most frequent block A, ties to the first seen; -1: no group */
+  char ps[9];                         /* "" if no name was published */
+} rfm_scan_station;
+/* Defaults: 2.4 MS/s (the add-on's RTL-SDR rate), 100 kHz raster over +-1.1 MHz, 10 dB, current device. */
+RFM_API void rfm_scan_config_default(rfm_scan_config* cfg);
+/* Validates the raster (RFM_ERR_INVALID: step < 4 Fs / N, count outside 1 .. N, a channel with |f_j| + 100 kHz > Fs/2,
+ * a rate whose WFM decimation chain has no stage) before touching a device. */
+RFM_API int rfm_scan_create(const rfm_scan_config* cfg, rfm_scan** out);
+RFM_API void rfm_scan_destroy(rfm_scan* s);
+/* Whole capture [n][2] u8 in host memory (copied with cudaMemcpyAsync) or device memory (complete before the call,
+ * 2-byte aligned); n >= one call (RFM_ERR_INVALID otherwise).  Blocking.  Zero candidates: no receiver is created and
+ * the scan has 0 stations. */
+RFM_API int rfm_scan_run_u8(rfm_scan* s, const uint8_t* iq, uint64_t n, int iq_on_device);
+RFM_API int rfm_scan_spectrum(rfm_scan* s, float* psd, uint32_t max, uint32_t* n_bins);   /* N floats, centred */
+RFM_API int rfm_scan_channel_power(rfm_scan* s, double* out, uint32_t max);              /* C_j, linear */
+RFM_API int rfm_scan_stations(rfm_scan* s, rfm_scan_station* out, uint32_t max, uint32_t* n);
+/* Device time of the last run's two stages (CUDA events): the spectrum kernels, and the confirmation from the first
+ * front-end launch to the end of the last demodulator call (0 without candidates). */
+RFM_API int rfm_scan_timing(rfm_scan* s, double* spectrum_ms, double* confirm_ms);
+
 #ifdef __cplusplus
 }
 #endif

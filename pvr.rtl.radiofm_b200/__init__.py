@@ -72,12 +72,27 @@ EXPORTED_SYMBOLS = (
     "rfm_downsample_process_complex_device", "rfm_downsample_process_real_device",
     "rfm_rdsproc_create", "rfm_rdsproc_destroy", "rfm_rdsproc_process_rate", "rfm_rdsproc_reset", "rfm_rdsproc_process",
     "rfm_rdsproc_process_device", "rfm_rdsproc_take_bits", "rfm_rdsproc_take_groups",
+    "rfm_scan_config_default", "rfm_scan_create", "rfm_scan_destroy", "rfm_scan_run_u8", "rfm_scan_spectrum",
+    "rfm_scan_channel_power", "rfm_scan_stations", "rfm_scan_timing",
 )
 
 
 _ADD_FRAME_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.POINTER(C.c_uint8), C.c_uint32)
 _SET_NAME_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_char_p)
 _SETTING_CB = C.CFUNCTYPE(C.c_int, C.c_void_p)
+
+
+class ScanConfig(C.Structure):
+    """rfm_scan_config (include/radiofm_b200.h)."""
+    _fields_ = [("sample_rate", C.c_double), ("raster_first", C.c_double), ("raster_step", C.c_double),
+                ("raster_count", C.c_uint32), ("min_snr_db", C.c_double), ("device", C.c_int32)]
+
+
+class ScanStation(C.Structure):
+    """rfm_scan_station (include/radiofm_b200.h)."""
+    _fields_ = [("freq", C.c_double), ("power_dbfs", C.c_float), ("snr_db", C.c_float),
+                ("stereo_detected", C.c_int32), ("pilot_level", C.c_float), ("interface_level", C.c_float),
+                ("baseband_level", C.c_float), ("rds_groups", C.c_uint32), ("pi", C.c_int32), ("ps", C.c_char * 9)]
 
 
 class RdsGroupCallbacks(C.Structure):
@@ -244,6 +259,16 @@ def lib():
         L.rfm_rdsproc_process_device.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint32, C.c_void_p]
         L.rfm_rdsproc_take_bits.argtypes = [C.c_void_p, C.c_uint32, _u8p, C.c_uint32, _u32p]
         L.rfm_rdsproc_take_groups.argtypes = [C.c_void_p, C.c_uint32, _u16p, C.c_uint32, _u32p]
+        L.rfm_scan_config_default.restype = None
+        L.rfm_scan_config_default.argtypes = [C.POINTER(ScanConfig)]
+        L.rfm_scan_create.argtypes = [C.POINTER(ScanConfig), C.POINTER(C.c_void_p)]
+        L.rfm_scan_destroy.restype = None
+        L.rfm_scan_destroy.argtypes = [C.c_void_p]
+        L.rfm_scan_run_u8.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int]
+        L.rfm_scan_spectrum.argtypes = [C.c_void_p, _f32p, C.c_uint32, _u32p]
+        L.rfm_scan_channel_power.argtypes = [C.c_void_p, _f64p, C.c_uint32]
+        L.rfm_scan_stations.argtypes = [C.c_void_p, C.POINTER(ScanStation), C.c_uint32, _u32p]
+        L.rfm_scan_timing.argtypes = [C.c_void_p, _f64p, _f64p]
         L.rfm_rds_check_block.restype = C.c_uint32
         L.rfm_rds_check_block.argtypes = [C.c_uint32, C.c_uint32, C.c_int, _u32p]
         _lib = L
@@ -900,6 +925,77 @@ class RdsProcessorBatch:
         k = C.c_uint32(0)
         _check(lib().rfm_rdsproc_take_groups(self._h, row, _p(out, _u16p), max_groups, C.byref(k)))
         return out[:k.value].copy()
+
+
+SCAN_BINS = 4096
+
+
+def scan_config(fs: float, raster_first: float, raster_step: float, raster_count: int, min_snr_db: float = 10.0,
+                device: int = -1) -> ScanConfig:
+    cfg = ScanConfig()
+    lib().rfm_scan_config_default(C.byref(cfg))
+    cfg.sample_rate, cfg.raster_first, cfg.raster_step = fs, raster_first, raster_step
+    cfg.raster_count, cfg.min_snr_db, cfg.device = raster_count, min_snr_db, device
+    return cfg
+
+
+class BandScan:
+    """Band scan of one wideband u8 capture (rfm_scan_*): averaged spectrum, channel powers on a raster (Hz from the
+    capture centre), candidates, and every candidate confirmed with the reference's receiver -- the add-on's tuner
+    auto-scan (ChannelSettings.cpp:96-147) for all channels at once."""
+
+    def __init__(self, fs: float, raster_first: float, raster_step: float, raster_count: int, min_snr_db: float = 10.0,
+                 device: int = -1):
+        cfg = scan_config(fs, raster_first, raster_step, raster_count, min_snr_db, device)
+        self.raster_count = raster_count
+        self._h = C.c_void_p()
+        _check(lib().rfm_scan_create(C.byref(cfg), C.byref(self._h)))
+
+    def close(self):
+        if getattr(self, "_h", None):
+            lib().rfm_scan_destroy(self._h)
+            self._h = None
+
+    __del__ = _quiet_del(close)
+
+    def run_u8(self, capture_u8: np.ndarray):
+        """Host capture [n, 2] uint8."""
+        cap = np.ascontiguousarray(capture_u8, dtype=np.uint8).reshape(-1, 2)
+        _check(lib().rfm_scan_run_u8(self._h, cap.ctypes.data_as(C.c_void_p), cap.shape[0], 0))
+
+    def run_device(self, d_capture_ptr: int, n: int):
+        """Device capture [n, 2] uint8 at d_capture_ptr, complete before the call (e.g. after torch.cuda.synchronize())."""
+        _check(lib().rfm_scan_run_u8(self._h, C.c_void_p(d_capture_ptr), n, 1))
+
+    def spectrum(self) -> np.ndarray:
+        out = np.zeros(SCAN_BINS, dtype=np.float32)
+        k = C.c_uint32(0)
+        _check(lib().rfm_scan_spectrum(self._h, _p(out, _f32p), out.size, C.byref(k)))
+        return out[:k.value]
+
+    def channel_power(self) -> np.ndarray:
+        out = np.zeros(self.raster_count, dtype=np.float64)
+        _check(lib().rfm_scan_channel_power(self._h, _p(out, _f64p), out.size))
+        return out
+
+    def stations(self) -> list[dict]:
+        n = C.c_uint32(0)
+        buf = (ScanStation * self.raster_count)()          # at most one station per channel
+        _check(lib().rfm_scan_stations(self._h, buf, len(buf), C.byref(n)))
+        return [scan_station_dict(buf[i]) for i in range(n.value)]
+
+    def timing(self) -> tuple[float, float]:
+        """(spectrum, confirmation) device milliseconds of the last run."""
+        a, b = C.c_double(0), C.c_double(0)
+        _check(lib().rfm_scan_timing(self._h, C.byref(a), C.byref(b)))
+        return a.value, b.value
+
+
+def scan_station_dict(st: ScanStation) -> dict:
+    return {"freq": st.freq, "power_dbfs": np.float32(st.power_dbfs), "snr_db": np.float32(st.snr_db),
+            "stereo": bool(st.stereo_detected), "pilot_level": np.float32(st.pilot_level),
+            "if_level": np.float32(st.interface_level), "bb_level": np.float32(st.baseband_level),
+            "rds_groups": int(st.rds_groups), "pi": int(st.pi), "ps": st.ps.decode("latin-1")}
 
 
 def math_probe(op: int, a: np.ndarray, b: np.ndarray | None = None) -> np.ndarray:
