@@ -7,7 +7,9 @@
  * (paths relative to the reference's src/).  Plain pointers and sizes only.
  *
  * Conventions
- *   - IQ in : interleaved I,Q.  u8 offset-binary (RTL-SDR, 127.5 == 0) or float32 complex.
+ *   - IQ in : interleaved I,Q, little-endian, in one of the rfm_iq_format formats below.  The _u8 / _cf32 entry points
+ *             are the reference's two (u8 offset-binary from the RTL-SDR, 127.5 == 0; float32 complex); the _iq entry
+ *             points take the format as an argument.
  *   - audio : interleaved float32 L,R at sample_rate_pcm.
  *   - Batched: a decoder handle owns n_streams independent streams that are always processed with
  *     the same block length (row-major [stream][sample]).  n_streams == 1 reproduces one cFmDecoder.
@@ -37,6 +39,18 @@ typedef enum rfm_status
   RFM_ERR_NO_DEVICE = -4,   /* no sm_100 device / extension unusable */
   RFM_ERR_OVERFLOW = -5     /* caller buffer too small */
 } rfm_status;
+
+/* IQ sample formats (interleaved I,Q, little-endian):
+ *   RFM_IQ_U8    RTL-SDR offset binary, float(u / 127.5 - 1) (RTL_SDR_Source.cpp:207-211)
+ *   RFM_IQ_S8    cs8 (HackRF), (float)v * 2^-7
+ *   RFM_IQ_S16   cs16 (USRP, bladeRF, LimeSDR, Airspy, SDRplay: the SoapySDR / UHD host format), (float)v * 2^-15
+ *   RFM_IQ_CF32  float32 complex, taken as is
+ * The s8 / s16 conversions are exact in float32: an s8 / s16 input gives bit for bit what the cf32 path gives for the
+ * converted samples.  Full scale is the container's: a stream that uses fewer bits (bladeRF SC16_Q11: 12 bits in 16)
+ * reads 2^(16-12) = 24 dB low; levels and the scan's dBFS values are relative to the container. */
+typedef enum rfm_iq_format { RFM_IQ_U8 = 0, RFM_IQ_S8 = 1, RFM_IQ_S16 = 2, RFM_IQ_CF32 = 3 } rfm_iq_format;
+/* bytes per complex sample: 2, 2, 4, 8; 0 for an unknown format */
+RFM_API uint32_t rfm_iq_format_bytes(int format);
 
 RFM_API const char* rfm_last_error(void);
 RFM_API const char* rfm_version(void);
@@ -121,6 +135,16 @@ RFM_API int rfm_decoder_process_u8_device(rfm_decoder* d, const uint8_t* d_iq, s
 RFM_API int rfm_decoder_process_cf32_device(rfm_decoder* d, const float* d_iq, size_t iq_stride, uint32_t n,
                                             float* d_audio, size_t audio_stride, uint32_t* n_audio_floats,
                                             void* cuda_stream);
+/* The three calls above for any rfm_iq_format: iq is [n_streams][n] samples of `format` (iq_stride in samples).  An
+ * unknown format returns RFM_ERR_INVALID; so does a device pointer that is not aligned to the sample size
+ * (rfm_iq_format_bytes). */
+RFM_API int rfm_decoder_process_iq(rfm_decoder* d, int format, const void* iq, uint32_t n, float* audio,
+                                   size_t audio_stride, uint32_t* n_audio_floats);
+RFM_API int rfm_decoder_submit_iq(rfm_decoder* d, int format, const void* iq, uint32_t n, float* audio,
+                                  size_t audio_stride, uint32_t* n_audio_floats);
+RFM_API int rfm_decoder_process_iq_device(rfm_decoder* d, int format, const void* d_iq, size_t iq_stride, uint32_t n,
+                                          float* d_audio, size_t audio_stride, uint32_t* n_audio_floats,
+                                          void* cuda_stream);
 
 /* Make `cuda_stream` wait for every block enqueued so far (no host blocking) / block the host until done. */
 RFM_API int rfm_decoder_wait(rfm_decoder* d, void* cuda_stream);
@@ -207,6 +231,14 @@ RFM_API int rfm_freqshift_process_u8(rfm_freqshift* f, const uint8_t* iq, int sh
 /* device pointers; mode 0: cf32 rows (d_out may alias d_in), 1: one shared u8 capture, 2: u8 rows; strides in samples */
 RFM_API int rfm_freqshift_process_device(rfm_freqshift* f, int mode, const void* d_in, size_t in_stride, float* d_out,
                                          size_t out_stride, uint32_t n, void* cuda_stream);
+/* Any rfm_iq_format, converted on the fly: iq is one shared capture [n] (shared_capture != 0) or [rows][n] samples of
+ * `format`; out [rows][n][2] float.  Host form (blocking) and device form (enqueue only; strides in samples, in_stride is
+ * ignored for a shared capture, d_in aligned to the sample size). */
+RFM_API int rfm_freqshift_process_iq(rfm_freqshift* f, int format, int shared_capture, const void* iq, uint32_t n,
+                                     float* out);
+RFM_API int rfm_freqshift_process_iq_device(rfm_freqshift* f, int format, int shared_capture, const void* d_in,
+                                            size_t in_stride, float* d_out, size_t out_stride, uint32_t n,
+                                            void* cuda_stream);
 
 /* ------------------------------------------------------------------------------------------------
  * CRDSDownConvert (DownConvert.h:68-169, DownConvert.cpp:271-489), batched over rows: NCO_OSC mixer (the
@@ -248,6 +280,14 @@ RFM_API int rfm_downconvert_set_premix(rfm_downconvert* d, const float* d_table,
 /* device pointers, enqueue only; mode 0: cf32 rows, 1: one shared u8 capture, 2: u8 rows; strides in samples */
 RFM_API int rfm_downconvert_process_device(rfm_downconvert* d, int mode, const void* d_in, size_t in_stride, float* d_out,
                                            size_t out_stride, uint32_t n, uint32_t* n_out, void* cuda_stream);
+/* Any rfm_iq_format, converted on the fly: iq is one shared capture [n] (shared_capture != 0) or [rows][n] samples of
+ * `format`; out [rows][n >> stages][2] float.  Host form (blocking) and device form (enqueue only; strides in samples,
+ * in_stride is ignored for a shared capture, d_in aligned to the sample size). */
+RFM_API int rfm_downconvert_process_iq(rfm_downconvert* d, int format, int shared_capture, const void* iq, uint32_t n,
+                                       float* out, uint32_t* n_out);
+RFM_API int rfm_downconvert_process_iq_device(rfm_downconvert* d, int format, int shared_capture, const void* d_in,
+                                              size_t in_stride, float* d_out, size_t out_stride, uint32_t n,
+                                              uint32_t* n_out, void* cuda_stream);
 
 /* ------------------------------------------------------------------------------------------------
  * cDownsampleFilter (DownConvert.h:21-60, DownConvert.cpp:58-256), batched over rows: Lanczos-windowed sinc FIR with
@@ -466,8 +506,8 @@ RFM_API int rfm_demux_signal_status(rfm_demux* m, float* interface_level_db, flo
 /* ------------------------------------------------------------------------------------------------
  * Band scan of one wideband capture: the add-on's tuner auto-scan (ChannelSettings.cpp:96-147: retune one frequency,
  * wait, check cFmDecoder::StereoDetected) generalised to every channel of a capture in one pass.
- *   spectrum   Welch average over N = 4096 periodic-Hann segments, hop N/2, of x = float(u / 127.5 - 1)
- *              (RTL_SDR_Source.cpp:207-211): P[k] = sum_s |X_s[k]|^2 / (S N sum w^2), so sum_k P is the mean power of
+ *   spectrum   Welch average over N = 4096 periodic-Hann segments, hop N/2, of the capture converted to float as
+ *              rfm_iq_format says (u8: float(u / 127.5 - 1), RTL_SDR_Source.cpp:207-211): P[k] = sum_s |X_s[k]|^2 / (S N sum w^2), so sum_k P is the mean power of
  *              the windowed signal (a complex tone of modulus 1 is 0 dBFS).  Centred: index k <-> (k - N/2) Fs / N Hz.
  *              Independent of the device, its SM count and any SM partition (fixed work split, no atomics).
  *   channels   raster point f_j = raster_first + j raster_step owns the bins with f_j - step/2 <= f < f_j + step/2;
@@ -503,9 +543,12 @@ RFM_API void rfm_scan_config_default(rfm_scan_config* cfg);
  * a rate whose WFM decimation chain has no stage) before touching a device. */
 RFM_API int rfm_scan_create(const rfm_scan_config* cfg, rfm_scan** out);
 RFM_API void rfm_scan_destroy(rfm_scan* s);
-/* Whole capture [n][2] u8 in host memory (copied with cudaMemcpyAsync) or device memory (complete before the call,
- * 2-byte aligned); n >= one call (RFM_ERR_INVALID otherwise).  Blocking.  Zero candidates: no receiver is created and
- * the scan has 0 stations. */
+/* Whole capture of n samples of `format` (rfm_iq_format) in host memory (copied with cudaMemcpyAsync) or device memory
+ * (complete before the call, aligned to the sample size: 2 / 2 / 4 / 8 bytes); n >= one call (RFM_ERR_INVALID
+ * otherwise, as for an unknown format).  Blocking.  Zero candidates: no receiver is created and the scan has 0
+ * stations. */
+RFM_API int rfm_scan_run(rfm_scan* s, int format, const void* iq, uint64_t n, int iq_on_device);
+/* rfm_scan_run(s, RFM_IQ_U8, iq, n, iq_on_device) */
 RFM_API int rfm_scan_run_u8(rfm_scan* s, const uint8_t* iq, uint64_t n, int iq_on_device);
 RFM_API int rfm_scan_spectrum(rfm_scan* s, float* psd, uint32_t max, uint32_t* n_bins);   /* N floats, centred */
 RFM_API int rfm_scan_channel_power(rfm_scan* s, double* out, uint32_t max);              /* C_j, linear */

@@ -74,7 +74,51 @@ EXPORTED_SYMBOLS = (
     "rfm_rdsproc_process_device", "rfm_rdsproc_take_bits", "rfm_rdsproc_take_groups",
     "rfm_scan_config_default", "rfm_scan_create", "rfm_scan_destroy", "rfm_scan_run_u8", "rfm_scan_spectrum",
     "rfm_scan_channel_power", "rfm_scan_stations", "rfm_scan_timing",
+    "rfm_iq_format_bytes", "rfm_decoder_process_iq", "rfm_decoder_submit_iq", "rfm_decoder_process_iq_device",
+    "rfm_freqshift_process_iq", "rfm_freqshift_process_iq_device", "rfm_downconvert_process_iq",
+    "rfm_downconvert_process_iq_device", "rfm_scan_run",
 )
+
+# rfm_iq_format (include/radiofm_b200.h): interleaved I,Q; s8 = v * 2^-7, s16 = v * 2^-15 (exact), full scale of the container
+IQ_U8, IQ_S8, IQ_S16, IQ_CF32 = 0, 1, 2, 3
+_IQ_NAMES = {"u8": IQ_U8, "uint8": IQ_U8, "s8": IQ_S8, "int8": IQ_S8, "s16": IQ_S16, "int16": IQ_S16,
+             "cf32": IQ_CF32, "float32": IQ_CF32, "complex64": IQ_CF32}
+
+
+def iq_format(f) -> int:
+    """IQ format of a dtype (numpy or torch: uint8, int8, int16, float32 / complex64), a name ("u8", "s8", "s16",
+    "cf32") or an rfm_iq_format value."""
+    if isinstance(f, (int, np.integer)) and not isinstance(f, bool):
+        if int(f) not in (IQ_U8, IQ_S8, IQ_S16, IQ_CF32):
+            raise ValueError(f"unknown IQ format {f}")
+        return int(f)
+    name = str(f).replace("torch.", "")
+    if name not in _IQ_NAMES:
+        try:
+            name = str(np.dtype(f))
+        except TypeError:
+            pass
+    if name not in _IQ_NAMES:
+        raise ValueError(f"no IQ format for {f!r}: use uint8, int8, int16 or float32 / complex64")
+    return _IQ_NAMES[name]
+
+
+def iq_format_bytes(f) -> int:
+    """Bytes per complex sample of an IQ format: 2, 2, 4, 8."""
+    return int(lib().rfm_iq_format_bytes(iq_format(f)))
+
+
+_IQ_DTYPES = {IQ_U8: np.uint8, IQ_S8: np.int8, IQ_S16: np.int16, IQ_CF32: np.float32}
+
+
+def _iq_host(iq, rows: int | None = None):
+    """Host IQ -> (format, C-contiguous array with a trailing (I, Q) axis); rows: reshape to [rows, n, 2]."""
+    a = np.asarray(iq)
+    if a.dtype == np.complex64:
+        a = np.ascontiguousarray(a).view(np.float32)
+    fmt = iq_format(a.dtype)
+    a = np.ascontiguousarray(a, dtype=_IQ_DTYPES[fmt])
+    return fmt, (a.reshape(rows, -1, 2) if rows else a.reshape(-1, 2))
 
 
 _ADD_FRAME_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.POINTER(C.c_uint8), C.c_uint32)
@@ -269,6 +313,19 @@ def lib():
         L.rfm_scan_channel_power.argtypes = [C.c_void_p, _f64p, C.c_uint32]
         L.rfm_scan_stations.argtypes = [C.c_void_p, C.POINTER(ScanStation), C.c_uint32, _u32p]
         L.rfm_scan_timing.argtypes = [C.c_void_p, _f64p, _f64p]
+        L.rfm_iq_format_bytes.restype = C.c_uint32
+        L.rfm_iq_format_bytes.argtypes = [C.c_int]
+        L.rfm_decoder_process_iq.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_uint32, _f32p, C.c_size_t, _u32p]
+        L.rfm_decoder_submit_iq.argtypes = L.rfm_decoder_process_iq.argtypes
+        L.rfm_decoder_process_iq_device.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t, C.c_uint32, C.c_void_p,
+                                                    C.c_size_t, _u32p, C.c_void_p]
+        L.rfm_freqshift_process_iq.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_uint32, _f32p]
+        L.rfm_freqshift_process_iq_device.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p,
+                                                      C.c_size_t, C.c_uint32, C.c_void_p]
+        L.rfm_downconvert_process_iq.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_uint32, _f32p, _u32p]
+        L.rfm_downconvert_process_iq_device.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p,
+                                                        C.c_size_t, C.c_uint32, _u32p, C.c_void_p]
+        L.rfm_scan_run.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.c_int]
         L.rfm_rds_check_block.restype = C.c_uint32
         L.rfm_rds_check_block.argtypes = [C.c_uint32, C.c_uint32, C.c_int, _u32p]
         _lib = L
@@ -376,7 +433,32 @@ class FmDecoderBatch:
         _check(lib().rfm_decoder_process_cf32(self._h, _p(iq, _f32p), n, _p(audio, _f32p), stride, C.byref(k)))
         return audio[:, :k.value].copy()
 
+    def process_iq(self, iq: np.ndarray, submit: bool = False) -> np.ndarray:
+        """iq [S, n, 2] of uint8 / int8 / int16 / float32 (or [S, n] complex64) -> audio [S, floats] float32.  The
+        format comes from the dtype (iq_format).  submit: enqueue only (rfm_decoder_submit_iq); the audio is valid after
+        synchronize(), and iq must stay alive until then."""
+        fmt, iq = _iq_host(iq, self.n_streams)
+        n = iq.shape[1]
+        stride = max(self.max_audio_floats(n), 2)
+        audio = np.empty((self.n_streams, stride), dtype=np.float32)
+        k = C.c_uint32(0)
+        call = lib().rfm_decoder_submit_iq if submit else lib().rfm_decoder_process_iq
+        _check(call(self._h, fmt, iq.ctypes.data_as(C.c_void_p), n, _p(audio, _f32p), stride, C.byref(k)))
+        if submit:
+            self._submitted = (iq, audio)
+            return audio[:, :k.value]
+        return audio[:, :k.value].copy()
+
     # ---- device buffers (raw pointers, e.g. torch tensors' data_ptr()) ----
+    def process_iq_device(self, fmt, d_iq_ptr: int, iq_stride: int, n: int, d_audio_ptr: int, audio_stride: int,
+                          cuda_stream: int = 0) -> int:
+        """fmt: iq_format() of the device rows (a dtype such as torch.int16, a name or an rfm_iq_format value)."""
+        k = C.c_uint32(0)
+        _check(lib().rfm_decoder_process_iq_device(self._h, iq_format(fmt), C.c_void_p(d_iq_ptr), iq_stride, n,
+                                                   C.c_void_p(d_audio_ptr), audio_stride, C.byref(k),
+                                                   C.c_void_p(cuda_stream)))
+        return int(k.value)
+
     def process_u8_device(self, d_iq_ptr: int, iq_stride: int, n: int, d_audio_ptr: int, audio_stride: int,
                           cuda_stream: int = 0) -> int:
         k = C.c_uint32(0)
@@ -698,6 +780,22 @@ class FreqShiftBatch:
         _check(lib().rfm_freqshift_process_u8(self._h, _p(iq_u8, _u8p), int(shared_capture), n, _p(out, _f32p)))
         return out
 
+    def process_iq(self, iq: np.ndarray, shared_capture: bool) -> np.ndarray:
+        """iq of uint8 / int8 / int16 / float32 (complex64): one capture [n, 2] shared by every row, or [rows, n, 2] ->
+        out [rows, n, 2] float32."""
+        fmt, iq = _iq_host(iq)
+        n = iq.shape[0] // (1 if shared_capture else self.rows)
+        out = np.empty((self.rows, n, 2), dtype=np.float32)
+        _check(lib().rfm_freqshift_process_iq(self._h, fmt, int(shared_capture), iq.ctypes.data_as(C.c_void_p), n,
+                                              _p(out, _f32p)))
+        return out
+
+    def process_iq_device(self, fmt, shared_capture: bool, d_in_ptr: int, in_stride: int, d_out_ptr: int, out_stride: int,
+                          n: int, cuda_stream: int = 0):
+        _check(lib().rfm_freqshift_process_iq_device(self._h, iq_format(fmt), int(shared_capture), C.c_void_p(d_in_ptr),
+                                                     in_stride, C.c_void_p(d_out_ptr), out_stride, n,
+                                                     C.c_void_p(cuda_stream)))
+
     def process_device(self, mode: int, d_in_ptr: int, in_stride: int, d_out_ptr: int, out_stride: int, n: int,
                        cuda_stream: int = 0):
         _check(lib().rfm_freqshift_process_device(self._h, mode, C.c_void_p(d_in_ptr), in_stride, C.c_void_p(d_out_ptr),
@@ -754,6 +852,25 @@ class DownConvertBatch:
         _check(lib().rfm_downconvert_process_u8(self._h, _p(iq_u8, _u8p), int(shared_capture), n, _p(out, _f32p),
                                                 C.byref(k)))
         return out[:, :k.value].copy()
+
+    def process_iq(self, iq: np.ndarray, shared_capture: bool) -> np.ndarray:
+        """iq of uint8 / int8 / int16 / float32 (complex64): one capture [n, 2] shared by every row, or [rows, n, 2] ->
+        out [rows, n >> stages, 2] float32."""
+        fmt, iq = _iq_host(iq)
+        n = iq.shape[0] // (1 if shared_capture else self.rows)
+        out = np.empty((self.rows, max(n >> self.n_stages, 1), 2), dtype=np.float32)
+        k = C.c_uint32(0)
+        _check(lib().rfm_downconvert_process_iq(self._h, fmt, int(shared_capture), iq.ctypes.data_as(C.c_void_p), n,
+                                                _p(out, _f32p), C.byref(k)))
+        return out[:, :k.value].copy()
+
+    def process_iq_device(self, fmt, shared_capture: bool, d_in_ptr: int, in_stride: int, d_out_ptr: int,
+                          out_stride: int, n: int, cuda_stream: int = 0) -> int:
+        k = C.c_uint32(0)
+        _check(lib().rfm_downconvert_process_iq_device(self._h, iq_format(fmt), int(shared_capture), C.c_void_p(d_in_ptr),
+                                                       in_stride, C.c_void_p(d_out_ptr), out_stride, n, C.byref(k),
+                                                       C.c_void_p(cuda_stream)))
+        return int(k.value)
 
     def process_device(self, mode: int, d_in_ptr: int, in_stride: int, d_out_ptr: int, out_stride: int, n: int,
                        cuda_stream: int = 0) -> int:
@@ -940,7 +1057,7 @@ def scan_config(fs: float, raster_first: float, raster_step: float, raster_count
 
 
 class BandScan:
-    """Band scan of one wideband u8 capture (rfm_scan_*): averaged spectrum, channel powers on a raster (Hz from the
+    """Band scan of one wideband capture (rfm_scan_*; u8, s8, s16 or cf32): averaged spectrum, channel powers on a raster (Hz from the
     capture centre), candidates, and every candidate confirmed with the reference's receiver -- the add-on's tuner
     auto-scan (ChannelSettings.cpp:96-147) for all channels at once."""
 
@@ -962,6 +1079,19 @@ class BandScan:
         """Host capture [n, 2] uint8."""
         cap = np.ascontiguousarray(capture_u8, dtype=np.uint8).reshape(-1, 2)
         _check(lib().rfm_scan_run_u8(self._h, cap.ctypes.data_as(C.c_void_p), cap.shape[0], 0))
+
+    def run(self, capture):
+        """capture: a host array [n, 2] of uint8 / int8 / int16 / float32 ([n] complex64), or a CUDA tensor of those
+        dtypes, complete before the call (e.g. after torch.cuda.synchronize()).  The format comes from the dtype."""
+        if hasattr(capture, "data_ptr") and getattr(capture, "is_cuda", False):
+            fmt = iq_format(capture.dtype)
+            if not capture.is_contiguous():
+                raise ValueError("device capture must be contiguous")
+            n = capture.numel() // (1 if fmt == IQ_CF32 and capture.is_complex() else 2)
+            _check(lib().rfm_scan_run(self._h, fmt, C.c_void_p(capture.data_ptr()), n, 1))
+            return
+        fmt, cap = _iq_host(capture)
+        _check(lib().rfm_scan_run(self._h, fmt, cap.ctypes.data_as(C.c_void_p), cap.shape[0], 0))
 
     def run_device(self, d_capture_ptr: int, n: int):
         """Device capture [n, 2] uint8 at d_capture_ptr, complete before the call (e.g. after torch.cuda.synchronize())."""

@@ -4,7 +4,7 @@
 // Execution model.  One decoder = n_streams independent IQ streams processed in lock step, split into G groups
 // (G = 1 unless asked otherwise; the host-pointer entry points use groups to overlap H2D / compute / D2H).
 // Each group owns three CUDA streams and runs every block as a three-stage software pipeline:
-//     stage F (stream sF):  if_level, front (u8 -> tune -> FIR / ds), time-parallel FM-demodulator PLL
+//     stage F (stream sF):  if_level, front (IQ format -> float -> tune -> FIR / ds), time-parallel FM-demodulator PLL
 //     stage A (stream sA, high priority):  bb_lanes (DC tracker / meters || pilot PLL)
 //     stage B (stream sB):  { resample -> lp29 -> audio_tail }, { halfband* -> rds lp -> rds pll -> matched
 //                           filter -> slicer }, tails
@@ -28,6 +28,7 @@
 #include <vector>
 
 #include "../../include/radiofm_b200.h"
+#include "rfm_dsp.cuh"
 #include "rfm_kernels.cuh"
 #include "rfm_plan.h"
 #include "rfm_rdsgroup.h"
@@ -598,7 +599,7 @@ bool DebugSkip(const char* what)
 }
 
 // Stage F of one block for one group (stream sF): IF meter, front end.
-void EnqueueStageF(rfm_decoder* d, Group& g, const void* d_in, size_t in_stride, bool u8, const BlockGeom& bg,
+void EnqueueStageF(rfm_decoder* d, Group& g, const void* d_in, size_t in_stride, IqFormat fmt, const BlockGeom& bg,
                    unsigned par)
 {
   const DecoderPlan& p = d->plan;
@@ -611,9 +612,9 @@ void EnqueueStageF(rfm_decoder* d, Group& g, const void* d_in, size_t in_stride,
   fp.coeff = d->d_in_coeff.p; fp.coeff_host = p.in_coeff.data(); fp.tail = g.tail.p; fp.z = g.z[par].p; fp.z_stride = d->z_stride;
   fp.sm_count = d->part.rest ? d->part.rest_sms : 0;
   fp.fused = d->cfg.fir_fused != 0;
-  RFM_PROF(g.prof, "k_if_level", st, launch_if_level(fp, g.state.p, u8, st));
-  RFM_PROF(g.prof, "k_front", st, launch_front(fp, u8, st));
-  RFM_PROF(g.prof, "k_front_tail", st, launch_front_tail(fp, u8, st));
+  RFM_PROF(g.prof, "k_if_level", st, launch_if_level(fp, g.state.p, fmt, st));
+  RFM_PROF(g.prof, "k_front", st, launch_front(fp, fmt, st));
+  RFM_PROF(g.prof, "k_front_tail", st, launch_front_tail(fp, fmt, st));
 
   // FM-demodulator PLL, time-parallel (throughput work like the front end).  It overwrites incr[par], which the
   // lanes of block k-2 were reading.
@@ -784,7 +785,7 @@ void EnqueueStageB(rfm_decoder* d, Group& g, const BlockGeom& bg, unsigned par, 
 
 // One block for all groups.  Inputs / outputs are device pointers for the whole batch (host pointers when
 // host_staged).  Work is only enqueued; the device entry points return without waiting (rfm_decoder_wait).
-int ProcessDevice(rfm_decoder* d, const void* d_in, size_t in_stride, bool u8, unsigned n, float* d_audio,
+int ProcessDevice(rfm_decoder* d, const void* d_in, size_t in_stride, IqFormat fmt, unsigned n, float* d_audio,
                   size_t audio_stride, uint32_t* n_audio_floats, cudaStream_t user, bool host_staged,
                   bool host_sync = true)
 {
@@ -844,7 +845,7 @@ int ProcessDevice(rfm_decoder* d, const void* d_in, size_t in_stride, bool u8, u
     RFM_CUDA(cudaEventRecord(d->ev_osc[par3], d->s_osc));
   }
 
-  const size_t esz = u8 ? 2 : 8;
+  const size_t esz = IqBytes(fmt);
   for (auto& g : d->groups)
   {
     const unsigned char* in_g = reinterpret_cast<const unsigned char*>(d_in) + (size_t)g.s0 * in_stride * esz;
@@ -878,7 +879,7 @@ int ProcessDevice(rfm_decoder* d, const void* d_in, size_t in_stride, bool u8, u
       audio_stride_dev = d->audio_cap;
     }
     if (!DebugSkip("front"))
-      EnqueueStageF(d, g, in_dev, in_stride_dev, u8, bg, par);
+      EnqueueStageF(d, g, in_dev, in_stride_dev, fmt, bg, par);
     RFM_CUDA(cudaEventRecord(g.ev_front[par], g.sF));
     // ---- stage A
     RFM_CUDA(cudaStreamWaitEvent(g.sA, g.ev_front[par], 0));
@@ -969,6 +970,11 @@ extern "C"
 
 const char* rfm_last_error(void) { return g_err.c_str(); }
 const char* rfm_version(void) { return "radiofm_b200 0.2 (sm_100a)"; }
+
+uint32_t rfm_iq_format_bytes(int format)
+{
+  return (format >= RFM_IQ_U8 && format <= RFM_IQ_CF32) ? IqBytes(format) : 0u;
+}
 uint64_t rfm_launch_count(void) { return g_launches.load(); }
 
 void rfm_config_default(rfm_config* c)
@@ -1252,9 +1258,9 @@ uint32_t rfm_decoder_max_audio_floats(const rfm_decoder* d, uint32_t n)
   return 2 * ((unsigned)(nb / d->plan.a_ratio) + 4);
 }
 
-static int EnsureStaging(rfm_decoder* d, bool u8)
+static int EnsureStaging(rfm_decoder* d, int fmt)
 {
-  const size_t esz = u8 ? 2 : 8;
+  const size_t esz = IqBytes(fmt);
   for (auto& g : d->groups)
   {
     const size_t need = (size_t)g.S * d->maxn * esz;
@@ -1269,40 +1275,51 @@ static int EnsureStaging(rfm_decoder* d, bool u8)
   return RFM_OK;
 }
 
-int rfm_decoder_process_u8(rfm_decoder* d, const uint8_t* iq, uint32_t n, float* audio, size_t audio_stride,
-                           uint32_t* n_audio_floats)
+static bool KnownFormat(int fmt) { return fmt >= RFM_IQ_U8 && fmt <= RFM_IQ_CF32; }
+
+// Host buffers of any format: staged into device memory (cudaMemcpyAsync) and decoded; `submit` only enqueues.
+static int ProcessHost(rfm_decoder* d, int fmt, const void* iq, uint32_t n, float* audio, size_t audio_stride,
+                       uint32_t* n_audio_floats, bool submit)
 {
   if (!d || !iq || !audio)
     return Fail(RFM_ERR_INVALID, "null argument");
+  if (!KnownFormat(fmt))
+    return Fail(RFM_ERR_INVALID, "unknown IQ format");
   RFM_CUDA(cudaSetDevice(d->device));
-  int rc = EnsureStaging(d, true);
+  int rc = EnsureStaging(d, fmt);
   if (rc != RFM_OK)
     return rc;
-  return ProcessDevice(d, iq, n, true, n, audio, audio_stride, n_audio_floats, nullptr, true);
+  return ProcessDevice(d, iq, n, static_cast<IqFormat>(fmt), n, audio, audio_stride, n_audio_floats, nullptr, true, !submit);
+}
+
+int rfm_decoder_process_u8(rfm_decoder* d, const uint8_t* iq, uint32_t n, float* audio, size_t audio_stride,
+                           uint32_t* n_audio_floats)
+{
+  return ProcessHost(d, RFM_IQ_U8, iq, n, audio, audio_stride, n_audio_floats, false);
 }
 
 int rfm_decoder_process_cf32(rfm_decoder* d, const float* iq, uint32_t n, float* audio, size_t audio_stride,
                              uint32_t* n_audio_floats)
 {
-  if (!d || !iq || !audio)
-    return Fail(RFM_ERR_INVALID, "null argument");
-  RFM_CUDA(cudaSetDevice(d->device));
-  int rc = EnsureStaging(d, false);
-  if (rc != RFM_OK)
-    return rc;
-  return ProcessDevice(d, iq, n, false, n, audio, audio_stride, n_audio_floats, nullptr, true);
+  return ProcessHost(d, RFM_IQ_CF32, iq, n, audio, audio_stride, n_audio_floats, false);
+}
+
+int rfm_decoder_process_iq(rfm_decoder* d, int format, const void* iq, uint32_t n, float* audio, size_t audio_stride,
+                           uint32_t* n_audio_floats)
+{
+  return ProcessHost(d, format, iq, n, audio, audio_stride, n_audio_floats, false);
 }
 
 int rfm_decoder_submit_u8(rfm_decoder* d, const uint8_t* iq, uint32_t n, float* audio, size_t audio_stride,
                           uint32_t* n_audio_floats)
 {
-  if (!d || !iq || !audio)
-    return Fail(RFM_ERR_INVALID, "null argument");
-  RFM_CUDA(cudaSetDevice(d->device));
-  int rc = EnsureStaging(d, true);
-  if (rc != RFM_OK)
-    return rc;
-  return ProcessDevice(d, iq, n, true, n, audio, audio_stride, n_audio_floats, nullptr, true, false);
+  return ProcessHost(d, RFM_IQ_U8, iq, n, audio, audio_stride, n_audio_floats, true);
+}
+
+int rfm_decoder_submit_iq(rfm_decoder* d, int format, const void* iq, uint32_t n, float* audio, size_t audio_stride,
+                          uint32_t* n_audio_floats)
+{
+  return ProcessHost(d, format, iq, n, audio, audio_stride, n_audio_floats, true);
 }
 
 int rfm_decoder_process_u8_device(rfm_decoder* d, const uint8_t* d_iq, size_t iq_stride, uint32_t n, float* d_audio,
@@ -1310,7 +1327,7 @@ int rfm_decoder_process_u8_device(rfm_decoder* d, const uint8_t* d_iq, size_t iq
 {
   if (!d || !d_iq || !d_audio || iq_stride < n)
     return Fail(RFM_ERR_INVALID, "bad argument");
-  return ProcessDevice(d, d_iq, iq_stride, true, n, d_audio, audio_stride, n_audio_floats,
+  return ProcessDevice(d, d_iq, iq_stride, kIqU8, n, d_audio, audio_stride, n_audio_floats,
                        static_cast<cudaStream_t>(cuda_stream), false);
 }
 
@@ -1319,7 +1336,21 @@ int rfm_decoder_process_cf32_device(rfm_decoder* d, const float* d_iq, size_t iq
 {
   if (!d || !d_iq || !d_audio || iq_stride < n)
     return Fail(RFM_ERR_INVALID, "bad argument");
-  return ProcessDevice(d, d_iq, iq_stride, false, n, d_audio, audio_stride, n_audio_floats,
+  return ProcessDevice(d, d_iq, iq_stride, kIqCF32, n, d_audio, audio_stride, n_audio_floats,
+                       static_cast<cudaStream_t>(cuda_stream), false);
+}
+
+int rfm_decoder_process_iq_device(rfm_decoder* d, int format, const void* d_iq, size_t iq_stride, uint32_t n,
+                                  float* d_audio, size_t audio_stride, uint32_t* n_audio_floats, void* cuda_stream)
+{
+  if (!d || !d_iq || !d_audio || iq_stride < n)
+    return Fail(RFM_ERR_INVALID, "bad argument");
+  if (!KnownFormat(format))
+    return Fail(RFM_ERR_INVALID, "unknown IQ format");
+  // every sample is read with loads of its own size
+  if (reinterpret_cast<uintptr_t>(d_iq) % IqBytes(format) != 0)
+    return Fail(RFM_ERR_INVALID, "device IQ must be aligned to its sample size (2 / 2 / 4 / 8 bytes for u8 / s8 / s16 / cf32)");
+  return ProcessDevice(d, d_iq, iq_stride, static_cast<IqFormat>(format), n, d_audio, audio_stride, n_audio_floats,
                        static_cast<cudaStream_t>(cuda_stream), false);
 }
 

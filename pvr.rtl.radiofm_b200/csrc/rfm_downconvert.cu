@@ -1,6 +1,6 @@
 // rfm_downconvert.cu -- CRDSDownConvert (DownConvert.h:68-169, DownConvert.cpp:271-727) on the GPU, batched over rows
 // (one row per station of a wideband capture, or per stream), optionally fused with the u8 -> float conversion of
-// cRtlSdrSource::ReadAsyncCB (RTL_SDR_Source.cpp:207-211).
+// cRtlSdrSource::ReadAsyncCB (RTL_SDR_Source.cpp:207-211) or the exact s8 / s16 -> float conversions (rfm_dsp.cuh).
 //
 //   SetFrequency      -> per-row NCO_OSC rotation constants (DownConvert.cpp:311-320)
 //   SetDataRate /
@@ -65,7 +65,7 @@ struct DcStage
 
 struct DcParams
 {
-  const void* in;        // IN 0: cf32 [rows][in_stride]; 1: one shared u8 capture [n][2]; 2: u8 [rows][in_stride][2]
+  const void* in;        // [rows][in_stride] samples of the kernel's IQ format, or one shared capture [n] (SHARED)
   size_t in_stride;      // samples
   const float2* osc;     // NCO phasors [rows][osc_stride] (osc_stride == 0: one table for every row)
   size_t osc_stride;
@@ -85,14 +85,20 @@ struct DcParams
   unsigned pre_period, pre_pos;
 };
 
-template <int IN>
+// F: IqFormat.  A shared cf32 capture is read as rows of stride 0 (no instantiation of its own).
+template <int F, bool SHARED>
 __device__ __forceinline__ float2 dc_load(const DcParams& p, unsigned row, unsigned i)
 {
-  if (IN == 0)
+  if (F == kIqCF32)
     return reinterpret_cast<const float2*>(p.in)[(size_t)row * p.in_stride + i];
-  const unsigned char* b = reinterpret_cast<const unsigned char*>(p.in) + 2 * ((IN == 2 ? (size_t)row * p.in_stride : 0) + i);
+  if (F == kIqS16)
+  {
+    const unsigned w = reinterpret_cast<const unsigned*>(p.in)[(SHARED ? 0 : (size_t)row * p.in_stride) + i];
+    return make_float2(rfm_s16_to_float(w, 0u), rfm_s16_to_float(w, 1u));
+  }
+  const unsigned char* b = reinterpret_cast<const unsigned char*>(p.in) + 2 * ((!SHARED ? (size_t)row * p.in_stride : 0) + i);
   const unsigned w = *reinterpret_cast<const unsigned short*>(b);
-  return make_float2(rfm_u8_to_float(w, 0u), rfm_u8_to_float(w, 1u));
+  return make_float2(rfm_iq8_to_float<F>(w, 0u), rfm_iq8_to_float<F>(w, 1u));
 }
 
 // DownConvert.cpp:464-465 (and FreqShift.cpp:63-69: the same four products, one subtraction, one addition)
@@ -105,17 +111,17 @@ __device__ __forceinline__ float2 dc_mix(float2 d, float2 o)
 }
 
 // input sample i of this call for `row`, pre-mixed if a table is set, times the NCO phasor
-template <int IN>
+template <int F, bool SHARED>
 __device__ __forceinline__ float2 dc_sample(const DcParams& p, const float2* osc, unsigned row, unsigned i)
 {
-  float2 d = dc_load<IN>(p, row, i);
+  float2 d = dc_load<F, SHARED>(p, row, i);
   if (p.pre)
     d = dc_mix(d, p.pre[(size_t)row * p.pre_stride + (p.pre_pos + i) % p.pre_period]);
   return dc_mix(d, osc[i]);
 }
 
 // L2 prefetch of the global operands of tile [pos, pos + tn) (issued a tile ahead: the loads then hit L2)
-template <int IN>
+template <int F, bool SHARED>
 __device__ __forceinline__ void dc_prefetch(const DcParams& p, const float2* osc, unsigned row, unsigned pos, unsigned tn,
                                             unsigned tid)
 {
@@ -124,10 +130,12 @@ __device__ __forceinline__ void dc_prefetch(const DcParams& p, const float2* osc
     return;
   if (p.osc_stride)
     asm volatile("prefetch.global.L2 [%0];" ::"l"(osc + pos + i));
-  if (IN == 0)
+  if (F == kIqCF32)
     asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const float2*>(p.in) + (size_t)row * p.in_stride + pos + i));
-  if (IN == 2 && (i & 63u) == 0)
+  if (!SHARED && (F == kIqU8 || F == kIqS8) && (i & 63u) == 0)
     asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const unsigned char*>(p.in) + 2 * ((size_t)row * p.in_stride + pos + i)));
+  if (!SHARED && F == kIqS16 && (i & 31u) == 0)
+    asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const unsigned char*>(p.in) + 4 * ((size_t)row * p.in_stride + pos + i)));
 }
 
 // --------------------------------------------------------------------------------------------------
@@ -255,7 +263,7 @@ __global__ void __launch_bounds__(256) k_dc_osc_fill(float2* table, size_t strid
 // --------------------------------------------------------------------------------------------------
 // generic chain: any stage kinds, interleaved V buffers (the k_rds_front scheme without the LP)
 // --------------------------------------------------------------------------------------------------
-template <int IN>
+template <int F, bool SHARED>
 __global__ void __launch_bounds__(kDcThreads) k_dc_chain(DcParams p)
 {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -300,7 +308,7 @@ __global__ void __launch_bounds__(kDcThreads) k_dc_chain(DcParams p)
     const bool store = pos >= c_lo;
     const unsigned tn = min(kDcTileGeneric, (store ? c_hi : c_lo) - pos);
     for (unsigned i = tid; i < tn; i += kDcThreads)
-      B[0][p.st[0].hist + i] = dc_sample<IN>(p, osc, row, pos + i);
+      B[0][p.st[0].hist + i] = dc_sample<F, SHARED>(p, osc, row, pos + i);
     __syncthreads();
     unsigned n = tn;
     for (unsigned k = 0; k < p.nst; ++k)
@@ -374,7 +382,7 @@ __device__ __forceinline__ void dc_stage(const DcTapsPk<L>& taps, const float2* 
   }
 }
 
-template <int IN, int L>
+template <int F, bool SHARED, int L>
 __global__ void __launch_bounds__(kDcThreadsFast) k_dc_chain_uniform(DcParams p, DcTapsPk<L> taps)
 {
   constexpr int R = 5;                 // largest group: sizes the slack behind each buffer
@@ -427,7 +435,7 @@ __global__ void __launch_bounds__(kDcThreadsFast) k_dc_chain_uniform(DcParams p,
       unsigned pi = (unsigned)(((unsigned long long)p.pre_pos + pos + tid) % p.pre_period);
       for (unsigned i = tid; i < tn; i += kDcThreadsFast)
       {
-        const float2 d = dc_mix(dc_load<IN>(p, row, pos + i), pre[pi]);
+        const float2 d = dc_mix(dc_load<F, SHARED>(p, row, pos + i), pre[pi]);
         ((i & 1u) ? O_(0) : E_(0))[HH + (i >> 1)] = dc_mix(d, osc[pos + i]);
         pi += step;
         pi = pi >= p.pre_period ? pi - p.pre_period : pi;
@@ -435,13 +443,13 @@ __global__ void __launch_bounds__(kDcThreadsFast) k_dc_chain_uniform(DcParams p,
     }
     else
       for (unsigned i = tid; i < tn; i += kDcThreadsFast)
-        ((i & 1u) ? O_(0) : E_(0))[HH + (i >> 1)] = dc_sample<IN>(p, osc, row, pos + i);
+        ((i & 1u) ? O_(0) : E_(0))[HH + (i >> 1)] = dc_sample<F, SHARED>(p, osc, row, pos + i);
     __syncthreads();
     // operands of the next tile on their way into L2 while this one is filtered
     {
       const unsigned npos = pos + tn;
       if (npos < c_hi)
-        dc_prefetch<IN>(p, osc, row, npos, min(kDcTileFast, ((npos >= c_lo) ? c_hi : c_lo) - npos), tid);
+        dc_prefetch<F, SHARED>(p, osc, row, npos, min(kDcTileFast, ((npos >= c_lo) ? c_hi : c_lo) - npos), tid);
     }
     unsigned n = tn;
     for (unsigned k = 0; k < p.nst; ++k)
@@ -534,7 +542,8 @@ struct rfm_downconvert
   float2 *d_osc = nullptr, *d_tails[2] = {nullptr, nullptr};
   // host-pointer entry points: staging
   float2 *d_in = nullptr, *d_out = nullptr;
-  uint8_t* d_u8 = nullptr;
+  uint8_t* d_raw = nullptr;   // u8 / s8 / s16 input, raw_bytes
+  size_t raw_bytes = 0;
   DcTaps<51> taps51;
 };
 
@@ -576,7 +585,7 @@ int ResetState(rfm_downconvert* d)
   return ok ? RFM_OK : DcFail(RFM_ERR_CUDA, "rfm_downconvert: state reset failed");
 }
 
-template <int IN>
+template <int F, bool SHARED>
 void LaunchChain(rfm_downconvert* d, const DcParams& p, cudaStream_t st)
 {
   dim3 grid(p.nchunks, p.rows);
@@ -589,8 +598,8 @@ void LaunchChain(rfm_downconvert* d, const DcParams& p, cudaStream_t st)
       smem += 2 * (size_t)(25 + n / 2 + 5) * sizeof(float2);
       n >>= 1;
     }
-    EnsureDynSmem(k_dc_chain_uniform<IN, 51>, smem);
-    k_dc_chain_uniform<IN, 51><<<grid, kDcThreadsFast, smem, st>>>(p, MakeDcTapsPk(d->taps51));
+    EnsureDynSmem(k_dc_chain_uniform<F, SHARED, 51>, smem);
+    k_dc_chain_uniform<F, SHARED, 51><<<grid, kDcThreadsFast, smem, st>>>(p, MakeDcTapsPk(d->taps51));
   }
   else
   {
@@ -603,13 +612,14 @@ void LaunchChain(rfm_downconvert* d, const DcParams& p, cudaStream_t st)
       n >>= 1;
     }
     const size_t smem = floats * sizeof(float) + f2 * sizeof(float2);
-    EnsureDynSmem(k_dc_chain<IN>, smem);
-    k_dc_chain<IN><<<grid, kDcThreads, smem, st>>>(p);
+    EnsureDynSmem(k_dc_chain<F, SHARED>, smem);
+    k_dc_chain<F, SHARED><<<grid, kDcThreads, smem, st>>>(p);
   }
 }
 
-int Run(rfm_downconvert* d, int mode, const void* d_in, size_t in_stride, float2* d_out, size_t out_stride, uint32_t n,
-        uint32_t* n_out, cudaStream_t st)
+// fmt: IqFormat; shared: one capture for every row (a shared cf32 capture is read as rows of stride 0)
+int Run(rfm_downconvert* d, int fmt, bool shared, const void* d_in, size_t in_stride, float2* d_out, size_t out_stride,
+        uint32_t n, uint32_t* n_out, cudaStream_t st)
 {
   if (n_out)
     *n_out = 0;
@@ -627,7 +637,7 @@ int Run(rfm_downconvert* d, int mode, const void* d_in, size_t in_stride, float2
   k_dc_osc_fill<<<dim3(std::min(64u, (n + 1023) / 1024), orows), 256, 0, st>>>(d->d_osc, d->cap, n, d->d_cyc);
   DcParams p;
   memset(&p, 0, sizeof(p));
-  p.in = d_in; p.in_stride = in_stride;
+  p.in = d_in; p.in_stride = (shared && fmt == kIqCF32) ? 0 : in_stride;
   p.osc = d->d_osc; p.osc_stride = d->osc_shared ? 0 : d->cap;
   p.n = n; p.rows = d->rows; p.nst = d->nst;
   for (unsigned k = 0; k < d->nst; ++k)
@@ -676,12 +686,13 @@ int Run(rfm_downconvert* d, int mode, const void* d_in, size_t in_stride, float2
   p.pre = d->pre; p.pre_stride = d->pre_stride; p.pre_period = d->pre_period ? d->pre_period : 1; p.pre_pos = d->pre_pos;
   if (d->pre)
     d->pre_pos = (unsigned)(((uint64_t)d->pre_pos + n) % d->pre_period);
-  if (mode == 0)
-    LaunchChain<0>(d, p, st);
-  else if (mode == 1)
-    LaunchChain<1>(d, p, st);
-  else
-    LaunchChain<2>(d, p, st);
+  switch (fmt)
+  {
+    case kIqU8: shared ? LaunchChain<kIqU8, true>(d, p, st) : LaunchChain<kIqU8, false>(d, p, st); break;
+    case kIqS8: shared ? LaunchChain<kIqS8, true>(d, p, st) : LaunchChain<kIqS8, false>(d, p, st); break;
+    case kIqS16: shared ? LaunchChain<kIqS16, true>(d, p, st) : LaunchChain<kIqS16, false>(d, p, st); break;
+    default: LaunchChain<kIqCF32, false>(d, p, st); break;
+  }
   d->tails_cur ^= 1;
   rfm::g_launches += 3;
   if (n_out)
@@ -771,7 +782,7 @@ void rfm_downconvert_destroy(rfm_downconvert* d)
   cudaSetDevice(d->device);
   cudaFree(d->d_cos); cudaFree(d->d_sin); cudaFree(d->d_osc1); cudaFree(d->d_osc); cudaFree(d->d_cyc);
   cudaFree(d->d_tails[0]); cudaFree(d->d_tails[1]);
-  cudaFree(d->d_in); cudaFree(d->d_out); cudaFree(d->d_u8);
+  cudaFree(d->d_in); cudaFree(d->d_out); cudaFree(d->d_raw);
   for (auto* t : d->d_taps)
     cudaFree(t);
   delete d;
@@ -849,8 +860,45 @@ int rfm_downconvert_process_cf32(rfm_downconvert* d, const float* iq, uint32_t n
   if (cudaMemcpy(d->d_in, iq, (size_t)d->rows * n * 8, cudaMemcpyHostToDevice) != cudaSuccess)
     return DcFail(RFM_ERR_CUDA, "rfm_downconvert: H2D copy failed");
   uint32_t m = 0;
-  int rc = Run(d, 0, d->d_in, n, d->d_out, n >> d->nst, n, &m, 0);
+  int rc = Run(d, kIqCF32, false, d->d_in, n, d->d_out, n >> d->nst, n, &m, 0);
   if (rc == RFM_OK && m && cudaMemcpy(out, d->d_out, (size_t)d->rows * m * 8, cudaMemcpyDeviceToHost) != cudaSuccess)
+    rc = DcFail(RFM_ERR_CUDA, "rfm_downconvert: D2H copy failed");
+  if (n_out)
+    *n_out = m;
+  return rc;
+}
+
+int rfm_downconvert_process_iq(rfm_downconvert* d, int format, int shared_capture, const void* iq, uint32_t n, float* out,
+                               uint32_t* n_out)
+{
+  const uint32_t esz = rfm_iq_format_bytes(format);
+  if (!d || !iq || !out || esz == 0)
+    return DcFail(RFM_ERR_INVALID, "rfm_downconvert_process_iq: invalid argument");
+  if (format == RFM_IQ_CF32 && !shared_capture)
+    return rfm_downconvert_process_cf32(d, static_cast<const float*>(iq), n, out, n_out);
+  cudaSetDevice(d->device);
+  if (n > d->cap)
+    return DcFail(RFM_ERR_INVALID, "rfm_downconvert: n exceeds max_len");
+  // u8 and s8 fit the staging the u8 path has always allocated (rows x max_len x 2 bytes); s16 / cf32 grow it
+  const size_t need = std::max<size_t>((size_t)d->rows * d->cap * 2, (size_t)(shared_capture ? 1 : d->rows) * n * esz);
+  if (d->raw_bytes < need)
+  {
+    cudaFree(d->d_raw);
+    d->d_raw = nullptr;
+    d->raw_bytes = 0;
+    if (DevAlloc(&d->d_raw, need) != cudaSuccess)
+      return DcFail(RFM_ERR_CUDA, "rfm_downconvert: staging allocation failed");
+    d->raw_bytes = need;
+  }
+  if (!d->d_out && (DevAlloc(&d->d_out, (size_t)d->rows * (d->cap / 2 + 1)) != cudaSuccess))
+    return DcFail(RFM_ERR_CUDA, "rfm_downconvert: staging allocation failed");
+  if (cudaMemcpyAsync(d->d_raw, iq, (size_t)(shared_capture ? 1 : d->rows) * n * esz, cudaMemcpyHostToDevice, 0) != cudaSuccess)
+    return DcFail(RFM_ERR_CUDA, "rfm_downconvert: H2D copy failed");
+  uint32_t m = 0;
+  int rc = Run(d, format, shared_capture != 0, d->d_raw, n, d->d_out, n >> d->nst, n, &m, 0);
+  if (rc == RFM_OK && m &&
+      (cudaMemcpyAsync(out, d->d_out, (size_t)d->rows * m * 8, cudaMemcpyDeviceToHost, 0) != cudaSuccess ||
+       cudaStreamSynchronize(0) != cudaSuccess))
     rc = DcFail(RFM_ERR_CUDA, "rfm_downconvert: D2H copy failed");
   if (n_out)
     *n_out = m;
@@ -860,24 +908,22 @@ int rfm_downconvert_process_cf32(rfm_downconvert* d, const float* iq, uint32_t n
 int rfm_downconvert_process_u8(rfm_downconvert* d, const uint8_t* iq, int shared_capture, uint32_t n, float* out,
                                uint32_t* n_out)
 {
-  if (!d || !iq || !out)
-    return DcFail(RFM_ERR_INVALID, "rfm_downconvert_process_u8: invalid argument");
+  return rfm_downconvert_process_iq(d, RFM_IQ_U8, shared_capture, iq, n, out, n_out);
+}
+
+int rfm_downconvert_process_iq_device(rfm_downconvert* d, int format, int shared_capture, const void* d_in,
+                                      size_t in_stride, float* d_out, size_t out_stride, uint32_t n, uint32_t* n_out,
+                                      void* cuda_stream)
+{
+  const uint32_t esz = rfm_iq_format_bytes(format);
+  if (!d || !d_in || !d_out || esz == 0)
+    return DcFail(RFM_ERR_INVALID, "rfm_downconvert_process_iq_device: invalid argument");
+  if (reinterpret_cast<uintptr_t>(d_in) % esz != 0)
+    return DcFail(RFM_ERR_INVALID, "rfm_downconvert_process_iq_device: d_in must be aligned to the sample size "
+                                   "(2 / 2 / 4 / 8 bytes for u8 / s8 / s16 / cf32)");
   cudaSetDevice(d->device);
-  if (!d->d_u8 && (DevAlloc(&d->d_u8, (size_t)d->rows * d->cap * 2) != cudaSuccess))
-    return DcFail(RFM_ERR_CUDA, "rfm_downconvert: staging allocation failed");
-  if (!d->d_out && (DevAlloc(&d->d_out, (size_t)d->rows * (d->cap / 2 + 1)) != cudaSuccess))
-    return DcFail(RFM_ERR_CUDA, "rfm_downconvert: staging allocation failed");
-  if (n > d->cap)
-    return DcFail(RFM_ERR_INVALID, "rfm_downconvert: n exceeds max_len");
-  if (cudaMemcpy(d->d_u8, iq, (size_t)(shared_capture ? 1 : d->rows) * n * 2, cudaMemcpyHostToDevice) != cudaSuccess)
-    return DcFail(RFM_ERR_CUDA, "rfm_downconvert: H2D copy failed");
-  uint32_t m = 0;
-  int rc = Run(d, shared_capture ? 1 : 2, d->d_u8, n, d->d_out, n >> d->nst, n, &m, 0);
-  if (rc == RFM_OK && m && cudaMemcpy(out, d->d_out, (size_t)d->rows * m * 8, cudaMemcpyDeviceToHost) != cudaSuccess)
-    rc = DcFail(RFM_ERR_CUDA, "rfm_downconvert: D2H copy failed");
-  if (n_out)
-    *n_out = m;
-  return rc;
+  return Run(d, format, shared_capture != 0, d_in, in_stride, reinterpret_cast<float2*>(d_out), out_stride, n, n_out,
+             static_cast<cudaStream_t>(cuda_stream));
 }
 
 int rfm_downconvert_process_device(rfm_downconvert* d, int mode, const void* d_in, size_t in_stride, float* d_out,
@@ -886,8 +932,8 @@ int rfm_downconvert_process_device(rfm_downconvert* d, int mode, const void* d_i
   if (!d || !d_in || !d_out || mode < 0 || mode > 2)
     return DcFail(RFM_ERR_INVALID, "rfm_downconvert_process_device: invalid argument");
   cudaSetDevice(d->device);
-  return Run(d, mode, d_in, in_stride, reinterpret_cast<float2*>(d_out), out_stride, n, n_out,
-             static_cast<cudaStream_t>(cuda_stream));
+  return Run(d, mode == 0 ? kIqCF32 : kIqU8, mode == 1, d_in, in_stride, reinterpret_cast<float2*>(d_out), out_stride, n,
+             n_out, static_cast<cudaStream_t>(cuda_stream));
 }
 
 } // extern "C"

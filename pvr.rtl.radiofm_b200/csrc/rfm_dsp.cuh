@@ -1,5 +1,5 @@
 // rfm_dsp.cuh -- device building blocks shared by the chain kernels (rfm_kernels.cu) and the stand-alone primitives
-// (rfm_downconvert.cu): exact u8 -> float conversion, the decimate-by-2 stage bodies of CRDSDownConvert.
+// (rfm_downconvert.cu): exact u8 / s8 / s16 -> float conversions, the decimate-by-2 stage bodies of CRDSDownConvert.
 #pragma once
 
 #include <cuda_runtime.h>
@@ -18,6 +18,38 @@ __device__ __forceinline__ float rfm_u8_to_float(unsigned word, unsigned byte_se
   const float u = __fsub_rn(m, 8388608.0f);
   const float t = __fmaf_rn(u, 0x1.01p-7f, -1.0f);
   return __fmaf_rn(u, 0x1.010102p-23f, t);
+}
+
+// Formats of the caller's IQ (rfm_iq_format in include/radiofm_b200.h): interleaved I,Q, little-endian.
+enum IqFormat : int
+{
+  kIqU8 = 0,  // RTL-SDR offset binary, rfm_u8_to_float
+  kIqS8 = 1,  // cs8 (HackRF): v * 2^-7
+  kIqS16 = 2, // cs16 (SoapySDR / UHD host format): v * 2^-15
+  kIqCF32 = 3
+};
+__host__ __device__ constexpr unsigned IqBytes(int f) { return f == kIqCF32 ? 8u : f == kIqS16 ? 4u : 2u; }
+
+// Signed byte byte_sel of word -> v * 2^-7.  Flipping the sign bit makes v + 128 an unsigned byte, which lands in the
+// mantissa of 2^23 as for the u8 form; every step is exact, so the result is (float)v * 2^-7 for all 256 codes.
+__device__ __forceinline__ float rfm_s8_to_float(unsigned word, unsigned byte_sel)
+{
+  const float m = __uint_as_float(__byte_perm(word ^ 0x80808080u, 0x4B000000u, 0x7540u + byte_sel)); // 2^23 + v + 128
+  return __fmul_rn(__fsub_rn(m, 8388736.0f), 0x1p-7f);
+}
+
+// Signed half hi (0: bits 0-15, 1: bits 16-31) of word -> v * 2^-15, exact for all 65536 codes (same construction).
+__device__ __forceinline__ float rfm_s16_to_float(unsigned word, unsigned hi)
+{
+  const float m = __uint_as_float(__byte_perm(word ^ 0x80008000u, 0x4B000000u, hi ? 0x7632u : 0x7610u)); // 2^23 + v + 2^15
+  return __fmul_rn(__fsub_rn(m, 8421376.0f), 0x1p-15f);
+}
+
+// One byte-sized component of a u8 or s8 word
+template <int F>
+__device__ __forceinline__ float rfm_iq8_to_float(unsigned word, unsigned byte_sel)
+{
+  return F == kIqS8 ? rfm_s8_to_float(word, byte_sel) : rfm_u8_to_float(word, byte_sel);
 }
 
 // OscGn = 1.95 - (re^2 + im^2) of the NCO_OSC rotating vector (DownConvert.cpp:441): the double literal makes it

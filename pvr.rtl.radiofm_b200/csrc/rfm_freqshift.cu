@@ -1,6 +1,6 @@
 // rfm_freqshift.cu -- cFreqShift (FreqShift.h:12-27, FreqShift.cpp:10-76) on the GPU, batched over rows (one row per
 // station of a wideband capture, or per stream), optionally fused with the u8 -> float conversion of
-// cRtlSdrSource::ReadAsyncCB (RTL_SDR_Source.cpp:207-211).
+// cRtlSdrSource::ReadAsyncCB (RTL_SDR_Source.cpp:207-211) or the exact s8 / s16 -> float conversions (rfm_dsp.cuh).
 //
 // Bug-compatible with the reference's x86 branch: the NCO phase is a float32 that is advanced by a float32 increment
 // and NEVER wrapped (FreqShift.cpp:71-72).  The phase sequence is therefore a sequential float recurrence
@@ -14,9 +14,15 @@
 #include <vector>
 
 #include "../../include/radiofm_b200.h"
+#include "rfm_dsp.cuh"
 #include "rfm_math.cuh"
 
 using namespace rfm;
+
+namespace rfm
+{
+void SetLastError(const std::string& m);
+}
 
 namespace
 {
@@ -47,7 +53,9 @@ __global__ void __launch_bounds__(32) k_fs_phase(const float* inc, float* time, 
     time[r] = acc;
 }
 
-template <int MODE> // 0: cf32 rows in place, 1: one shared u8 capture -> cf32 rows, 2: u8 rows -> cf32 rows
+// F: IqFormat of the input rows (cf32 rows may be mixed in place), or of one capture shared by every row (SHARED; a
+// shared cf32 capture is read as rows of stride 0)
+template <int F, bool SHARED>
 __global__ void __launch_bounds__(256) k_fs_mix(const float* ph, size_t ph_stride, const void* in, size_t in_stride,
                                                 float2* out, size_t out_stride, unsigned n, const float* lut)
 {
@@ -58,12 +66,22 @@ __global__ void __launch_bounds__(256) k_fs_mix(const float* ph, size_t ph_strid
   float s, c;
   rfm_sincos(ph[(size_t)r * ph_stride + i], &s, &c);
   float2 d;
-  if (MODE == 0)
+  if (F == kIqCF32)
     d = reinterpret_cast<const float2*>(in)[(size_t)r * in_stride + i];
+  else if (F == kIqU8)
+  {
+    const uchar2 u = reinterpret_cast<const uchar2*>(in)[(SHARED ? 0 : (size_t)r * in_stride) + i];
+    d = make_float2(lut[u.x], lut[u.y]);
+  }
+  else if (F == kIqS8)
+  {
+    const unsigned w = reinterpret_cast<const unsigned short*>(in)[(SHARED ? 0 : (size_t)r * in_stride) + i];
+    d = make_float2(rfm_s8_to_float(w, 0u), rfm_s8_to_float(w, 1u));
+  }
   else
   {
-    const uchar2 u = reinterpret_cast<const uchar2*>(in)[(MODE == 1 ? 0 : (size_t)r * in_stride) + i];
-    d = make_float2(lut[u.x], lut[u.y]);
+    const unsigned w = reinterpret_cast<const unsigned*>(in)[(SHARED ? 0 : (size_t)r * in_stride) + i];
+    d = make_float2(rfm_s16_to_float(w, 0u), rfm_s16_to_float(w, 1u));
   }
   float2 o;
   o.x = subf(mulf(d.x, c), mulf(d.y, s)); // FreqShift.cpp:63-69
@@ -82,7 +100,8 @@ struct rfm_freqshift
   bool at_zero = true;
   unsigned ph0_n = 0;
   float2* d_io = nullptr;
-  uint8_t* d_u8 = nullptr;
+  uint8_t* d_raw = nullptr;   // host input of the _iq / _u8 calls, raw_bytes
+  size_t raw_bytes = 0;
   std::string err;
 };
 
@@ -113,7 +132,8 @@ int rfm_freqshift_create(uint32_t rows, const float* nco_freq, float in_rate, ui
             cudaMalloc(&f->d_ph, (size_t)rows * max_len * 4) == cudaSuccess && cudaMalloc(&f->d_lut, 1024) == cudaSuccess &&
             cudaMalloc(&f->d_time_end, rows * 4) == cudaSuccess &&
             cudaMalloc(&f->d_io, (size_t)rows * max_len * 8) == cudaSuccess &&
-            cudaMalloc(&f->d_u8, (size_t)rows * max_len * 2) == cudaSuccess;
+            cudaMalloc(&f->d_raw, (size_t)rows * max_len * 2) == cudaSuccess;
+  f->raw_bytes = ok ? (size_t)rows * max_len * 2 : 0;
   if (ok)
   {
     cudaMemcpy(f->d_inc, inc.data(), rows * 4, cudaMemcpyHostToDevice);
@@ -135,7 +155,7 @@ void rfm_freqshift_destroy(rfm_freqshift* f)
     return;
   cudaSetDevice(f->device);
   cudaFree(f->d_time_end);
-  cudaFree(f->d_inc); cudaFree(f->d_time); cudaFree(f->d_ph); cudaFree(f->d_lut); cudaFree(f->d_io); cudaFree(f->d_u8);
+  cudaFree(f->d_inc); cudaFree(f->d_time); cudaFree(f->d_ph); cudaFree(f->d_lut); cudaFree(f->d_io); cudaFree(f->d_raw);
   delete f;
 }
 
@@ -148,8 +168,8 @@ int rfm_freqshift_reset(rfm_freqshift* f) // FreqShift.cpp:18-21
   return cudaMemsetAsync(f->d_time, 0, f->rows * 4, 0) == cudaSuccess ? RFM_OK : RFM_ERR_CUDA;
 }
 
-static int Run(rfm_freqshift* f, int mode, const void* d_in, size_t in_stride, float2* d_out, size_t out_stride,
-               uint32_t n, cudaStream_t st)
+static int Run(rfm_freqshift* f, int fmt, bool shared, const void* d_in, size_t in_stride, float2* d_out,
+               size_t out_stride, uint32_t n, cudaStream_t st)
 {
   if (f->at_zero && f->ph0_n == n)
     cudaMemcpyAsync(f->d_time, f->d_time_end, f->rows * 4, cudaMemcpyDeviceToDevice, st); // table still valid
@@ -165,12 +185,15 @@ static int Run(rfm_freqshift* f, int mode, const void* d_in, size_t in_stride, f
   }
   f->at_zero = false;
   dim3 grid((n + 255) / 256, f->rows);
-  if (mode == 0)
-    k_fs_mix<0><<<grid, 256, 0, st>>>(f->d_ph, f->cap, d_in, in_stride, d_out, out_stride, n, f->d_lut);
-  else if (mode == 1)
-    k_fs_mix<1><<<grid, 256, 0, st>>>(f->d_ph, f->cap, d_in, in_stride, d_out, out_stride, n, f->d_lut);
-  else
-    k_fs_mix<2><<<grid, 256, 0, st>>>(f->d_ph, f->cap, d_in, in_stride, d_out, out_stride, n, f->d_lut);
+#define RFM_FS_MIX(F, SHARED) k_fs_mix<F, SHARED><<<grid, 256, 0, st>>>(f->d_ph, f->cap, d_in, in_stride, d_out, out_stride, n, f->d_lut)
+  switch (fmt)
+  {
+    case kIqU8: if (shared) RFM_FS_MIX(kIqU8, true); else RFM_FS_MIX(kIqU8, false); break;
+    case kIqS8: if (shared) RFM_FS_MIX(kIqS8, true); else RFM_FS_MIX(kIqS8, false); break;
+    case kIqS16: if (shared) RFM_FS_MIX(kIqS16, true); else RFM_FS_MIX(kIqS16, false); break;
+    default: in_stride = shared ? 0 : in_stride; RFM_FS_MIX(kIqCF32, false); break;
+  }
+#undef RFM_FS_MIX
   return cudaGetLastError() == cudaSuccess ? RFM_OK : RFM_ERR_CUDA;
 }
 
@@ -184,26 +207,61 @@ int rfm_freqshift_process_cf32(rfm_freqshift* f, float* iq, uint32_t n)
   const size_t bytes = (size_t)f->rows * n * 8;
   if (cudaMemcpy(f->d_io, iq, bytes, cudaMemcpyHostToDevice) != cudaSuccess)
     return RFM_ERR_CUDA;
-  int rc = Run(f, 0, f->d_io, n, f->d_io, n, n, 0);
+  int rc = Run(f, kIqCF32, false, f->d_io, n, f->d_io, n, n, 0);
   if (rc == RFM_OK && cudaMemcpy(iq, f->d_io, bytes, cudaMemcpyDeviceToHost) != cudaSuccess)
+    rc = RFM_ERR_CUDA;
+  return rc;
+}
+
+int rfm_freqshift_process_iq(rfm_freqshift* f, int format, int shared_capture, const void* iq, uint32_t n, float* out)
+{
+  const uint32_t esz = rfm_iq_format_bytes(format);
+  if (!f || !iq || !out || n > f->cap || esz == 0)
+    return RFM_ERR_INVALID;
+  if (n == 0)
+    return RFM_OK;
+  cudaSetDevice(f->device);
+  const size_t in_bytes = (size_t)(shared_capture ? 1 : f->rows) * n * esz;
+  if (f->raw_bytes < in_bytes)
+  {
+    cudaFree(f->d_raw);
+    f->d_raw = nullptr;
+    f->raw_bytes = 0;
+    if (cudaMalloc(&f->d_raw, in_bytes) != cudaSuccess)
+      return RFM_ERR_CUDA;
+    f->raw_bytes = in_bytes;
+  }
+  if (cudaMemcpyAsync(f->d_raw, iq, in_bytes, cudaMemcpyHostToDevice, 0) != cudaSuccess)
+    return RFM_ERR_CUDA;
+  int rc = Run(f, format, shared_capture != 0, f->d_raw, n, f->d_io, n, n, 0);
+  if (rc == RFM_OK && (cudaMemcpyAsync(out, f->d_io, (size_t)f->rows * n * 8, cudaMemcpyDeviceToHost, 0) != cudaSuccess ||
+                       cudaStreamSynchronize(0) != cudaSuccess))
     rc = RFM_ERR_CUDA;
   return rc;
 }
 
 int rfm_freqshift_process_u8(rfm_freqshift* f, const uint8_t* iq, int shared_capture, uint32_t n, float* out)
 {
-  if (!f || !iq || !out || n > f->cap)
+  return rfm_freqshift_process_iq(f, RFM_IQ_U8, shared_capture, iq, n, out);
+}
+
+int rfm_freqshift_process_iq_device(rfm_freqshift* f, int format, int shared_capture, const void* d_in, size_t in_stride,
+                                    float* d_out, size_t out_stride, uint32_t n, void* cuda_stream)
+{
+  const uint32_t esz = rfm_iq_format_bytes(format);
+  if (!f || !d_in || !d_out || n > f->cap || esz == 0)
     return RFM_ERR_INVALID;
+  if (reinterpret_cast<uintptr_t>(d_in) % esz != 0)
+  {
+    rfm::SetLastError("rfm_freqshift_process_iq_device: d_in must be aligned to the sample size (2 / 2 / 4 / 8 bytes for "
+                      "u8 / s8 / s16 / cf32)");
+    return RFM_ERR_INVALID;
+  }
   if (n == 0)
     return RFM_OK;
   cudaSetDevice(f->device);
-  const size_t in_bytes = (size_t)(shared_capture ? 1 : f->rows) * n * 2;
-  if (cudaMemcpy(f->d_u8, iq, in_bytes, cudaMemcpyHostToDevice) != cudaSuccess)
-    return RFM_ERR_CUDA;
-  int rc = Run(f, shared_capture ? 1 : 2, f->d_u8, n, f->d_io, n, n, 0);
-  if (rc == RFM_OK && cudaMemcpy(out, f->d_io, (size_t)f->rows * n * 8, cudaMemcpyDeviceToHost) != cudaSuccess)
-    rc = RFM_ERR_CUDA;
-  return rc;
+  return Run(f, format, shared_capture != 0, d_in, in_stride, reinterpret_cast<float2*>(d_out), out_stride, n,
+             static_cast<cudaStream_t>(cuda_stream));
 }
 
 int rfm_freqshift_process_device(rfm_freqshift* f, int mode, const void* d_in, size_t in_stride, float* d_out,
@@ -214,7 +272,8 @@ int rfm_freqshift_process_device(rfm_freqshift* f, int mode, const void* d_in, s
   if (n == 0)
     return RFM_OK;
   cudaSetDevice(f->device);
-  return Run(f, mode, d_in, in_stride, reinterpret_cast<float2*>(d_out), out_stride, n, static_cast<cudaStream_t>(cuda_stream));
+  return Run(f, mode == 0 ? kIqCF32 : kIqU8, mode == 1, d_in, in_stride, reinterpret_cast<float2*>(d_out), out_stride, n,
+             static_cast<cudaStream_t>(cuda_stream));
 }
 
 } // extern "C"

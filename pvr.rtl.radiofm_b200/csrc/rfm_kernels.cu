@@ -6,7 +6,7 @@
 // results are bit-identical to the CPU chain (see DESIGN.md, "Numerics").
 //
 // Kernel map (SURVEY.md section 7 / 8a rows in brackets):
-//   k_front        [a1 a3 a5]   u8 -> LUT -> fine-tuner rotate -> Lanczos FIR / ds; tile of outputs
+//   k_front        [a1 a3 a5]   u8 | s8 | s16 | cf32 -> float -> fine-tuner rotate -> Lanczos FIR / ds; tile of outputs
 //                               per CTA, input + halo staged in shared memory
 //   k_front_tail   [a5 state]   last `order` tuned samples -> m_stateComplex
 //   k_bb_lanes     [a4 a6 a13 a15 a16] one lane per stream: IF meter, FM-demod PLL + DC tracker,
@@ -58,18 +58,30 @@ void EnsureDynSmemImpl(const void* func, size_t smem)
 // ==================================================================================================
 constexpr unsigned kFrontTile = 128; // outputs per CTA == threads per CTA
 
-// fine-tuned sample i of this block: (u8 -> float) * table[(idx0 + i) mod 64]
+// fine-tuned sample i of this block: (IQ format F -> float) * table[(idx0 + i) mod 64]
 // RTL_SDR_Source.cpp:207-211, FmDecode.cpp:66-82 (std::complex product: ac-bd, ad+bc)
-template <bool U8>
+template <int F>
 __device__ __forceinline__ float2 tuned_sample(const void* __restrict__ row, unsigned i, unsigned idx0,
                                                const float* lut, const float2* tuner)
 {
   float are, aim;
-  if (U8)
+  if (F == kIqU8)
   {
     const uchar2 u = reinterpret_cast<const uchar2*>(row)[i];
     are = lut[u.x];
     aim = lut[u.y];
+  }
+  else if (F == kIqS8)
+  {
+    const unsigned w = reinterpret_cast<const unsigned short*>(row)[i];
+    are = rfm_s8_to_float(w, 0u);
+    aim = rfm_s8_to_float(w, 1u);
+  }
+  else if (F == kIqS16)
+  {
+    const unsigned w = reinterpret_cast<const unsigned*>(row)[i];
+    are = rfm_s16_to_float(w, 0u);
+    aim = rfm_s16_to_float(w, 1u);
   }
   else
   {
@@ -86,7 +98,7 @@ __device__ __forceinline__ float2 tuned_sample(const void* __restrict__ row, uns
   return o;
 }
 
-template <bool U8>
+template <int F>
 __global__ void __launch_bounds__(kFrontTile) k_front(FrontParams p)
 {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -112,13 +124,13 @@ __global__ void __launch_bounds__(kFrontTile) k_front(FrontParams p)
   // V = tail(order) ++ block(n); this tile needs V[vlo .. vlo + count)
   const unsigned vlo = p.p0 + o0 * p.ds;
   const unsigned count = (nt - 1) * p.ds + p.order;
-  const size_t esz = U8 ? 2 : 8;
+  const size_t esz = IqBytes(F);
   const unsigned char* row = reinterpret_cast<const unsigned char*>(p.in) + (size_t)s * p.in_stride * esz;
   const float2* tail = reinterpret_cast<const float2*>(p.tail) + (size_t)s * p.order;
   for (unsigned v = tid; v < count; v += kFrontTile)
   {
     const unsigned V = vlo + v;
-    X[v] = (V < p.order) ? tail[V] : tuned_sample<U8>(row, V - p.order, p.idx0, s_lut, p.tuner ? s_tuner : nullptr);
+    X[v] = (V < p.order) ? tail[V] : tuned_sample<F>(row, V - p.order, p.idx0, s_lut, p.tuner ? s_tuner : nullptr);
   }
   __syncthreads();
 
@@ -138,20 +150,20 @@ __global__ void __launch_bounds__(kFrontTile) k_front(FrontParams p)
   }
 }
 
-template <bool U8>
+template <int F>
 __global__ void __launch_bounds__(256) k_front_tail(FrontParams p)
 {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float2* tmp = reinterpret_cast<float2*>(smem_raw);
   const unsigned s = blockIdx.x;
-  const size_t esz = U8 ? 2 : 8;
+  const size_t esz = IqBytes(F);
   const unsigned char* row = reinterpret_cast<const unsigned char*>(p.in) + (size_t)s * p.in_stride * esz;
   float2* tail = reinterpret_cast<float2*>(p.tail) + (size_t)s * p.order;
   const float2* tuner = reinterpret_cast<const float2*>(p.tuner);
   for (unsigned k = threadIdx.x; k < p.order; k += blockDim.x)
   {
     const unsigned V = p.n + k; // new tail = V[n .. n + order)
-    tmp[k] = (V < p.order) ? tail[V] : tuned_sample<U8>(row, V - p.order, p.idx0, p.lut, tuner);
+    tmp[k] = (V < p.order) ? tail[V] : tuned_sample<F>(row, V - p.order, p.idx0, p.lut, tuner);
   }
   __syncthreads();
   for (unsigned k = threadIdx.x; k < p.order; k += blockDim.x)
@@ -186,7 +198,8 @@ struct FrontGeom
   __host__ __device__ static constexpr int pos(int w) { return w + w / SEG; }
 };
 
-template <bool U8, int DS>
+// BYTES: two-byte samples (u8, s8) staged in 16-byte chunks, else one load per sample (s16, cf32); F: IqFormat
+template <bool BYTES, int DS, int F = BYTES ? kIqU8 : kIqCF32>
 __global__ void __launch_bounds__(128) k_front_tiled(FrontParams p, FrontCoef cf)
 {
   using G = FrontGeom<DS>;
@@ -212,7 +225,8 @@ __global__ void __launch_bounds__(128) k_front_tiled(FrontParams p, FrontCoef cf
   // ---- window: new samples i in [i_lo, i_hi) of this block, sample i lands at w = i + order - vlo
   const int i_lo = max(0, (int)vlo - G::ORDER);
   const int i_hi = min((int)p.n, (int)(vlo + count) - G::ORDER);
-  if (U8)
+  static_assert(BYTES == (F == kIqU8 || F == kIqS8), "staging follows the sample size");
+  if (BYTES)
   {
     const unsigned char* row = reinterpret_cast<const unsigned char*>(p.in) + (size_t)s * p.in_stride * 2;
     // 16-byte chunks of 8 samples, aligned in memory: chunk c holds samples k0 + 8c .. k0 + 8c + 7
@@ -249,8 +263,8 @@ __global__ void __launch_bounds__(128) k_front_tiled(FrontParams p, FrontCoef cf
         for (int e = 0; e < 8; ++e)
         {
           const unsigned word = wd[e >> 1];
-          const float are = rfm_u8_to_float(word, (e & 1) ? 2u : 0u);
-          const float aim = rfm_u8_to_float(word, (e & 1) ? 3u : 1u);
+          const float are = rfm_iq8_to_float<F>(word, (e & 1) ? 2u : 0u);
+          const float aim = rfm_iq8_to_float<F>(word, (e & 1) ? 3u : 1u);
           float2 o;
           o.x = subf(mulf(are, tw[e].x), mulf(aim, tw[e].y));   // FmDecode.cpp:66-82
           o.y = addf(mulf(are, tw[e].y), mulf(aim, tw[e].x));
@@ -279,14 +293,29 @@ __global__ void __launch_bounds__(128) k_front_tiled(FrontParams p, FrontCoef cf
         if (i >= i_lo && i < i_hi)
         {
           const unsigned word = wd[e >> 1];
-          const float are = rfm_u8_to_float(word, (e & 1) ? 2u : 0u);
-          const float aim = rfm_u8_to_float(word, (e & 1) ? 3u : 1u);
+          const float are = rfm_iq8_to_float<F>(word, (e & 1) ? 2u : 0u);
+          const float aim = rfm_iq8_to_float<F>(word, (e & 1) ? 3u : 1u);
           float2 o;
           o.x = subf(mulf(are, tw[e].x), mulf(aim, tw[e].y));
           o.y = addf(mulf(are, tw[e].y), mulf(aim, tw[e].x));
           X[G::pos(i + G::ORDER - (int)vlo)] = o;
         }
       }
+    }
+  }
+  else if (F == kIqS16)
+  {
+    // one 32-bit word per sample: the rows are read as the cf32 rows below, half the bytes
+    const unsigned* row = reinterpret_cast<const unsigned*>(p.in) + (size_t)s * p.in_stride;
+    for (int i = i_lo + (int)tid; i < i_hi; i += G::T)
+    {
+      const unsigned w = row[i];
+      const float2 a = make_float2(rfm_s16_to_float(w, 0u), rfm_s16_to_float(w, 1u));
+      const float2 b = tuner[(p.idx0 + (unsigned)i) & 63u];
+      float2 o;
+      o.x = subf(mulf(a.x, b.x), mulf(a.y, b.y));
+      o.y = addf(mulf(a.x, b.y), mulf(a.y, b.x));
+      X[G::pos(i + G::ORDER - (int)vlo)] = o;
     }
   }
   else
@@ -344,7 +373,7 @@ __global__ void __launch_bounds__(128) k_front_tiled(FrontParams p, FrontCoef cf
 }
 
 // --------------------------------------------------------------------------------------------------
-// TMA form of the same kernel for u8 input and ds = 1, 5, 11 (390 625 S/s, 1.2 and 2.4 MS/s).
+// TMA form of the same kernel for u8 and s8 input (same byte geometry) and ds = 1, 5, 11 (390 625 S/s, 1.2, 2.4 MS/s).
 //   * the raw u8 window -- ((384-1) ds + order) IQ pairs plus alignment -- is fetched by the TMA unit: one elected
 //     thread issues cp.async.bulk.tensor.2d over a tensor map of the caller's [S][n] rows (8-byte elements = 4 IQ
 //     pairs, boxes of 256 elements = 2 KB) and the CTA waits on an mbarrier.  Out-of-range coordinates (before the
@@ -376,9 +405,9 @@ struct FrontGeom3
 
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 
-template <int DS, bool FUSED>
-__global__ void __launch_bounds__(128) k_front_tma(FrontParams p, FrontCoef cf, const __grid_constant__ CUtensorMap tmap,
-                                                   unsigned tiles_per_row, unsigned total_tiles)
+template <int F, int DS, bool FUSED>
+__device__ __forceinline__ void front_tma(const FrontParams& p, const FrontCoef& cf, const CUtensorMap& tmap,
+                                          unsigned tiles_per_row, unsigned total_tiles)
 {
   using G = FrontGeom3<DS>;
   extern __shared__ __align__(128) unsigned char smem_front_tma[];
@@ -449,8 +478,8 @@ __global__ void __launch_bounds__(128) k_front_tma(FrontParams p, FrontCoef cf, 
     const unsigned* raw32 = reinterpret_cast<const unsigned*>(raw) + tid;
     auto tuned_pair = [&](int j) {
       const unsigned word = raw32[G::T * j];
-      const float are0 = rfm_u8_to_float(word, 0u), aim0 = rfm_u8_to_float(word, 1u);
-      const float are1 = rfm_u8_to_float(word, 2u), aim1 = rfm_u8_to_float(word, 3u);
+      const float are0 = rfm_iq8_to_float<F>(word, 0u), aim0 = rfm_iq8_to_float<F>(word, 1u);
+      const float are1 = rfm_iq8_to_float<F>(word, 2u), aim1 = rfm_iq8_to_float<F>(word, 3u);
       float4 o;
       o.x = subf(mulf(are0, tw0.x), mulf(aim0, tw0.y));   // FmDecode.cpp:66-82
       o.y = addf(mulf(are0, tw0.y), mulf(aim0, tw0.x));
@@ -521,6 +550,22 @@ __global__ void __launch_bounds__(128) k_front_tma(FrontParams p, FrontCoef cf, 
   }
 }
 
+// u8 and s8 share the byte geometry (tensor map, boxes, pair-per-lane staging); only the conversion of a pair differs
+template <int DS, bool FUSED>
+__global__ void __launch_bounds__(128) k_front_tma(FrontParams p, FrontCoef cf, const __grid_constant__ CUtensorMap tmap,
+                                                   unsigned tiles_per_row, unsigned total_tiles)
+{
+  front_tma<kIqU8, DS, FUSED>(p, cf, tmap, tiles_per_row, total_tiles);
+}
+template <int DS, bool FUSED>
+__global__ void __launch_bounds__(128) k_front_cs8_tma(FrontParams p, FrontCoef cf, const __grid_constant__ CUtensorMap tmap,
+                                                       unsigned tiles_per_row, unsigned total_tiles)
+{
+  front_tma<kIqS8, DS, FUSED>(p, cf, tmap, tiles_per_row, total_tiles);
+}
+template <int F, int DS, bool FUSED>
+static constexpr auto front_tma_kernel() { return F == kIqS8 ? k_front_cs8_tma<DS, FUSED> : k_front_tma<DS, FUSED>; }
+
 // cuTensorMapEncodeTiled through the runtime's driver entry point (libcuda is not linked)
 static bool EncodeFrontMap(const FrontParams& p, CUtensorMap* map)
 {
@@ -549,14 +594,15 @@ static bool EncodeFrontMap(const FrontParams& p, CUtensorMap* map)
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <int DS, bool FUSED>
+template <int F, int DS, bool FUSED>
 static bool launch_front_tma(const FrontParams& p, const FrontCoef& cf, cudaStream_t st)
 {
   using G = FrontGeom3<DS>;
   CUtensorMap map;
   if (!EncodeFrontMap(p, &map))
     return false;
-  EnsureDynSmem(k_front_tma<DS, FUSED>, G::SMEM);
+  const auto kernel = front_tma_kernel<F, DS, FUSED>();
+  EnsureDynSmem(kernel, G::SMEM);
   const unsigned tpr = cdiv(p.nout, G::OB), total = tpr * p.S;
   // persistent: one wave of resident CTAs (as many as fit on the device), each walks total / grid tiles
   int dev = 0, sms = 0, occ = 0;
@@ -564,85 +610,104 @@ static bool launch_front_tma(const FrontParams& p, const FrontCoef& cf, cudaStre
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   if (p.sm_count) // the launching stream lives in an SM partition
     sms = (int)p.sm_count;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_front_tma<DS, FUSED>, G::T, G::SMEM) != cudaSuccess)
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, G::T, G::SMEM) != cudaSuccess)
     occ = 1;
   const unsigned grid = std::min<unsigned>(total, (unsigned)(std::max(sms, 1) * std::max(occ, 1)));
-  k_front_tma<DS, FUSED><<<grid, G::T, G::SMEM, st>>>(p, cf, map, tpr, total);
+  kernel<<<grid, G::T, G::SMEM, st>>>(p, cf, map, tpr, total);
   return true;
 }
 
-template <bool U8, int DS>
+template <int F, int DS>
 static void launch_front_tiled(const FrontParams& p, const FrontCoef& cf, cudaStream_t st)
 {
   using G = FrontGeom<DS>;
+  constexpr bool kBytes = F == kIqU8 || F == kIqS8;
   const size_t smem = (size_t)G::WP * sizeof(float2);
-  EnsureDynSmem(k_front_tiled<U8, DS>, smem);
+  EnsureDynSmem(k_front_tiled<kBytes, DS, F>, smem);
   dim3 grid(cdiv(p.nout, G::OB), p.S);
-  k_front_tiled<U8, DS><<<grid, G::T, smem, st>>>(p, cf);
+  k_front_tiled<kBytes, DS, F><<<grid, G::T, smem, st>>>(p, cf);
 }
 
-void launch_front(const FrontParams& p, bool u8, cudaStream_t st)
+template <int F>
+static bool launch_front_tma_ds(const FrontParams& p, const FrontCoef& cf, cudaStream_t st)
+{
+  if (p.fused)
+    return p.ds == 11 ? launch_front_tma<F, 11, true>(p, cf, st) : p.ds == 5 ? launch_front_tma<F, 5, true>(p, cf, st) : launch_front_tma<F, 1, true>(p, cf, st);
+  return p.ds == 11 ? launch_front_tma<F, 11, false>(p, cf, st) : p.ds == 5 ? launch_front_tma<F, 5, false>(p, cf, st) : launch_front_tma<F, 1, false>(p, cf, st);
+}
+
+template <int F>
+static void launch_front_tiled_ds(const FrontParams& p, const FrontCoef& cf, cudaStream_t st)
+{
+  switch (p.ds)
+  {
+    case 1: launch_front_tiled<F, 1>(p, cf, st); break;
+    case 4: launch_front_tiled<F, 4>(p, cf, st); break;
+    case 5: launch_front_tiled<F, 5>(p, cf, st); break;
+    default: launch_front_tiled<F, 11>(p, cf, st); break;
+  }
+}
+
+template <int F>
+static void launch_front_generic(const FrontParams& p, cudaStream_t st)
+{
+  const unsigned coef_n = (p.order + 2 + 1) & ~1u;
+  const size_t smem = (256 + 128 + coef_n) * sizeof(float) + ((size_t)(kFrontTile - 1) * p.ds + p.order) * sizeof(float2);
+  dim3 grid(cdiv(p.nout, kFrontTile), p.S);
+  EnsureDynSmem(k_front<F>, smem);
+  k_front<F><<<grid, kFrontTile, smem, st>>>(p);
+}
+
+void launch_front(const FrontParams& p, IqFormat fmt, cudaStream_t st)
 {
   if (p.nout == 0 || p.S == 0)
     return;
+  // u8 / s8: two bytes per sample; the tiled kernel's byte staging needs an even row base
+  const bool bytes = fmt == kIqU8 || fmt == kIqS8;
   const bool tiled = p.order == 8 * p.ds && (p.ds == 1 || p.ds == 4 || p.ds == 5 || p.ds == 11) && p.coeff_host &&
-                     (!u8 || ((reinterpret_cast<uintptr_t>(p.in) | (p.in_stride * 2)) & 1u) == 0);
+                     (!bytes || ((reinterpret_cast<uintptr_t>(p.in) | (p.in_stride * 2)) & 1u) == 0);
   if (tiled)
   {
     FrontCoef cf;
     memset(&cf, 0, sizeof(cf));
     memcpy(cf.c, p.coeff_host, (p.order + 2) * sizeof(float));
-    // TMA form: u8 rows that a tensor map can describe (16-byte aligned base and row pitch, whole 8-byte elements)
-    if (u8 && p.tuner && (p.ds == 1 || p.ds == 5 || p.ds == 11) && p.n % 4 == 0 && p.n >= 4 &&
+    // TMA form: u8 / s8 rows that a tensor map can describe (16-byte aligned base and row pitch, whole 8-byte elements)
+    if (bytes && p.tuner && (p.ds == 1 || p.ds == 5 || p.ds == 11) && p.n % 4 == 0 && p.n >= 4 &&
         (reinterpret_cast<uintptr_t>(p.in) & 15u) == 0 && (p.in_stride * 2) % 16 == 0)
     {
-      bool ok;
-      if (p.fused)
-        ok = p.ds == 11 ? launch_front_tma<11, true>(p, cf, st) : p.ds == 5 ? launch_front_tma<5, true>(p, cf, st) : launch_front_tma<1, true>(p, cf, st);
-      else
-        ok = p.ds == 11 ? launch_front_tma<11, false>(p, cf, st) : p.ds == 5 ? launch_front_tma<5, false>(p, cf, st) : launch_front_tma<1, false>(p, cf, st);
-      if (ok)
+      if (fmt == kIqU8 ? launch_front_tma_ds<kIqU8>(p, cf, st) : launch_front_tma_ds<kIqS8>(p, cf, st))
         return;
     }
-#define RFM_FT(DS)                                    \
-  if (u8)                                             \
-    launch_front_tiled<true, DS>(p, cf, st);          \
-  else                                                \
-    launch_front_tiled<false, DS>(p, cf, st)
-    switch (p.ds)
+    switch (fmt)
     {
-      case 1: RFM_FT(1); break;
-      case 4: RFM_FT(4); break;
-      case 5: RFM_FT(5); break;
-      default: RFM_FT(11); break;
+      case kIqU8: launch_front_tiled_ds<kIqU8>(p, cf, st); break;
+      case kIqS8: launch_front_tiled_ds<kIqS8>(p, cf, st); break;
+      case kIqS16: launch_front_tiled_ds<kIqS16>(p, cf, st); break;
+      default: launch_front_tiled_ds<kIqCF32>(p, cf, st); break;
     }
-#undef RFM_FT
     return;
   }
-  const unsigned coef_n = (p.order + 2 + 1) & ~1u;
-  const size_t smem = (256 + 128 + coef_n) * sizeof(float) + ((size_t)(kFrontTile - 1) * p.ds + p.order) * sizeof(float2);
-  dim3 grid(cdiv(p.nout, kFrontTile), p.S);
-  if (u8)
+  switch (fmt)
   {
-    EnsureDynSmem(k_front<true>, smem);
-    k_front<true><<<grid, kFrontTile, smem, st>>>(p);
-  }
-  else
-  {
-    EnsureDynSmem(k_front<false>, smem);
-    k_front<false><<<grid, kFrontTile, smem, st>>>(p);
+    case kIqU8: launch_front_generic<kIqU8>(p, st); break;
+    case kIqS8: launch_front_generic<kIqS8>(p, st); break;
+    case kIqS16: launch_front_generic<kIqS16>(p, st); break;
+    default: launch_front_generic<kIqCF32>(p, st); break;
   }
 }
 
-void launch_front_tail(const FrontParams& p, bool u8, cudaStream_t st)
+void launch_front_tail(const FrontParams& p, IqFormat fmt, cudaStream_t st)
 {
   if (p.S == 0 || p.n == 0)
     return;
   const size_t smem = (size_t)p.order * sizeof(float2);
-  if (u8)
-    k_front_tail<true><<<p.S, 256, smem, st>>>(p);
-  else
-    k_front_tail<false><<<p.S, 256, smem, st>>>(p);
+  switch (fmt)
+  {
+    case kIqU8: k_front_tail<kIqU8><<<p.S, 256, smem, st>>>(p); break;
+    case kIqS8: k_front_tail<kIqS8><<<p.S, 256, smem, st>>>(p); break;
+    case kIqS16: k_front_tail<kIqS16><<<p.S, 256, smem, st>>>(p); break;
+    default: k_front_tail<kIqCF32><<<p.S, 256, smem, st>>>(p); break;
+  }
 }
 
 // ==================================================================================================
@@ -714,7 +779,7 @@ __device__ __forceinline__ void bar_arrive_imm() { asm volatile("bar.arrive %0, 
 // --------------------------------------------------------------------------------------------------
 // IF level meter: RMSLevelApprox over the first ceil(n/64) tuned samples, FmDecode.cpp:427,505-519
 // --------------------------------------------------------------------------------------------------
-template <bool U8>
+template <int F>
 __global__ void __launch_bounds__(128) k_if_level(FrontParams f, float* state)
 {
   // one warp per stream: the |x|^2 terms are formed in parallel (coalesced), the float sum itself runs in sample
@@ -725,7 +790,7 @@ __global__ void __launch_bounds__(128) k_if_level(FrontParams f, float* state)
   if (s >= f.S)
     return;
   const unsigned cnt = (f.n + 63) / 64;
-  const size_t esz = U8 ? 2 : 8;
+  const size_t esz = IqBytes(F);
   const unsigned char* row = reinterpret_cast<const unsigned char*>(f.in) + (size_t)s * f.in_stride * esz;
   const float2* tuner = reinterpret_cast<const float2*>(f.tuner);
   float level = 0.0f;
@@ -734,7 +799,7 @@ __global__ void __launch_bounds__(128) k_if_level(FrontParams f, float* state)
     const unsigned m = min(1024u, cnt - i0);
     for (unsigned i = lane; i < m; i += 32)
     {
-      const float2 t = tuned_sample<U8>(row, i0 + i, f.idx0, f.lut, tuner);
+      const float2 t = tuned_sample<F>(row, i0 + i, f.idx0, f.lut, tuner);
       terms[warp][i] = addf(mulf(t.x, t.x), mulf(t.y, t.y));
     }
     __syncwarp();
@@ -751,14 +816,17 @@ __global__ void __launch_bounds__(128) k_if_level(FrontParams f, float* state)
   }
 }
 
-void launch_if_level(const FrontParams& p, float* state, bool u8, cudaStream_t st)
+void launch_if_level(const FrontParams& p, float* state, IqFormat fmt, cudaStream_t st)
 {
   if (p.S == 0 || p.n == 0)
     return;
-  if (u8)
-    k_if_level<true><<<cdiv(p.S, 4), 128, 0, st>>>(p, state);
-  else
-    k_if_level<false><<<cdiv(p.S, 4), 128, 0, st>>>(p, state);
+  switch (fmt)
+  {
+    case kIqU8: k_if_level<kIqU8><<<cdiv(p.S, 4), 128, 0, st>>>(p, state); break;
+    case kIqS8: k_if_level<kIqS8><<<cdiv(p.S, 4), 128, 0, st>>>(p, state); break;
+    case kIqS16: k_if_level<kIqS16><<<cdiv(p.S, 4), 128, 0, st>>>(p, state); break;
+    default: k_if_level<kIqCF32><<<cdiv(p.S, 4), 128, 0, st>>>(p, state); break;
+  }
 }
 
 // --------------------------------------------------------------------------------------------------

@@ -82,10 +82,10 @@ enum StateField
   SF_COUNT
 };
 
-// ---- front end: (u8 | cf32) -> fine tuner -> Lanczos FIR / ds -----------------------------------------
+// ---- front end: (u8 | s8 | s16 | cf32) -> fine tuner -> Lanczos FIR / ds ---------------------------------
 struct FrontParams
 {
-  const void* in;          // u8 [S][in_stride][2] or cf32 [S][in_stride]
+  const void* in;          // [S][in_stride] samples of the IQ format (rfm_dsp.cuh IqFormat)
   size_t in_stride;        // samples per row
   unsigned n;              // new samples per stream
   unsigned S;
@@ -103,11 +103,12 @@ struct FrontParams
   unsigned sm_count = 0;   // SMs of the launching stream's partition (0: the whole device); sizes persistent grids
   bool fused = false;      // tolerance mode (rfm_config::fir_fused): FFMA in the FIR, not bit-exact
 };
-void launch_front(const FrontParams& p, bool u8, cudaStream_t st);
-void launch_front_tail(const FrontParams& p, bool u8, cudaStream_t st);
+enum IqFormat : int; // rfm_dsp.cuh (an enum, so that no bool or stray integer converts to a format)
+void launch_front(const FrontParams& p, IqFormat fmt, cudaStream_t st);
+void launch_front_tail(const FrontParams& p, IqFormat fmt, cudaStream_t st);
 
 // ---- baseband lanes: IF meter, FM-demod PLL, DC tracker, BB meters, pilot PLL, 38 kHz demux multiply --
-void launch_if_level(const FrontParams& p, float* state, bool u8, cudaStream_t st);
+void launch_if_level(const FrontParams& p, float* state, IqFormat fmt, cudaStream_t st);
 
 // ---- FM-demodulator PLL: speculative chunk-parallel pass + exactness check / sequential repair --------------------
 struct DemodSpecParams

@@ -21,6 +21,7 @@
 #include <vector>
 
 #include "../../include/radiofm_b200.h"
+#include "rfm_dsp.cuh"
 #include "rfm_kernels.cuh"
 #include "rfm_plan.h"
 #include "rfm_rdssync.h"
@@ -953,8 +954,8 @@ int rfm_downsample_process_complex_device(rfm_downsample* f, const float* d_in, 
   fp.p0 = pos; fp.nout = nout; fp.idx0 = 0; fp.lut = f->d_lut; fp.tuner = nullptr;
   fp.coeff = f->d_coeff; fp.coeff_host = nullptr; // generic kernel (the tiled one has the fine tuner built in)
   fp.tail = f->d_tail; fp.z = reinterpret_cast<cf32*>(d_out); fp.z_stride = out_stride;
-  launch_front(fp, false, st);
-  launch_front_tail(fp, false, st);
+  launch_front(fp, kIqCF32, st);
+  launch_front_tail(fp, kIqCF32, st);
   f->pos_int = pos + nout * ds - n; // :132
   rfm::g_launches += 2;
   if (n_out)

@@ -1,4 +1,4 @@
-// rfm_scan.cu -- band scan of one wideband u8 capture: which FM stations does it hold, how strong are they, and what
+// rfm_scan.cu -- band scan of one wideband capture (u8, s8, s16 or cf32): which FM stations does it hold, how strong are they, and what
 // do they identify as.  The reference's tuner dialog answers this one frequency at a time (ChannelSettings.cpp:96-147:
 // retune, wait, cFmDecoder::StereoDetected); here every channel of the capture is decided in one pass.
 //
@@ -93,9 +93,23 @@ __device__ __forceinline__ void ScanPass(const float2* __restrict__ x, float2* _
   }
 }
 
-// Partial Welch sums: CTA b transforms segments [b * 32, b * 32 + 32) of the capture (u8 I,Q pairs; segment g covers
-// samples [g N/2, g N/2 + N)) and writes sum |X_g[k]|^2 over them, natural bin order, to partial[b][k].
-__global__ void __launch_bounds__(kScanThreads) k_scan_psd(const unsigned short* __restrict__ cap, uint64_t n_seg,
+// One capture sample of IqFormat F (rfm_dsp.cuh): its storage type and its value as float
+template <int F> struct ScanIn { using T = unsigned short; };   // u8, s8: one byte each for I and Q
+template <> struct ScanIn<rfm::kIqS16> { using T = unsigned; };
+template <> struct ScanIn<rfm::kIqCF32> { using T = float2; };
+__device__ __forceinline__ float2 ScanSample(unsigned w)
+{
+  return make_float2(rfm::rfm_s16_to_float(w, 0u), rfm::rfm_s16_to_float(w, 1u));
+}
+__device__ __forceinline__ float2 ScanSample(float2 v)
+{
+  return v;
+}
+
+// Partial Welch sums: CTA b transforms segments [b * 32, b * 32 + 32) of the capture (I,Q samples of format F; segment g
+// covers samples [g N/2, g N/2 + N)) and writes sum |X_g[k]|^2 over them, natural bin order, to partial[b][k].
+template <int F>
+__global__ void __launch_bounds__(kScanThreads) k_scan_psd(const typename ScanIn<F>::T* __restrict__ cap, uint64_t n_seg,
                                                            const float* __restrict__ win, const float2* __restrict__ tw,
                                                            float* __restrict__ partial)
 {
@@ -111,14 +125,29 @@ __global__ void __launch_bounds__(kScanThreads) k_scan_psd(const unsigned short*
     acc[j] = 0.0f;
   for (uint64_t g = g0; g < g1; ++g)
   {
-    const unsigned short* seg = cap + g * kScanHop;
-#pragma unroll
-    for (unsigned j = 0; j < kScanPerThread; ++j)
+    const typename ScanIn<F>::T* seg = cap + g * kScanHop;
+    if constexpr (F == rfm::kIqU8 || F == rfm::kIqS8)
     {
-      const unsigned i = tid + j * kScanThreads;
-      const unsigned w = __ldg(seg + i);
-      const float h = __ldg(win + i);
-      A[i] = make_float2(h * rfm::rfm_u8_to_float(w, 0u), h * rfm::rfm_u8_to_float(w, 1u));
+#pragma unroll
+      for (unsigned j = 0; j < kScanPerThread; ++j)
+      {
+        const unsigned i = tid + j * kScanThreads;
+        const unsigned w = __ldg(seg + i);
+        const float h = __ldg(win + i);
+        A[i] = make_float2(h * rfm::rfm_iq8_to_float<F>(w, 0u), h * rfm::rfm_iq8_to_float<F>(w, 1u));
+      }
+    }
+    else
+    {
+      // partly unrolled: fully unrolled, the wider loads of the whole segment were hoisted into 190 registers
+#pragma unroll 4
+      for (unsigned j = 0; j < kScanPerThread; ++j)
+      {
+        const unsigned i = tid + j * kScanThreads;
+        const float2 x = ScanSample(__ldg(seg + i));
+        const float h = __ldg(win + i);
+        A[i] = make_float2(h * x.x, h * x.y);
+      }
     }
     __syncthreads();
     ScanPass<0>(A, B, tw, tid);
@@ -199,7 +228,7 @@ namespace
 {
 // The candidates' receivers: one rfm_downconvert row and one rfm_decoder stream per candidate, `calls` calls of
 // n_call capture samples each, the front end on the decoder's companion stream, three baseband slots.
-int Confirm(rfm_scan* s, const uint8_t* d_cap, uint64_t calls, const std::vector<uint32_t>& cand)
+int Confirm(rfm_scan* s, int fmt, const uint8_t* d_cap, uint64_t calls, const std::vector<uint32_t>& cand)
 {
   const uint32_t M = (uint32_t)cand.size();
   std::vector<float> nco(M);
@@ -255,8 +284,8 @@ int Confirm(rfm_scan* s, const uint8_t* d_cap, uint64_t calls, const std::vector
       if (k >= kScanSlots)
         cudaStreamWaitEvent((cudaStream_t)front, ev_free[slot], 0);   // the slot's previous call has left the decoder
       uint32_t m = 0, na = 0;
-      rc = rfm_downconvert_process_device(dc, 1, d_cap + 2 * k * (uint64_t)s->n_call, s->n_call,
-                                          reinterpret_cast<float*>(bb[slot]), kScanCallBb, s->n_call, &m, front);
+      rc = rfm_downconvert_process_iq_device(dc, fmt, 1, d_cap + rfm::IqBytes(fmt) * k * (uint64_t)s->n_call, s->n_call,
+                                             reinterpret_cast<float*>(bb[slot]), kScanCallBb, s->n_call, &m, front);
       if (rc == RFM_OK && m != kScanCallBb)
         rc = ScanFail(RFM_ERR_CUDA, "rfm_scan: unexpected front-end output length");
       if (rc != RFM_OK)
@@ -477,49 +506,67 @@ void rfm_scan_destroy(rfm_scan* s)
 
 int rfm_scan_run_u8(rfm_scan* s, const uint8_t* iq, uint64_t n, int iq_on_device)
 {
+  return rfm_scan_run(s, RFM_IQ_U8, iq, n, iq_on_device);
+}
+
+int rfm_scan_run(rfm_scan* s, int format, const void* iq, uint64_t n, int iq_on_device)
+{
   if (!s || !iq)
-    return ScanFail(RFM_ERR_INVALID, "rfm_scan_run_u8: null argument");
+    return ScanFail(RFM_ERR_INVALID, "rfm_scan_run: null argument");
+  const uint32_t esz = rfm_iq_format_bytes(format);
+  if (esz == 0)
+    return ScanFail(RFM_ERR_INVALID, "rfm_scan_run: unknown IQ format");
   if (n < s->n_call)
-    return ScanFail(RFM_ERR_INVALID, "rfm_scan_run_u8: the capture is shorter than one demodulator call");
-  if (iq_on_device && (reinterpret_cast<uintptr_t>(iq) & 1))
-    return ScanFail(RFM_ERR_INVALID, "rfm_scan_run_u8: device capture must be 2-byte aligned");
+    return ScanFail(RFM_ERR_INVALID, "rfm_scan_run: the capture is shorter than one demodulator call");
+  if (iq_on_device && (reinterpret_cast<uintptr_t>(iq) % esz) != 0)
+    return ScanFail(RFM_ERR_INVALID, "rfm_scan_run: device capture must be aligned to the sample size "
+                                     "(2 / 2 / 4 / 8 bytes for u8 / s8 / s16 / cf32)");
   if (cudaSetDevice(s->device) != cudaSuccess)
     return ScanFail(RFM_ERR_CUDA, "cudaSetDevice failed");
   s->have = false;
-  const uint8_t* d_cap = iq;
+  const uint8_t* d_cap = static_cast<const uint8_t*>(iq);
   if (!iq_on_device)
   {
-    if (s->cap_bytes < 2 * n)
+    if (s->cap_bytes < esz * n)
     {
       cudaFree(s->d_cap);
       s->d_cap = nullptr;
       s->cap_bytes = 0;
-      if (DevAlloc(&s->d_cap, 2 * n) != cudaSuccess)
-        return ScanFail(RFM_ERR_CUDA, "rfm_scan_run_u8: capture allocation failed");
-      s->cap_bytes = 2 * n;
+      if (DevAlloc(&s->d_cap, esz * n) != cudaSuccess)
+        return ScanFail(RFM_ERR_CUDA, "rfm_scan_run: capture allocation failed");
+      s->cap_bytes = esz * n;
     }
-    if (cudaMemcpyAsync(s->d_cap, iq, 2 * n, cudaMemcpyHostToDevice, s->st) != cudaSuccess)
-      return ScanFail(RFM_ERR_CUDA, "rfm_scan_run_u8: H2D copy failed");
+    if (cudaMemcpyAsync(s->d_cap, iq, esz * n, cudaMemcpyHostToDevice, s->st) != cudaSuccess)
+      return ScanFail(RFM_ERR_CUDA, "rfm_scan_run: H2D copy failed");
     d_cap = s->d_cap;
   }
   // 1. spectrum
   const uint64_t n_seg = (n - kScanN) / kScanHop + 1;
   const uint64_t rows = (n_seg + kScanSegsPerCta - 1) / kScanSegsPerCta;
   if (rows > 0x7FFFFFFFull)
-    return ScanFail(RFM_ERR_INVALID, "rfm_scan_run_u8: capture too long");
+    return ScanFail(RFM_ERR_INVALID, "rfm_scan_run: capture too long");
   if (s->partial_rows < rows)
   {
     cudaFree(s->d_partial);
     s->d_partial = nullptr;
     s->partial_rows = 0;
     if (DevAlloc(&s->d_partial, (size_t)rows * kScanN) != cudaSuccess)
-      return ScanFail(RFM_ERR_CUDA, "rfm_scan_run_u8: partial-spectrum allocation failed");
+      return ScanFail(RFM_ERR_CUDA, "rfm_scan_run: partial-spectrum allocation failed");
     s->partial_rows = rows;
   }
-  rfm::EnsureDynSmem(k_scan_psd, kScanSmem);
   cudaEventRecord(s->ev[0], s->st);
-  k_scan_psd<<<(unsigned)rows, kScanThreads, kScanSmem, s->st>>>(reinterpret_cast<const unsigned short*>(d_cap), n_seg,
-                                                                 s->d_win, s->d_tw, s->d_partial);
+#define RFM_SCAN_PSD(F)                                                                                                 \
+  rfm::EnsureDynSmem(k_scan_psd<F>, kScanSmem);                                                                         \
+  k_scan_psd<F><<<(unsigned)rows, kScanThreads, kScanSmem, s->st>>>(                                                    \
+      reinterpret_cast<const typename ScanIn<F>::T*>(d_cap), n_seg, s->d_win, s->d_tw, s->d_partial)
+  switch (format)
+  {
+    case RFM_IQ_U8: RFM_SCAN_PSD(rfm::kIqU8); break;
+    case RFM_IQ_S8: RFM_SCAN_PSD(rfm::kIqS8); break;
+    case RFM_IQ_S16: RFM_SCAN_PSD(rfm::kIqS16); break;
+    default: RFM_SCAN_PSD(rfm::kIqCF32); break;
+  }
+#undef RFM_SCAN_PSD
   k_scan_reduce<<<kScanN / kScanThreads, kScanThreads, 0, s->st>>>(s->d_partial, (unsigned)rows,
                                                                    (double)n_seg * (double)kScanN * s->sum_w2, s->d_psd);
   cudaEventRecord(s->ev[1], s->st);
@@ -565,7 +612,7 @@ int rfm_scan_run_u8(rfm_scan* s, const uint8_t* iq, uint64_t n, int iq_on_device
   // 3. confirmation over every whole call of the capture
   if (!cand.empty())
   {
-    const int rc = Confirm(s, d_cap, n / s->n_call, cand);
+    const int rc = Confirm(s, format, d_cap, n / s->n_call, cand);
     if (rc != RFM_OK)
     {
       s->stations.clear();

@@ -1,4 +1,4 @@
-"""Wideband front end (SURVEY.md section 8d C5 / 8f N3): S stations of ONE shared u8 capture, each mixed to baseband,
+"""Wideband front end (SURVEY.md section 8d C5 / 8f N3): S stations of ONE shared capture, each mixed to baseband,
 decimated by CRDSDownConvert's SetWfmDataRate chain (7 x HB51 at 50 MS/s -> 390 625 S/s) and demodulated by a
 cFmDecoder(390625, 0, 48000, 15000, downsample = 1) -- all on the device, composed from the C-ABI primitives through
 device pointers.  Host logic only; the arithmetic lives in libradiofm_b200.so.
@@ -15,19 +15,25 @@ Two mixers, both reference classes:
               one fused kernel per call, nothing intermediate in HBM.
   "freqshift_unfused"  the same arithmetic as separate primitive calls (64 x rfm_freqshift + one rfm_downconvert over
               an S x 2 M complex buffer); kept as a cross-check of the primitives' device entry points.
+
+The capture is u8 (RTL-SDR) by default; input_format = "s8" (HackRF), "s16" (the SoapySDR / UHD host format) or "cf32"
+takes the other rfm_iq_format formats, converted inside the first kernel that reads the capture.
 """
 from __future__ import annotations
 
 import numpy as np
 
-from . import DownConvertBatch, FmDecoderBatch, FreqShiftBatch
+from . import DownConvertBatch, FmDecoderBatch, FreqShiftBatch, iq_format, iq_format_bytes
 
 
 class WidebandReceiver:
     def __init__(self, torch, station_freqs, fs: float = 50.0e6, front_block: int = 32000, blocks_per_call: int = 64,
-                 mixer: str = "osc", max_bw: float = 100000.0, device: int = 0, lanes_sms: int = 8, n_slots: int = 3):
+                 mixer: str = "osc", max_bw: float = 100000.0, device: int = 0, lanes_sms: int = 8, n_slots: int = 3,
+                 input_format="u8"):
         assert mixer in ("osc", "freqshift", "freqshift_unfused")
         self.torch, self.mixer, self.fs = torch, mixer, fs
+        self._fmt = iq_format(input_format)
+        self._esz = iq_format_bytes(self._fmt)
         self.freqs = np.ascontiguousarray(station_freqs, dtype=np.float64)
         self.S = S = self.freqs.size
         self.front_block, self.blocks_per_call = front_block, blocks_per_call
@@ -77,7 +83,8 @@ class WidebandReceiver:
                 o.close()
 
     def process_device(self, d_capture_ptr: int) -> int:
-        """One call = blocks_per_call front-end blocks of the shared capture (u8 [n_call][2] at d_capture_ptr, ready on the
+        """One call = blocks_per_call front-end blocks of the shared capture ([n_call] samples of the input format at
+        d_capture_ptr, aligned to the sample size, ready on the
         current stream).  Only enqueues; returns the audio floats per station that self.audio (this call's slot) will hold
         once wait() has ordered the current stream after the call."""
         torch = self.torch
@@ -88,12 +95,14 @@ class WidebandReceiver:
             self.s_front.wait_event(self.ev[slot])            # the slot's previous call has left the demodulator
         bb, audio = self.bbs[slot], self.audios[slot]
         if self.mixer in ("osc", "freqshift"):
-            m = self.dc.process_device(1, d_capture_ptr, self.n_call, bb.data_ptr(), self.n_bb, self.n_call, sf)
+            m = self.dc.process_iq_device(self._fmt, True, d_capture_ptr, self.n_call, bb.data_ptr(), self.n_bb,
+                                          self.n_call, sf)
         else:
             for b in range(self.blocks_per_call):
                 self.shift.reset()
-                self.shift.process_device(1, d_capture_ptr + 2 * b * self.front_block, self.front_block,
-                                          self.mixed.data_ptr() + 8 * b * self.front_block, self.n_call, self.front_block)
+                self.shift.process_iq_device(self._fmt, True, d_capture_ptr + self._esz * b * self.front_block,
+                                             self.front_block, self.mixed.data_ptr() + 8 * b * self.front_block,
+                                             self.n_call, self.front_block)
             self.s_front.wait_stream(torch.cuda.default_stream())
             m = self.dc.process_device(0, self.mixed.data_ptr(), self.n_call, bb.data_ptr(), self.n_bb, self.n_call, sf)
         assert m == self.n_bb
@@ -121,6 +130,21 @@ class WidebandReceiver:
         """Host convenience: capture [n_call, 2] uint8 -> audio [S, floats]."""
         torch = self.torch
         cap = torch.from_numpy(np.ascontiguousarray(capture_u8, dtype=np.uint8).reshape(self.n_call, 2)).to(self.bb.device)
+        k = self.process_device(cap.data_ptr())
+        self.wait()
+        torch.cuda.synchronize()
+        return self.audio[:, :k].cpu().numpy()
+
+    def process_iq(self, capture: np.ndarray) -> np.ndarray:
+        """Host convenience: capture [n_call, 2] of the input format's dtype (uint8 / int8 / int16 / float32, or
+        [n_call] complex64 for cf32) -> audio [S, floats]."""
+        torch = self.torch
+        a = np.asarray(capture)
+        if a.dtype == np.complex64:
+            a = np.ascontiguousarray(a).view(np.float32)
+        if iq_format(a.dtype) != self._fmt:
+            raise ValueError(f"capture dtype {a.dtype} is not the receiver's input format")
+        cap = torch.from_numpy(np.ascontiguousarray(a).reshape(self.n_call, 2)).to(self.bb.device)
         k = self.process_device(cap.data_ptr())
         self.wait()
         torch.cuda.synchronize()
