@@ -52,6 +52,30 @@ typedef enum rfm_iq_format { RFM_IQ_U8 = 0, RFM_IQ_S8 = 1, RFM_IQ_S16 = 2, RFM_I
 /* bytes per complex sample: 2, 2, 4, 8; 0 for an unknown format */
 RFM_API uint32_t rfm_iq_format_bytes(int format);
 
+/* IQ correction: the DC offset and the IQ gain / phase imbalance of a zero-IF receiver (HackRF, bladeRF, E4000 tuners),
+ * frequency-flat, one set of coefficients per capture.  Off by default everywhere.
+ *   Application  right after the format conversion, in float32, each step rounded on its own (no contraction):
+ *                r = I - dc_i, q = Q - dc_q, y = r + j (a q + b r).  Before the pre-mix table and the NCO.
+ *   Estimate     (rfm_iq_estimate) means m_I, m_Q and centred moments v_I, v_Q, c = E[I0 Q0] of the capture;
+ *                dc = (m_I, m_Q), a = sqrt(v_I / (v_Q - c^2 / v_I)), b = -a c / v_I (Gram-Schmidt: y is proper, its
+ *                real and imaginary parts uncorrelated with equal power).  Every value is computed in double and rounded
+ *                to float once.  v_I = 0 or v_I v_Q - c^2 <= 0 (or a non-finite result): a = 1, b = 0,
+ *                imbalance_valid = 0.  u8 / s8 / s16: 64-bit integer sums of codes, squares and cross products, centred
+ *                moments n S_xx - S_x S_y in 128-bit integers, then scaled -- bit-identical on any device and work
+ *                split; n <= 2^32.  cf32: double sums in an order that depends on n only.  oracle/iqcorr.py restates
+ *                both.
+ * Not covered: the decoder's own front end (rfm_decoder_*), frequency-dependent imbalance, tracking over time. */
+typedef struct rfm_iq_correction
+{
+  float dc_i, dc_q;         /* subtracted after the format conversion */
+  float a, b;               /* y = (I - dc_i) + j (a (Q - dc_q) + b (I - dc_i)) */
+  int32_t imbalance_valid;  /* 0: a = 1, b = 0 were forced (degenerate statistics) */
+} rfm_iq_correction;
+/* One pass over n samples of `format`, in host memory (copied to `device`) or device memory (complete before the call,
+ * aligned to the sample size).  Blocking.  RFM_ERR_INVALID for an unknown format, a misaligned device pointer, n = 0 or
+ * n > 2^32, with the reason in rfm_last_error().  device: -1 = current. */
+RFM_API int rfm_iq_estimate(int format, const void* iq, uint64_t n, int iq_on_device, int device, rfm_iq_correction* out);
+
 RFM_API const char* rfm_last_error(void);
 RFM_API const char* rfm_version(void);
 /* number of kernels this library has launched in this process (bench.py "gpu_launches") */
@@ -239,6 +263,9 @@ RFM_API int rfm_freqshift_process_iq(rfm_freqshift* f, int format, int shared_ca
 RFM_API int rfm_freqshift_process_iq_device(rfm_freqshift* f, int format, int shared_capture, const void* d_in,
                                             size_t in_stride, float* d_out, size_t out_stride, uint32_t n,
                                             void* cuda_stream);
+/* IQ correction (rfm_iq_correction) of every input sample of every later process call, of every row; NULL = off (the
+ * default).  Non-finite coefficients: RFM_ERR_INVALID. */
+RFM_API int rfm_freqshift_set_iq_correction(rfm_freqshift* f, const rfm_iq_correction* c);
 
 /* ------------------------------------------------------------------------------------------------
  * CRDSDownConvert (DownConvert.h:68-169, DownConvert.cpp:271-489), batched over rows: NCO_OSC mixer (the
@@ -288,6 +315,9 @@ RFM_API int rfm_downconvert_process_iq(rfm_downconvert* d, int format, int share
 RFM_API int rfm_downconvert_process_iq_device(rfm_downconvert* d, int format, int shared_capture, const void* d_in,
                                               size_t in_stride, float* d_out, size_t out_stride, uint32_t n,
                                               uint32_t* n_out, void* cuda_stream);
+/* IQ correction (rfm_iq_correction) of every input sample of every later process call, of every row, before the
+ * pre-mix table and the NCO; NULL = off (the default).  Non-finite coefficients: RFM_ERR_INVALID. */
+RFM_API int rfm_downconvert_set_iq_correction(rfm_downconvert* d, const rfm_iq_correction* c);
 
 /* ------------------------------------------------------------------------------------------------
  * cDownsampleFilter (DownConvert.h:21-60, DownConvert.cpp:58-256), batched over rows: Lanczos-windowed sinc FIR with
@@ -556,6 +586,13 @@ RFM_API int rfm_scan_stations(rfm_scan* s, rfm_scan_station* out, uint32_t max, 
 /* Device time of the last run's two stages (CUDA events): the spectrum kernels, and the confirmation from the first
  * front-end launch to the end of the last demodulator call (0 without candidates). */
 RFM_API int rfm_scan_timing(rfm_scan* s, double* spectrum_ms, double* confirm_ms);
+/* IQ correction of later runs (rfm_iq_correction): mode 0 off (the default), 1 estimate from each run's capture (one
+ * statistics pass before the spectrum; the capture must then hold at most 2^32 samples), 2 use `fixed` (copied).  The
+ * spectrum is that of the corrected samples and the confirmation's rfm_downconvert rows carry the same correction.
+ * RFM_ERR_INVALID for an unknown mode, a NULL `fixed` with mode 2 or non-finite coefficients. */
+RFM_API int rfm_scan_set_iq_correction(rfm_scan* s, int mode, const rfm_iq_correction* fixed);
+/* What the last run applied; mode 0: {0, 0, 1, 0, imbalance_valid = 0} */
+RFM_API int rfm_scan_iq_correction(rfm_scan* s, rfm_iq_correction* out);
 
 #ifdef __cplusplus
 }

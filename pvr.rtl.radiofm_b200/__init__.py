@@ -11,6 +11,7 @@ __graft_entry__.py.
 from __future__ import annotations
 
 import ctypes as C
+import dataclasses
 import os
 import subprocess
 
@@ -77,6 +78,8 @@ EXPORTED_SYMBOLS = (
     "rfm_iq_format_bytes", "rfm_decoder_process_iq", "rfm_decoder_submit_iq", "rfm_decoder_process_iq_device",
     "rfm_freqshift_process_iq", "rfm_freqshift_process_iq_device", "rfm_downconvert_process_iq",
     "rfm_downconvert_process_iq_device", "rfm_scan_run",
+    "rfm_iq_estimate", "rfm_downconvert_set_iq_correction", "rfm_freqshift_set_iq_correction",
+    "rfm_scan_set_iq_correction", "rfm_scan_iq_correction",
 )
 
 # rfm_iq_format (include/radiofm_b200.h): interleaved I,Q; s8 = v * 2^-7, s16 = v * 2^-15 (exact), full scale of the container
@@ -119,6 +122,62 @@ def _iq_host(iq, rows: int | None = None):
     fmt = iq_format(a.dtype)
     a = np.ascontiguousarray(a, dtype=_IQ_DTYPES[fmt])
     return fmt, (a.reshape(rows, -1, 2) if rows else a.reshape(-1, 2))
+
+
+class RfmIqCorrection(C.Structure):
+    """rfm_iq_correction (include/radiofm_b200.h)."""
+    _fields_ = [("dc_i", C.c_float), ("dc_q", C.c_float), ("a", C.c_float), ("b", C.c_float),
+                ("imbalance_valid", C.c_int32)]
+
+
+@dataclasses.dataclass(frozen=True)
+class IqCorrection:
+    """Frequency-flat IQ correction of a capture (rfm_iq_correction): y = (I - dc_i) + j (a (Q - dc_q) + b (I - dc_i)),
+    in float32 after the format conversion.  imbalance_valid False: a = 1, b = 0 were forced (degenerate statistics)."""
+    dc_i: np.float32
+    dc_q: np.float32
+    a: np.float32 = np.float32(1.0)
+    b: np.float32 = np.float32(0.0)
+    imbalance_valid: bool = True
+
+    def _c(self) -> RfmIqCorrection:
+        return RfmIqCorrection(float(np.float32(self.dc_i)), float(np.float32(self.dc_q)), float(np.float32(self.a)),
+                               float(np.float32(self.b)), int(bool(self.imbalance_valid)))
+
+    @staticmethod
+    def _from_c(c: RfmIqCorrection) -> "IqCorrection":
+        return IqCorrection(np.float32(c.dc_i), np.float32(c.dc_q), np.float32(c.a), np.float32(c.b),
+                            bool(c.imbalance_valid))
+
+
+def _corr_arg(c):
+    if c is None:
+        return None
+    if not isinstance(c, IqCorrection):
+        raise TypeError(f"expected an IqCorrection or None, got {type(c).__name__}")
+    return C.byref(c._c())
+
+
+def estimate_iq_correction(capture, fmt=None, n: int | None = None, device: int = -1) -> IqCorrection:
+    """rfm_iq_estimate: the blind DC / gain / phase estimate of one capture.  capture: a host array [n, 2] of uint8 /
+    int8 / int16 / float32 ([n] complex64), a contiguous CUDA tensor of those dtypes (complete before the call), or a
+    device pointer (int) with its format and sample count."""
+    out = RfmIqCorrection()
+    if isinstance(capture, (int, np.integer)):
+        if fmt is None or n is None:
+            raise ValueError("a device pointer needs fmt and n")
+        _check(lib().rfm_iq_estimate(iq_format(fmt), C.c_void_p(int(capture)), int(n), 1, device, C.byref(out)))
+    elif hasattr(capture, "data_ptr") and getattr(capture, "is_cuda", False):
+        f = iq_format(capture.dtype)
+        if not capture.is_contiguous():
+            raise ValueError("device capture must be contiguous")
+        cnt = capture.numel() // (1 if f == IQ_CF32 and capture.is_complex() else 2)
+        dev = capture.device.index if device < 0 and capture.device.index is not None else device
+        _check(lib().rfm_iq_estimate(f, C.c_void_p(capture.data_ptr()), cnt, 1, dev, C.byref(out)))
+    else:
+        f, cap = _iq_host(capture)
+        _check(lib().rfm_iq_estimate(f, cap.ctypes.data_as(C.c_void_p), cap.shape[0], 0, device, C.byref(out)))
+    return IqCorrection._from_c(out)
 
 
 _ADD_FRAME_CB = C.CFUNCTYPE(C.c_int, C.c_void_p, C.POINTER(C.c_uint8), C.c_uint32)
@@ -326,6 +385,11 @@ def lib():
         L.rfm_downconvert_process_iq_device.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p,
                                                         C.c_size_t, C.c_uint32, _u32p, C.c_void_p]
         L.rfm_scan_run.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.c_int]
+        L.rfm_iq_estimate.argtypes = [C.c_int, C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.POINTER(RfmIqCorrection)]
+        L.rfm_downconvert_set_iq_correction.argtypes = [C.c_void_p, C.POINTER(RfmIqCorrection)]
+        L.rfm_freqshift_set_iq_correction.argtypes = [C.c_void_p, C.POINTER(RfmIqCorrection)]
+        L.rfm_scan_set_iq_correction.argtypes = [C.c_void_p, C.c_int, C.POINTER(RfmIqCorrection)]
+        L.rfm_scan_iq_correction.argtypes = [C.c_void_p, C.POINTER(RfmIqCorrection)]
         L.rfm_rds_check_block.restype = C.c_uint32
         L.rfm_rds_check_block.argtypes = [C.c_uint32, C.c_uint32, C.c_int, _u32p]
         _lib = L
@@ -796,6 +860,10 @@ class FreqShiftBatch:
                                                      in_stride, C.c_void_p(d_out_ptr), out_stride, n,
                                                      C.c_void_p(cuda_stream)))
 
+    def set_iq_correction(self, c: IqCorrection | None):
+        """IQ correction of every later process call (None = off)."""
+        _check(lib().rfm_freqshift_set_iq_correction(self._h, _corr_arg(c)))
+
     def process_device(self, mode: int, d_in_ptr: int, in_stride: int, d_out_ptr: int, out_stride: int, n: int,
                        cuda_stream: int = 0):
         _check(lib().rfm_freqshift_process_device(self._h, mode, C.c_void_p(d_in_ptr), in_stride, C.c_void_p(d_out_ptr),
@@ -835,6 +903,10 @@ class DownConvertBatch:
         """Device table [rows][row_stride] float2 of a cFreqShift that is Reset() every `period` samples (0 = off)."""
         _check(lib().rfm_downconvert_set_premix(self._h, C.c_void_p(d_table_ptr) if d_table_ptr else None, row_stride,
                                                 period))
+
+    def set_iq_correction(self, c: IqCorrection | None):
+        """IQ correction of every later process call, before the pre-mix table and the NCO (None = off)."""
+        _check(lib().rfm_downconvert_set_iq_correction(self._h, _corr_arg(c)))
 
     def process_cf32(self, iq: np.ndarray) -> np.ndarray:
         iq = np.ascontiguousarray(iq, dtype=np.float32).reshape(self.rows, -1, 2)
@@ -1062,11 +1134,29 @@ class BandScan:
     auto-scan (ChannelSettings.cpp:96-147) for all channels at once."""
 
     def __init__(self, fs: float, raster_first: float, raster_step: float, raster_count: int, min_snr_db: float = 10.0,
-                 device: int = -1):
+                 device: int = -1, iq_correction=None):
         cfg = scan_config(fs, raster_first, raster_step, raster_count, min_snr_db, device)
         self.raster_count = raster_count
         self._h = C.c_void_p()
         _check(lib().rfm_scan_create(C.byref(cfg), C.byref(self._h)))
+        self.set_iq_correction(iq_correction)
+
+    def set_iq_correction(self, c):
+        """IQ correction of later runs: None (off), "estimate" (from each run's capture) or a fixed IqCorrection."""
+        if c is None:
+            _check(lib().rfm_scan_set_iq_correction(self._h, 0, None))
+        elif isinstance(c, str):
+            if c != "estimate":
+                raise ValueError(f"unknown IQ correction mode {c!r}: use None, \"estimate\" or an IqCorrection")
+            _check(lib().rfm_scan_set_iq_correction(self._h, 1, None))
+        else:
+            _check(lib().rfm_scan_set_iq_correction(self._h, 2, _corr_arg(c)))
+
+    def iq_correction(self) -> IqCorrection:
+        """The correction the last run applied (identity with imbalance_valid False when off)."""
+        out = RfmIqCorrection()
+        _check(lib().rfm_scan_iq_correction(self._h, C.byref(out)))
+        return IqCorrection._from_c(out)
 
     def close(self):
         if getattr(self, "_h", None):

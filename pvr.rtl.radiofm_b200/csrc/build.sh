@@ -19,7 +19,7 @@ NVFLAGS="$ARCH -O3 -std=c++17 -lineinfo -fmad=false $DEFS -Xcompiler -fPIC,-fvis
 CXXFLAGS="-O2 -std=c++17 -fPIC -fvisibility=hidden -ffp-contract=off $DEFS"
 mkdir -p $B
 pids=""
-for f in rfm_kernels rfm_api rfm_probe rfm_freqshift rfm_downconvert rfm_primitives rfm_scan; do
+for f in rfm_kernels rfm_api rfm_probe rfm_freqshift rfm_downconvert rfm_primitives rfm_scan rfm_iqcorr; do
   $NVCC $NVFLAGS -c $f.cu -o $B/$f.o &
   pids="$pids $!"
 done
@@ -32,5 +32,5 @@ pids="$pids $!"
 for p in $pids; do
   wait $p
 done
-$NVCC $ARCH -shared -o $OUT $B/rfm_kernels.o $B/rfm_api.o $B/rfm_probe.o $B/rfm_freqshift.o $B/rfm_downconvert.o $B/rfm_primitives.o $B/rfm_scan.o $B/rfm_plan.o $B/rfm_rdssync.o $B/rfm_rdsgroup.o $B/rfm_source.o $B/rfm_demux.o -lcudart_static -lpthread -ldl -lrt
+$NVCC $ARCH -shared -o $OUT $B/rfm_kernels.o $B/rfm_api.o $B/rfm_probe.o $B/rfm_freqshift.o $B/rfm_downconvert.o $B/rfm_primitives.o $B/rfm_scan.o $B/rfm_iqcorr.o $B/rfm_plan.o $B/rfm_rdssync.o $B/rfm_rdsgroup.o $B/rfm_source.o $B/rfm_demux.o -lcudart_static -lpthread -ldl -lrt
 echo "built $(readlink -f $OUT)"

@@ -19,6 +19,7 @@
 // 2 * (taps - 1) samples per call -- the reference itself silently mis-filters shorter / odd inputs (its in-place
 // stages overwrite the samples they later copy into their delay line, DownConvert.cpp:519-520,544-547).
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdint.h>
 #include <string.h>
 
@@ -87,7 +88,7 @@ struct DcParams
 
 // F: IqFormat.  A shared cf32 capture is read as rows of stride 0 (no instantiation of its own).
 template <int F, bool SHARED>
-__device__ __forceinline__ float2 dc_load(const DcParams& p, unsigned row, unsigned i)
+__device__ __forceinline__ float2 dc_convert(const DcParams& p, unsigned row, unsigned i)
 {
   if (F == kIqCF32)
     return reinterpret_cast<const float2*>(p.in)[(size_t)row * p.in_stride + i];
@@ -101,6 +102,14 @@ __device__ __forceinline__ float2 dc_load(const DcParams& p, unsigned row, unsig
   return make_float2(rfm_iq8_to_float<F>(w, 0u), rfm_iq8_to_float<F>(w, 1u));
 }
 
+// CORR: the IQ correction follows the conversion (rfm_iq_correct)
+template <int F, bool SHARED, bool CORR>
+__device__ __forceinline__ float2 dc_load(const DcParams& p, const IqCorr& corr, unsigned row, unsigned i)
+{
+  const float2 x = dc_convert<F, SHARED>(p, row, i);
+  return CORR ? rfm_iq_correct(x, corr) : x;
+}
+
 // DownConvert.cpp:464-465 (and FreqShift.cpp:63-69: the same four products, one subtraction, one addition)
 __device__ __forceinline__ float2 dc_mix(float2 d, float2 o)
 {
@@ -111,10 +120,11 @@ __device__ __forceinline__ float2 dc_mix(float2 d, float2 o)
 }
 
 // input sample i of this call for `row`, pre-mixed if a table is set, times the NCO phasor
-template <int F, bool SHARED>
-__device__ __forceinline__ float2 dc_sample(const DcParams& p, const float2* osc, unsigned row, unsigned i)
+template <int F, bool SHARED, bool CORR>
+__device__ __forceinline__ float2 dc_sample(const DcParams& p, const IqCorr& corr, const float2* osc, unsigned row,
+                                            unsigned i)
 {
-  float2 d = dc_load<F, SHARED>(p, row, i);
+  float2 d = dc_load<F, SHARED, CORR>(p, corr, row, i);
   if (p.pre)
     d = dc_mix(d, p.pre[(size_t)row * p.pre_stride + (p.pre_pos + i) % p.pre_period]);
   return dc_mix(d, osc[i]);
@@ -263,8 +273,8 @@ __global__ void __launch_bounds__(256) k_dc_osc_fill(float2* table, size_t strid
 // --------------------------------------------------------------------------------------------------
 // generic chain: any stage kinds, interleaved V buffers (the k_rds_front scheme without the LP)
 // --------------------------------------------------------------------------------------------------
-template <int F, bool SHARED>
-__global__ void __launch_bounds__(kDcThreads) k_dc_chain(DcParams p)
+template <int F, bool SHARED, bool CORR>
+__global__ void __launch_bounds__(kDcThreads) k_dc_chain(DcParams p, IqCorr corr)
 {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* s_h = reinterpret_cast<float*>(smem_raw);
@@ -308,7 +318,7 @@ __global__ void __launch_bounds__(kDcThreads) k_dc_chain(DcParams p)
     const bool store = pos >= c_lo;
     const unsigned tn = min(kDcTileGeneric, (store ? c_hi : c_lo) - pos);
     for (unsigned i = tid; i < tn; i += kDcThreads)
-      B[0][p.st[0].hist + i] = dc_sample<F, SHARED>(p, osc, row, pos + i);
+      B[0][p.st[0].hist + i] = dc_sample<F, SHARED, CORR>(p, corr, osc, row, pos + i);
     __syncthreads();
     unsigned n = tn;
     for (unsigned k = 0; k < p.nst; ++k)
@@ -382,8 +392,8 @@ __device__ __forceinline__ void dc_stage(const DcTapsPk<L>& taps, const float2* 
   }
 }
 
-template <int F, bool SHARED, int L>
-__global__ void __launch_bounds__(kDcThreadsFast) k_dc_chain_uniform(DcParams p, DcTapsPk<L> taps)
+template <int F, bool SHARED, int L, bool CORR>
+__global__ void __launch_bounds__(kDcThreadsFast) k_dc_chain_uniform(DcParams p, DcTapsPk<L> taps, IqCorr corr)
 {
   constexpr int R = 5;                 // largest group: sizes the slack behind each buffer
   constexpr unsigned HH = (L - 1) / 2; // history entries in each of E and O
@@ -435,7 +445,7 @@ __global__ void __launch_bounds__(kDcThreadsFast) k_dc_chain_uniform(DcParams p,
       unsigned pi = (unsigned)(((unsigned long long)p.pre_pos + pos + tid) % p.pre_period);
       for (unsigned i = tid; i < tn; i += kDcThreadsFast)
       {
-        const float2 d = dc_mix(dc_load<F, SHARED>(p, row, pos + i), pre[pi]);
+        const float2 d = dc_mix(dc_load<F, SHARED, CORR>(p, corr, row, pos + i), pre[pi]);
         ((i & 1u) ? O_(0) : E_(0))[HH + (i >> 1)] = dc_mix(d, osc[pos + i]);
         pi += step;
         pi = pi >= p.pre_period ? pi - p.pre_period : pi;
@@ -443,7 +453,7 @@ __global__ void __launch_bounds__(kDcThreadsFast) k_dc_chain_uniform(DcParams p,
     }
     else
       for (unsigned i = tid; i < tn; i += kDcThreadsFast)
-        ((i & 1u) ? O_(0) : E_(0))[HH + (i >> 1)] = dc_sample<F, SHARED>(p, osc, row, pos + i);
+        ((i & 1u) ? O_(0) : E_(0))[HH + (i >> 1)] = dc_sample<F, SHARED, CORR>(p, corr, osc, row, pos + i);
     __syncthreads();
     // operands of the next tile on their way into L2 while this one is filtered
     {
@@ -545,6 +555,8 @@ struct rfm_downconvert
   uint8_t* d_raw = nullptr;   // u8 / s8 / s16 input, raw_bytes
   size_t raw_bytes = 0;
   DcTaps<51> taps51;
+  bool corr_on = false;      // rfm_downconvert_set_iq_correction
+  IqCorr corr = {0.f, 0.f, 1.f, 0.f};
 };
 
 namespace
@@ -585,7 +597,7 @@ int ResetState(rfm_downconvert* d)
   return ok ? RFM_OK : DcFail(RFM_ERR_CUDA, "rfm_downconvert: state reset failed");
 }
 
-template <int F, bool SHARED>
+template <int F, bool SHARED, bool CORR>
 void LaunchChain(rfm_downconvert* d, const DcParams& p, cudaStream_t st)
 {
   dim3 grid(p.nchunks, p.rows);
@@ -598,8 +610,8 @@ void LaunchChain(rfm_downconvert* d, const DcParams& p, cudaStream_t st)
       smem += 2 * (size_t)(25 + n / 2 + 5) * sizeof(float2);
       n >>= 1;
     }
-    EnsureDynSmem(k_dc_chain_uniform<F, SHARED, 51>, smem);
-    k_dc_chain_uniform<F, SHARED, 51><<<grid, kDcThreadsFast, smem, st>>>(p, MakeDcTapsPk(d->taps51));
+    EnsureDynSmem(k_dc_chain_uniform<F, SHARED, 51, CORR>, smem);
+    k_dc_chain_uniform<F, SHARED, 51, CORR><<<grid, kDcThreadsFast, smem, st>>>(p, MakeDcTapsPk(d->taps51), d->corr);
   }
   else
   {
@@ -612,9 +624,18 @@ void LaunchChain(rfm_downconvert* d, const DcParams& p, cudaStream_t st)
       n >>= 1;
     }
     const size_t smem = floats * sizeof(float) + f2 * sizeof(float2);
-    EnsureDynSmem(k_dc_chain<F, SHARED>, smem);
-    k_dc_chain<F, SHARED><<<grid, kDcThreads, smem, st>>>(p);
+    EnsureDynSmem(k_dc_chain<F, SHARED, CORR>, smem);
+    k_dc_chain<F, SHARED, CORR><<<grid, kDcThreads, smem, st>>>(p, d->corr);
   }
+}
+
+template <int F, bool SHARED>
+void LaunchChain(rfm_downconvert* d, const DcParams& p, cudaStream_t st)
+{
+  if (d->corr_on)
+    LaunchChain<F, SHARED, true>(d, p, st);
+  else
+    LaunchChain<F, SHARED, false>(d, p, st);
 }
 
 // fmt: IqFormat; shared: one capture for every row (a shared cf32 capture is read as rows of stride 0)
@@ -843,6 +864,17 @@ int rfm_downconvert_set_premix(rfm_downconvert* d, const float* d_table, size_t 
   d->pre_stride = row_stride;
   d->pre_period = d_table ? period : 0;
   d->pre_pos = 0;
+  return RFM_OK;
+}
+
+int rfm_downconvert_set_iq_correction(rfm_downconvert* d, const rfm_iq_correction* c)
+{
+  if (!d)
+    return DcFail(RFM_ERR_INVALID, "rfm_downconvert_set_iq_correction: null handle");
+  if (c && !(isfinite(c->dc_i) && isfinite(c->dc_q) && isfinite(c->a) && isfinite(c->b)))
+    return DcFail(RFM_ERR_INVALID, "rfm_downconvert_set_iq_correction: coefficients must be finite");
+  d->corr_on = c != nullptr;
+  d->corr = c ? IqCorr{c->dc_i, c->dc_q, c->a, c->b} : IqCorr{0.f, 0.f, 1.f, 0.f};
   return RFM_OK;
 }
 

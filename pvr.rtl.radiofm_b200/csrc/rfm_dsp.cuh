@@ -52,6 +52,21 @@ __device__ __forceinline__ float rfm_iq8_to_float(unsigned word, unsigned byte_s
   return F == kIqS8 ? rfm_s8_to_float(word, byte_sel) : rfm_u8_to_float(word, byte_sel);
 }
 
+// Frequency-flat IQ correction (rfm_iq_correction, include/radiofm_b200.h), applied right after the format conversion:
+// r = I - dc_i, q = Q - dc_q, y = r + j (a q + b r).  Two products and one sum, each rounded on its own, so a float32
+// restatement on the host (oracle/iqcorr.py) is bit-exact.  Passed to the kernels by value, never re-read from memory.
+struct IqCorr
+{
+  float dc_i, dc_q, a, b;
+};
+
+__device__ __forceinline__ float2 rfm_iq_correct(float2 x, const IqCorr& c)
+{
+  const float r = subf(x.x, c.dc_i);
+  const float q = subf(x.y, c.dc_q);
+  return make_float2(r, addf(mulf(c.a, q), mulf(c.b, r)));
+}
+
 // OscGn = 1.95 - (re^2 + im^2) of the NCO_OSC rotating vector (DownConvert.cpp:441): the double literal makes it
 // float(1.95 - double(q)).  For q in [0.5, 1.69] -- the oscillator's amplitude never leaves it -- the same value comes
 // out of five dependent float additions: s + e = 1.95f - q exactly (Fast2Sum), then the low part of the constant,

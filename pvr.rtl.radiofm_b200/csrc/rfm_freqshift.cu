@@ -8,6 +8,7 @@
 // mixing itself -- sin/cos of the phase (== x87 fsincos rounded to float, rfm_math.cuh), complex multiply with
 // individually rounded products (4 mul, 2 add) -- runs fully parallel (k_fs_mix).
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdint.h>
 
 #include <string>
@@ -54,10 +55,10 @@ __global__ void __launch_bounds__(32) k_fs_phase(const float* inc, float* time, 
 }
 
 // F: IqFormat of the input rows (cf32 rows may be mixed in place), or of one capture shared by every row (SHARED; a
-// shared cf32 capture is read as rows of stride 0)
-template <int F, bool SHARED>
+// shared cf32 capture is read as rows of stride 0).  CORR: the IQ correction follows the conversion (rfm_iq_correct).
+template <int F, bool SHARED, bool CORR>
 __global__ void __launch_bounds__(256) k_fs_mix(const float* ph, size_t ph_stride, const void* in, size_t in_stride,
-                                                float2* out, size_t out_stride, unsigned n, const float* lut)
+                                                float2* out, size_t out_stride, unsigned n, const float* lut, IqCorr corr)
 {
   const unsigned i = blockIdx.x * 256 + threadIdx.x;
   const unsigned r = blockIdx.y;
@@ -83,6 +84,8 @@ __global__ void __launch_bounds__(256) k_fs_mix(const float* ph, size_t ph_strid
     const unsigned w = reinterpret_cast<const unsigned*>(in)[(SHARED ? 0 : (size_t)r * in_stride) + i];
     d = make_float2(rfm_s16_to_float(w, 0u), rfm_s16_to_float(w, 1u));
   }
+  if (CORR)
+    d = rfm_iq_correct(d, corr);
   float2 o;
   o.x = subf(mulf(d.x, c), mulf(d.y, s)); // FreqShift.cpp:63-69
   o.y = addf(mulf(d.x, s), mulf(d.y, c));
@@ -103,6 +106,8 @@ struct rfm_freqshift
   uint8_t* d_raw = nullptr;   // host input of the _iq / _u8 calls, raw_bytes
   size_t raw_bytes = 0;
   std::string err;
+  bool corr_on = false;      // rfm_freqshift_set_iq_correction
+  IqCorr corr = {0.f, 0.f, 1.f, 0.f};
 };
 
 extern "C"
@@ -185,16 +190,36 @@ static int Run(rfm_freqshift* f, int fmt, bool shared, const void* d_in, size_t 
   }
   f->at_zero = false;
   dim3 grid((n + 255) / 256, f->rows);
-#define RFM_FS_MIX(F, SHARED) k_fs_mix<F, SHARED><<<grid, 256, 0, st>>>(f->d_ph, f->cap, d_in, in_stride, d_out, out_stride, n, f->d_lut)
+#define RFM_FS_MIX(F, SHARED)                                                                                          \
+  if (f->corr_on)                                                                                                      \
+    k_fs_mix<F, SHARED, true><<<grid, 256, 0, st>>>(f->d_ph, f->cap, d_in, in_stride, d_out, out_stride, n, f->d_lut,   \
+                                                    f->corr);                                                          \
+  else                                                                                                                 \
+    k_fs_mix<F, SHARED, false><<<grid, 256, 0, st>>>(f->d_ph, f->cap, d_in, in_stride, d_out, out_stride, n, f->d_lut,  \
+                                                     f->corr)
   switch (fmt)
   {
-    case kIqU8: if (shared) RFM_FS_MIX(kIqU8, true); else RFM_FS_MIX(kIqU8, false); break;
-    case kIqS8: if (shared) RFM_FS_MIX(kIqS8, true); else RFM_FS_MIX(kIqS8, false); break;
-    case kIqS16: if (shared) RFM_FS_MIX(kIqS16, true); else RFM_FS_MIX(kIqS16, false); break;
+    case kIqU8: if (shared) { RFM_FS_MIX(kIqU8, true); } else { RFM_FS_MIX(kIqU8, false); } break;
+    case kIqS8: if (shared) { RFM_FS_MIX(kIqS8, true); } else { RFM_FS_MIX(kIqS8, false); } break;
+    case kIqS16: if (shared) { RFM_FS_MIX(kIqS16, true); } else { RFM_FS_MIX(kIqS16, false); } break;
     default: in_stride = shared ? 0 : in_stride; RFM_FS_MIX(kIqCF32, false); break;
   }
 #undef RFM_FS_MIX
   return cudaGetLastError() == cudaSuccess ? RFM_OK : RFM_ERR_CUDA;
+}
+
+int rfm_freqshift_set_iq_correction(rfm_freqshift* f, const rfm_iq_correction* c)
+{
+  if (!f)
+    return RFM_ERR_INVALID;
+  if (c && !(isfinite(c->dc_i) && isfinite(c->dc_q) && isfinite(c->a) && isfinite(c->b)))
+  {
+    rfm::SetLastError("rfm_freqshift_set_iq_correction: coefficients must be finite");
+    return RFM_ERR_INVALID;
+  }
+  f->corr_on = c != nullptr;
+  f->corr = c ? IqCorr{c->dc_i, c->dc_q, c->a, c->b} : IqCorr{0.f, 0.f, 1.f, 0.f};
+  return RFM_OK;
 }
 
 int rfm_freqshift_process_cf32(rfm_freqshift* f, float* iq, uint32_t n)

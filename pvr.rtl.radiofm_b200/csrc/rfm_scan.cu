@@ -32,6 +32,8 @@ namespace rfm
 {
 extern std::atomic<uint64_t> g_launches;
 void SetLastError(const std::string& m);
+int IqEstimateDevice(int fmt, const void* d_in, uint64_t n, cudaStream_t st, rfm_iq_correction* out);  // rfm_iqcorr.cu
+int IqEstimateCheck(const char* who, int fmt, const void* iq, uint64_t n, bool on_device);
 }
 
 namespace
@@ -108,10 +110,11 @@ __device__ __forceinline__ float2 ScanSample(float2 v)
 
 // Partial Welch sums: CTA b transforms segments [b * 32, b * 32 + 32) of the capture (I,Q samples of format F; segment g
 // covers samples [g N/2, g N/2 + N)) and writes sum |X_g[k]|^2 over them, natural bin order, to partial[b][k].
-template <int F>
+// CORR: every sample is IQ-corrected (rfm_iq_correct) after its conversion, before the window.
+template <int F, bool CORR>
 __global__ void __launch_bounds__(kScanThreads) k_scan_psd(const typename ScanIn<F>::T* __restrict__ cap, uint64_t n_seg,
                                                            const float* __restrict__ win, const float2* __restrict__ tw,
-                                                           float* __restrict__ partial)
+                                                           float* __restrict__ partial, rfm::IqCorr corr)
 {
   extern __shared__ float2 scan_sm[];
   float2* A = scan_sm;
@@ -134,7 +137,14 @@ __global__ void __launch_bounds__(kScanThreads) k_scan_psd(const typename ScanIn
         const unsigned i = tid + j * kScanThreads;
         const unsigned w = __ldg(seg + i);
         const float h = __ldg(win + i);
-        A[i] = make_float2(h * rfm::rfm_iq8_to_float<F>(w, 0u), h * rfm::rfm_iq8_to_float<F>(w, 1u));
+        if constexpr (CORR)
+        {
+          const float2 x = rfm::rfm_iq_correct(
+              make_float2(rfm::rfm_iq8_to_float<F>(w, 0u), rfm::rfm_iq8_to_float<F>(w, 1u)), corr);
+          A[i] = make_float2(h * x.x, h * x.y);
+        }
+        else
+          A[i] = make_float2(h * rfm::rfm_iq8_to_float<F>(w, 0u), h * rfm::rfm_iq8_to_float<F>(w, 1u));
       }
     }
     else
@@ -144,7 +154,9 @@ __global__ void __launch_bounds__(kScanThreads) k_scan_psd(const typename ScanIn
       for (unsigned j = 0; j < kScanPerThread; ++j)
       {
         const unsigned i = tid + j * kScanThreads;
-        const float2 x = ScanSample(__ldg(seg + i));
+        float2 x = ScanSample(__ldg(seg + i));
+        if (CORR)
+          x = rfm::rfm_iq_correct(x, corr);
         const float h = __ldg(win + i);
         A[i] = make_float2(h * x.x, h * x.y);
       }
@@ -222,13 +234,17 @@ struct rfm_scan
   std::vector<double> chan;
   std::vector<rfm_scan_station> stations;
   double spectrum_ms = 0.0, confirm_ms = 0.0;
+  int corr_mode = 0;                      // rfm_scan_set_iq_correction
+  rfm_iq_correction corr_fixed = {0.f, 0.f, 1.f, 0.f, 0};
+  rfm_iq_correction corr_applied = {0.f, 0.f, 1.f, 0.f, 0};
 };
 
 namespace
 {
 // The candidates' receivers: one rfm_downconvert row and one rfm_decoder stream per candidate, `calls` calls of
 // n_call capture samples each, the front end on the decoder's companion stream, three baseband slots.
-int Confirm(rfm_scan* s, int fmt, const uint8_t* d_cap, uint64_t calls, const std::vector<uint32_t>& cand)
+int Confirm(rfm_scan* s, int fmt, const uint8_t* d_cap, uint64_t calls, const std::vector<uint32_t>& cand,
+            const rfm_iq_correction* corr)
 {
   const uint32_t M = (uint32_t)cand.size();
   std::vector<float> nco(M);
@@ -241,6 +257,8 @@ int Confirm(rfm_scan* s, int fmt, const uint8_t* d_cap, uint64_t calls, const st
   float2* bb[kScanSlots] = {};
   float* audio[kScanSlots] = {};
   int rc = rfm_downconvert_create(M, nco.data(), (float)s->cfg.sample_rate, kScanMaxBw, 1, s->n_call, s->device, &dc);
+  if (rc == RFM_OK)
+    rc = rfm_downconvert_set_iq_correction(dc, corr);
   size_t stride = 0;
   void* front = nullptr;
   if (rc == RFM_OK)
@@ -521,6 +539,12 @@ int rfm_scan_run(rfm_scan* s, int format, const void* iq, uint64_t n, int iq_on_
   if (iq_on_device && (reinterpret_cast<uintptr_t>(iq) % esz) != 0)
     return ScanFail(RFM_ERR_INVALID, "rfm_scan_run: device capture must be aligned to the sample size "
                                      "(2 / 2 / 4 / 8 bytes for u8 / s8 / s16 / cf32)");
+  if (s->corr_mode == 1)
+  {
+    const int rc = rfm::IqEstimateCheck("rfm_scan_run", format, iq, n, iq_on_device != 0);
+    if (rc != RFM_OK)
+      return rc;
+  }
   if (cudaSetDevice(s->device) != cudaSuccess)
     return ScanFail(RFM_ERR_CUDA, "cudaSetDevice failed");
   s->have = false;
@@ -555,10 +579,31 @@ int rfm_scan_run(rfm_scan* s, int format, const void* iq, uint64_t n, int iq_on_
     s->partial_rows = rows;
   }
   cudaEventRecord(s->ev[0], s->st);
+  // IQ correction: the statistics pass (mode 1) runs inside the spectrum's timed stage
+  s->corr_applied = rfm_iq_correction{0.f, 0.f, 1.f, 0.f, 0};
+  if (s->corr_mode == 1)
+  {
+    const int rc = rfm::IqEstimateDevice(format, d_cap, n, s->st, &s->corr_applied);
+    if (rc != RFM_OK)
+      return rc;
+  }
+  else if (s->corr_mode == 2)
+    s->corr_applied = s->corr_fixed;
+  const bool corr_on = s->corr_mode != 0;
+  const rfm::IqCorr corr = {s->corr_applied.dc_i, s->corr_applied.dc_q, s->corr_applied.a, s->corr_applied.b};
+#define RFM_SCAN_PSD_C(F, C)                                                                                            \
+  rfm::EnsureDynSmem(k_scan_psd<F, C>, kScanSmem);                                                                      \
+  k_scan_psd<F, C><<<(unsigned)rows, kScanThreads, kScanSmem, s->st>>>(                                                 \
+      reinterpret_cast<const typename ScanIn<F>::T*>(d_cap), n_seg, s->d_win, s->d_tw, s->d_partial, corr)
 #define RFM_SCAN_PSD(F)                                                                                                 \
-  rfm::EnsureDynSmem(k_scan_psd<F>, kScanSmem);                                                                         \
-  k_scan_psd<F><<<(unsigned)rows, kScanThreads, kScanSmem, s->st>>>(                                                    \
-      reinterpret_cast<const typename ScanIn<F>::T*>(d_cap), n_seg, s->d_win, s->d_tw, s->d_partial)
+  if (corr_on)                                                                                                          \
+  {                                                                                                                     \
+    RFM_SCAN_PSD_C(F, true);                                                                                            \
+  }                                                                                                                     \
+  else                                                                                                                  \
+  {                                                                                                                     \
+    RFM_SCAN_PSD_C(F, false);                                                                                           \
+  }
   switch (format)
   {
     case RFM_IQ_U8: RFM_SCAN_PSD(rfm::kIqU8); break;
@@ -567,6 +612,7 @@ int rfm_scan_run(rfm_scan* s, int format, const void* iq, uint64_t n, int iq_on_
     default: RFM_SCAN_PSD(rfm::kIqCF32); break;
   }
 #undef RFM_SCAN_PSD
+#undef RFM_SCAN_PSD_C
   k_scan_reduce<<<kScanN / kScanThreads, kScanThreads, 0, s->st>>>(s->d_partial, (unsigned)rows,
                                                                    (double)n_seg * (double)kScanN * s->sum_w2, s->d_psd);
   cudaEventRecord(s->ev[1], s->st);
@@ -612,7 +658,7 @@ int rfm_scan_run(rfm_scan* s, int format, const void* iq, uint64_t n, int iq_on_
   // 3. confirmation over every whole call of the capture
   if (!cand.empty())
   {
-    const int rc = Confirm(s, format, d_cap, n / s->n_call, cand);
+    const int rc = Confirm(s, format, d_cap, n / s->n_call, cand, corr_on ? &s->corr_applied : nullptr);
     if (rc != RFM_OK)
     {
       s->stations.clear();
@@ -653,6 +699,30 @@ int rfm_scan_stations(rfm_scan* s, rfm_scan_station* out, uint32_t max, uint32_t
     return ScanFail(RFM_ERR_OVERFLOW, "rfm_scan_stations: buffer too small");
   if (*n)
     memcpy(out, s->stations.data(), *n * sizeof(rfm_scan_station));
+  return RFM_OK;
+}
+
+int rfm_scan_set_iq_correction(rfm_scan* s, int mode, const rfm_iq_correction* fixed)
+{
+  if (!s)
+    return ScanFail(RFM_ERR_INVALID, "rfm_scan_set_iq_correction: null handle");
+  if (mode < 0 || mode > 2)
+    return ScanFail(RFM_ERR_INVALID, "rfm_scan_set_iq_correction: unknown mode (0 off, 1 estimate, 2 fixed)");
+  if (mode == 2 && !fixed)
+    return ScanFail(RFM_ERR_INVALID, "rfm_scan_set_iq_correction: mode 2 needs the fixed coefficients (NULL given)");
+  if (mode == 2 && !(isfinite(fixed->dc_i) && isfinite(fixed->dc_q) && isfinite(fixed->a) && isfinite(fixed->b)))
+    return ScanFail(RFM_ERR_INVALID, "rfm_scan_set_iq_correction: coefficients must be finite");
+  s->corr_mode = mode;
+  if (mode == 2)
+    s->corr_fixed = *fixed;
+  return RFM_OK;
+}
+
+int rfm_scan_iq_correction(rfm_scan* s, rfm_iq_correction* out)
+{
+  if (!s || !out || !s->have)
+    return ScanFail(RFM_ERR_INVALID, "rfm_scan_iq_correction: no completed run");
+  *out = s->corr_applied;
   return RFM_OK;
 }
 

@@ -17,7 +17,9 @@ Two mixers, both reference classes:
               an S x 2 M complex buffer); kept as a cross-check of the primitives' device entry points.
 
 The capture is u8 (RTL-SDR) by default; input_format = "s8" (HackRF), "s16" (the SoapySDR / UHD host format) or "cf32"
-takes the other rfm_iq_format formats, converted inside the first kernel that reads the capture.
+takes the other rfm_iq_format formats, converted inside the first kernel that reads the capture.  iq_correction (an
+IqCorrection, e.g. from estimate_iq_correction) removes a zero-IF receiver's DC offset and IQ imbalance in that same
+kernel, right after the conversion.
 """
 from __future__ import annotations
 
@@ -29,7 +31,7 @@ from . import DownConvertBatch, FmDecoderBatch, FreqShiftBatch, iq_format, iq_fo
 class WidebandReceiver:
     def __init__(self, torch, station_freqs, fs: float = 50.0e6, front_block: int = 32000, blocks_per_call: int = 64,
                  mixer: str = "osc", max_bw: float = 100000.0, device: int = 0, lanes_sms: int = 8, n_slots: int = 3,
-                 input_format="u8"):
+                 input_format="u8", iq_correction=None):
         assert mixer in ("osc", "freqshift", "freqshift_unfused")
         self.torch, self.mixer, self.fs = torch, mixer, fs
         self._fmt = iq_format(input_format)
@@ -54,6 +56,10 @@ class WidebandReceiver:
                 self.dc.set_premix(self.table.data_ptr(), front_block, front_block)
             else:
                 self.mixed = torch.empty((S, self.n_call, 2), dtype=torch.float32, device=dev)
+        # the correction goes to whichever object reads the capture: the shifter in the unfused form (the down-converter
+        # then reads mixed cf32 rows), the down-converter otherwise (the shifter only made the pre-mix table)
+        if iq_correction is not None:
+            (self.shift if mixer == "freqshift_unfused" else self.dc).set_iq_correction(iq_correction)
         self.n_bb = self.n_call >> self.dc.n_stages
         # The demodulator's lanes kernel (one warp per 32 stations, a latency chain) gets an SM partition of its own and
         # the front end runs on the demodulator's companion stream, i.e. on the OTHER SMs: sharing SMs with the
