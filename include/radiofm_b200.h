@@ -318,6 +318,20 @@ RFM_API int rfm_downconvert_process_iq_device(rfm_downconvert* d, int format, in
 /* IQ correction (rfm_iq_correction) of every input sample of every later process call, of every row, before the
  * pre-mix table and the NCO; NULL = off (the default).  Non-finite coefficients: RFM_ERR_INVALID. */
 RFM_API int rfm_downconvert_set_iq_correction(rfm_downconvert* d, const rfm_iq_correction* c);
+/* Phase-accumulator NCO pre-mixer, exact and parallel in time (DESIGN.md section 15; oracle/nco.py restates it).  In
+ * the place of the pre-mix table: after the format conversion and the IQ correction, before CRDSDownConvert's own NCO
+ * (normally at 0 Hz when this one is used).  Per row:
+ *   word    d = (uint32_t)(int64_t) llround(nco_freq / (double)in_rate * 2^32), |nco_freq| <= in_rate / 2; the sign as
+ *           for nco_freq of rfm_downconvert_create (-f brings a station at +f to 0 Hz)
+ *   phase   sample i of a call: phi = (phi_start + i d) mod 2^32; phi_start = 0 after this call and after
+ *           rfm_downconvert_reset, and advances by n d mod 2^32 with every call of n samples
+ *   phasor  e = T0[phi >> 24] T1[(phi >> 16) & 255] T2[(phi >> 8) & 255], T_m[k] = exp(j 2 pi k / 2^(8 (m + 1))) as
+ *           float(cos), float(sin) of a double angle; y = x e, every complex product the four products, one
+ *           subtraction and one addition of the reference's mixers, each rounded on its own.
+ * Error against exp(j 2 pi phi / 2^32): about -133 dBc; frequency within in_rate / 2^33.  nco_freq [rows] Hz; NULL
+ * switches it off.  RFM_ERR_INVALID for a non-finite or out-of-range frequency, or while a pre-mix table is set
+ * (rfm_downconvert_set_premix likewise refuses a table while the NCO is set). */
+RFM_API int rfm_downconvert_set_nco(rfm_downconvert* d, const double* nco_freq);
 
 /* ------------------------------------------------------------------------------------------------
  * cDownsampleFilter (DownConvert.h:21-60, DownConvert.cpp:58-256), batched over rows: Lanczos-windowed sinc FIR with
@@ -593,6 +607,11 @@ RFM_API int rfm_scan_timing(rfm_scan* s, double* spectrum_ms, double* confirm_ms
 RFM_API int rfm_scan_set_iq_correction(rfm_scan* s, int mode, const rfm_iq_correction* fixed);
 /* What the last run applied; mode 0: {0, 0, 1, 0, imbalance_valid = 0} */
 RFM_API int rfm_scan_iq_correction(rfm_scan* s, rfm_iq_correction* out);
+/* Mixer of the confirmation's rfm_downconvert rows in later runs: RFM_SCAN_MIXER_OSC (the default) sets each row's
+ * CRDSDownConvert NCO to -f_j; RFM_SCAN_MIXER_NCO creates the rows at 0 Hz and sets rfm_downconvert_set_nco(-f_j).
+ * RFM_ERR_INVALID for another value. */
+enum { RFM_SCAN_MIXER_OSC = 0, RFM_SCAN_MIXER_NCO = 1 };
+RFM_API int rfm_scan_set_mixer(rfm_scan* s, int mixer);
 
 #ifdef __cplusplus
 }

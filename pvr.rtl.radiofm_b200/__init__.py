@@ -80,6 +80,7 @@ EXPORTED_SYMBOLS = (
     "rfm_downconvert_process_iq_device", "rfm_scan_run",
     "rfm_iq_estimate", "rfm_downconvert_set_iq_correction", "rfm_freqshift_set_iq_correction",
     "rfm_scan_set_iq_correction", "rfm_scan_iq_correction",
+    "rfm_downconvert_set_nco", "rfm_scan_set_mixer",
 )
 
 # rfm_iq_format (include/radiofm_b200.h): interleaved I,Q; s8 = v * 2^-7, s16 = v * 2^-15 (exact), full scale of the container
@@ -390,6 +391,8 @@ def lib():
         L.rfm_freqshift_set_iq_correction.argtypes = [C.c_void_p, C.POINTER(RfmIqCorrection)]
         L.rfm_scan_set_iq_correction.argtypes = [C.c_void_p, C.c_int, C.POINTER(RfmIqCorrection)]
         L.rfm_scan_iq_correction.argtypes = [C.c_void_p, C.POINTER(RfmIqCorrection)]
+        L.rfm_downconvert_set_nco.argtypes = [C.c_void_p, _f64p]
+        L.rfm_scan_set_mixer.argtypes = [C.c_void_p, C.c_int]
         L.rfm_rds_check_block.restype = C.c_uint32
         L.rfm_rds_check_block.argtypes = [C.c_uint32, C.c_uint32, C.c_int, _u32p]
         _lib = L
@@ -908,6 +911,17 @@ class DownConvertBatch:
         """IQ correction of every later process call, before the pre-mix table and the NCO (None = off)."""
         _check(lib().rfm_downconvert_set_iq_correction(self._h, _corr_arg(c)))
 
+    def set_nco(self, nco_freq):
+        """Phase-accumulator NCO pre-mixer (rfm_downconvert_set_nco): one frequency per row in Hz, |f| <= in_rate / 2,
+        every phase restarted at 0; None switches it off.  Pass -f to bring a station at +f to 0 Hz."""
+        if nco_freq is None:
+            _check(lib().rfm_downconvert_set_nco(self._h, None))
+            return
+        f = np.ascontiguousarray(np.atleast_1d(nco_freq), dtype=np.float64)
+        if f.size != self.rows:
+            raise ValueError(f"{f.size} frequencies for {self.rows} rows")
+        _check(lib().rfm_downconvert_set_nco(self._h, _p(f, _f64p)))
+
     def process_cf32(self, iq: np.ndarray) -> np.ndarray:
         iq = np.ascontiguousarray(iq, dtype=np.float32).reshape(self.rows, -1, 2)
         n = iq.shape[1]
@@ -1128,18 +1142,32 @@ def scan_config(fs: float, raster_first: float, raster_step: float, raster_count
     return cfg
 
 
+SCAN_MIXERS = {"osc": 0, "nco": 1}   # rfm_scan_set_mixer: RFM_SCAN_MIXER_OSC, RFM_SCAN_MIXER_NCO
+
+
+def scan_mixer(mixer: str) -> int:
+    """The confirmation's mixer: "osc" (CRDSDownConvert's NCO_OSC at -f_j) or "nco" (rows at 0 Hz behind the phasor
+    NCO); ValueError otherwise."""
+    if not isinstance(mixer, str) or mixer not in SCAN_MIXERS:
+        raise ValueError(f"unknown scan mixer {mixer!r}: use \"osc\" or \"nco\"")
+    return SCAN_MIXERS[mixer]
+
+
 class BandScan:
     """Band scan of one wideband capture (rfm_scan_*; u8, s8, s16 or cf32): averaged spectrum, channel powers on a raster (Hz from the
     capture centre), candidates, and every candidate confirmed with the reference's receiver -- the add-on's tuner
-    auto-scan (ChannelSettings.cpp:96-147) for all channels at once."""
+    auto-scan (ChannelSettings.cpp:96-147) for all channels at once.  mixer = "nco" confirms with the phase-accumulator
+    NCO in front of rows at 0 Hz instead of CRDSDownConvert's NCO_OSC ("osc", the default)."""
 
     def __init__(self, fs: float, raster_first: float, raster_step: float, raster_count: int, min_snr_db: float = 10.0,
-                 device: int = -1, iq_correction=None):
+                 device: int = -1, iq_correction=None, mixer: str = "osc"):
+        mixer_id = scan_mixer(mixer)
         cfg = scan_config(fs, raster_first, raster_step, raster_count, min_snr_db, device)
         self.raster_count = raster_count
         self._h = C.c_void_p()
         _check(lib().rfm_scan_create(C.byref(cfg), C.byref(self._h)))
         self.set_iq_correction(iq_correction)
+        _check(lib().rfm_scan_set_mixer(self._h, mixer_id))
 
     def set_iq_correction(self, c):
         """IQ correction of later runs: None (off), "estimate" (from each run's capture) or a fixed IqCorrection."""

@@ -119,13 +119,55 @@ __device__ __forceinline__ float2 dc_mix(float2 d, float2 o)
   return r;
 }
 
-// input sample i of this call for `row`, pre-mixed if a table is set, times the NCO phasor
-template <int F, bool SHARED, bool CORR>
-__device__ __forceinline__ float2 dc_sample(const DcParams& p, const IqCorr& corr, const float2* osc, unsigned row,
-                                            unsigned i)
+// Phase-accumulator NCO pre-mixer (rfm_downconvert_set_nco; restated in oracle/nco.py).  Row r's phase at sample i of
+// a call is phi = (pos + i) d[r] mod 2^32, pos = samples since set_nco / reset mod 2^32 -- the same value as carrying
+// phi_start += n d from call to call, but every sample's phase is one integer multiply-add from its index, so time
+// chunks and their warm-up samples need no hand-over.  The phasor is the product of three 256-entry tables of
+// exp(j 2 pi k / 2^8), exp(j 2 pi k / 2^16) and exp(j 2 pi k / 2^24) (the lowest 8 phase bits are dropped), copied
+// into shared memory in front of the kernel's own buffers.
+struct DcNco
+{
+  const float2* tab;   // [3][256] T0, T1, T2
+  const unsigned* d;   // [rows] frequency words
+  unsigned pos;
+};
+constexpr unsigned kNcoTab = 3 * 256;                          // float2 entries
+constexpr unsigned kNcoSmem = kNcoTab * sizeof(float2);        // 6 KB
+
+// one row's NCO inside a CTA: the shared tables, phi_start of the call and the word
+struct NcoRow
+{
+  const float2* tab;
+  unsigned phi0, d;
+};
+
+__device__ __forceinline__ float2 nco_phasor(const NcoRow& n, unsigned i)
+{
+  const unsigned phi = n.phi0 + i * n.d;
+  const float2 t0 = n.tab[phi >> 24], t1 = n.tab[256 + ((phi >> 16) & 255u)], t2 = n.tab[512 + ((phi >> 8) & 255u)];
+  return dc_mix(dc_mix(t0, t1), t2);
+}
+
+// copy the tables into shared memory (the caller's next barrier publishes them) and set up the row
+template <unsigned THREADS>
+__device__ __forceinline__ NcoRow nco_row(const DcNco& nco, float2* s_tab, unsigned row, unsigned tid)
+{
+  for (unsigned i = tid; i < kNcoTab; i += THREADS)
+    s_tab[i] = nco.tab[i];
+  const unsigned d = nco.d[row];
+  return NcoRow{s_tab, nco.pos * d, d};
+}
+
+// input sample i of this call for `row`, pre-mixed (by the table if one is set, or by the phasor NCO), times the
+// NCO_OSC phasor
+template <int F, bool SHARED, bool CORR, bool NCO>
+__device__ __forceinline__ float2 dc_sample(const DcParams& p, const IqCorr& corr, const NcoRow& nco, const float2* osc,
+                                            unsigned row, unsigned i)
 {
   float2 d = dc_load<F, SHARED, CORR>(p, corr, row, i);
-  if (p.pre)
+  if (NCO)
+    d = dc_mix(d, nco_phasor(nco, i));
+  else if (p.pre)
     d = dc_mix(d, p.pre[(size_t)row * p.pre_stride + (p.pre_pos + i) % p.pre_period]);
   return dc_mix(d, osc[i]);
 }
@@ -273,11 +315,11 @@ __global__ void __launch_bounds__(256) k_dc_osc_fill(float2* table, size_t strid
 // --------------------------------------------------------------------------------------------------
 // generic chain: any stage kinds, interleaved V buffers (the k_rds_front scheme without the LP)
 // --------------------------------------------------------------------------------------------------
-template <int F, bool SHARED, bool CORR>
-__global__ void __launch_bounds__(kDcThreads) k_dc_chain(DcParams p, IqCorr corr)
+template <int F, bool SHARED, bool CORR, bool NCO>
+__global__ void __launch_bounds__(kDcThreads) k_dc_chain(DcParams p, IqCorr corr, DcNco nco)
 {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  float* s_h = reinterpret_cast<float*>(smem_raw);
+  float* s_h = reinterpret_cast<float*>(smem_raw + (NCO ? kNcoSmem : 0u));
   unsigned hoff[kDcMaxStages];
   unsigned acc_f = 0;
   for (unsigned k = 0; k < p.nst; ++k)
@@ -309,6 +351,9 @@ __global__ void __launch_bounds__(kDcThreads) k_dc_chain(DcParams p, IqCorr corr
   for (unsigned k = 0; k < p.nst; ++k)
     for (unsigned i = tid; i < p.st[k].hist; i += kDcThreads)
       B[k][i] = (c == 0) ? tin[p.tail_off[k] + i] : make_float2(0.f, 0.f);
+  NcoRow nrow = {};
+  if (NCO)
+    nrow = nco_row<kDcThreads>(nco, reinterpret_cast<float2*>(smem_raw), row, tid);
   __syncthreads();
   const float2* osc = p.osc + (size_t)row * p.osc_stride;
   float2* out = p.out + (size_t)row * p.out_stride;
@@ -318,7 +363,7 @@ __global__ void __launch_bounds__(kDcThreads) k_dc_chain(DcParams p, IqCorr corr
     const bool store = pos >= c_lo;
     const unsigned tn = min(kDcTileGeneric, (store ? c_hi : c_lo) - pos);
     for (unsigned i = tid; i < tn; i += kDcThreads)
-      B[0][p.st[0].hist + i] = dc_sample<F, SHARED, CORR>(p, corr, osc, row, pos + i);
+      B[0][p.st[0].hist + i] = dc_sample<F, SHARED, CORR, NCO>(p, corr, nrow, osc, row, pos + i);
     __syncthreads();
     unsigned n = tn;
     for (unsigned k = 0; k < p.nst; ++k)
@@ -392,13 +437,13 @@ __device__ __forceinline__ void dc_stage(const DcTapsPk<L>& taps, const float2* 
   }
 }
 
-template <int F, bool SHARED, int L, bool CORR>
-__global__ void __launch_bounds__(kDcThreadsFast) k_dc_chain_uniform(DcParams p, DcTapsPk<L> taps, IqCorr corr)
+template <int F, bool SHARED, int L, bool CORR, bool NCO>
+__global__ void __launch_bounds__(kDcThreadsFast) k_dc_chain_uniform(DcParams p, DcTapsPk<L> taps, IqCorr corr, DcNco nco)
 {
   constexpr int R = 5;                 // largest group: sizes the slack behind each buffer
   constexpr unsigned HH = (L - 1) / 2; // history entries in each of E and O
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  float2* vbuf = reinterpret_cast<float2*>(smem_raw);
+  float2* vbuf = reinterpret_cast<float2*>(smem_raw + (NCO ? kNcoSmem : 0u));
   // buffer offsets in closed form (every stage has the same history, the tile halves from stage to stage): arrays
   // indexed with the run-time stage number would live in local memory
   //   E(k) starts at sum_{j<k} 2 (HH + (T >> j) / 2 + R) = 2 k (HH + R) + 2 T - (T >> (k - 1)),  O(k) follows E(k)
@@ -428,6 +473,9 @@ __global__ void __launch_bounds__(kDcThreadsFast) k_dc_chain_uniform(DcParams p,
       O_(k)[e + i] = make_float2(0.f, 0.f);
     }
   }
+  NcoRow nrow = {};
+  if (NCO)
+    nrow = nco_row<kDcThreadsFast>(nco, reinterpret_cast<float2*>(smem_raw), row, tid);
   __syncthreads();
   const float2* osc = p.osc + (size_t)row * p.osc_stride;
   float2* out = p.out + (size_t)row * p.out_stride;
@@ -437,7 +485,7 @@ __global__ void __launch_bounds__(kDcThreadsFast) k_dc_chain_uniform(DcParams p,
     const bool store = pos >= c_lo;
     const unsigned tn = min(kDcTileFast, (store ? c_hi : c_lo) - pos);
     // mix; V index 2 * HH + i: even i -> E[HH + i / 2], odd i -> O[HH + i / 2]
-    if (p.pre)
+    if (!NCO && p.pre)
     {
       // the pre-mixer's table index walks with the sample: one modulo per tile and thread instead of one per sample
       const float2* pre = p.pre + (size_t)row * p.pre_stride;
@@ -453,7 +501,7 @@ __global__ void __launch_bounds__(kDcThreadsFast) k_dc_chain_uniform(DcParams p,
     }
     else
       for (unsigned i = tid; i < tn; i += kDcThreadsFast)
-        ((i & 1u) ? O_(0) : E_(0))[HH + (i >> 1)] = dc_sample<F, SHARED, CORR>(p, corr, osc, row, pos + i);
+        ((i & 1u) ? O_(0) : E_(0))[HH + (i >> 1)] = dc_sample<F, SHARED, CORR, NCO>(p, corr, nrow, osc, row, pos + i);
     __syncthreads();
     // operands of the next tile on their way into L2 while this one is filtered
     {
@@ -557,6 +605,10 @@ struct rfm_downconvert
   DcTaps<51> taps51;
   bool corr_on = false;      // rfm_downconvert_set_iq_correction
   IqCorr corr = {0.f, 0.f, 1.f, 0.f};
+  bool nco_on = false;       // rfm_downconvert_set_nco
+  unsigned* d_nco_d = nullptr;  // [rows] frequency words
+  float2* d_nco_tab = nullptr;  // [3][256] phasor tables
+  uint32_t nco_pos = 0;      // samples since set_nco / reset, mod 2^32
 };
 
 namespace
@@ -597,21 +649,22 @@ int ResetState(rfm_downconvert* d)
   return ok ? RFM_OK : DcFail(RFM_ERR_CUDA, "rfm_downconvert: state reset failed");
 }
 
-template <int F, bool SHARED, bool CORR>
-void LaunchChain(rfm_downconvert* d, const DcParams& p, cudaStream_t st)
+template <int F, bool SHARED, bool CORR, bool NCO>
+void LaunchChain(rfm_downconvert* d, const DcParams& p, const DcNco& nco, cudaStream_t st)
 {
   dim3 grid(p.nchunks, p.rows);
   if (d->uniform51)
   {
-    size_t smem = 0;
+    size_t smem = NCO ? kNcoSmem : 0;
     unsigned n = kDcTileFast;
     for (unsigned k = 0; k < p.nst; ++k)
     {
       smem += 2 * (size_t)(25 + n / 2 + 5) * sizeof(float2);
       n >>= 1;
     }
-    EnsureDynSmem(k_dc_chain_uniform<F, SHARED, 51, CORR>, smem);
-    k_dc_chain_uniform<F, SHARED, 51, CORR><<<grid, kDcThreadsFast, smem, st>>>(p, MakeDcTapsPk(d->taps51), d->corr);
+    EnsureDynSmem(k_dc_chain_uniform<F, SHARED, 51, CORR, NCO>, smem);
+    k_dc_chain_uniform<F, SHARED, 51, CORR, NCO><<<grid, kDcThreadsFast, smem, st>>>(p, MakeDcTapsPk(d->taps51), d->corr,
+                                                                                     nco);
   }
   else
   {
@@ -623,19 +676,19 @@ void LaunchChain(rfm_downconvert* d, const DcParams& p, cudaStream_t st)
       f2 += p.st[k].hist + n;
       n >>= 1;
     }
-    const size_t smem = floats * sizeof(float) + f2 * sizeof(float2);
-    EnsureDynSmem(k_dc_chain<F, SHARED, CORR>, smem);
-    k_dc_chain<F, SHARED, CORR><<<grid, kDcThreads, smem, st>>>(p, d->corr);
+    const size_t smem = (NCO ? kNcoSmem : 0) + floats * sizeof(float) + f2 * sizeof(float2);
+    EnsureDynSmem(k_dc_chain<F, SHARED, CORR, NCO>, smem);
+    k_dc_chain<F, SHARED, CORR, NCO><<<grid, kDcThreads, smem, st>>>(p, d->corr, nco);
   }
 }
 
 template <int F, bool SHARED>
-void LaunchChain(rfm_downconvert* d, const DcParams& p, cudaStream_t st)
+void LaunchChain(rfm_downconvert* d, const DcParams& p, const DcNco& nco, cudaStream_t st)
 {
   if (d->corr_on)
-    LaunchChain<F, SHARED, true>(d, p, st);
+    d->nco_on ? LaunchChain<F, SHARED, true, true>(d, p, nco, st) : LaunchChain<F, SHARED, true, false>(d, p, nco, st);
   else
-    LaunchChain<F, SHARED, false>(d, p, st);
+    d->nco_on ? LaunchChain<F, SHARED, false, true>(d, p, nco, st) : LaunchChain<F, SHARED, false, false>(d, p, nco, st);
 }
 
 // fmt: IqFormat; shared: one capture for every row (a shared cf32 capture is read as rows of stride 0)
@@ -707,12 +760,15 @@ int Run(rfm_downconvert* d, int fmt, bool shared, const void* d_in, size_t in_st
   p.pre = d->pre; p.pre_stride = d->pre_stride; p.pre_period = d->pre_period ? d->pre_period : 1; p.pre_pos = d->pre_pos;
   if (d->pre)
     d->pre_pos = (unsigned)(((uint64_t)d->pre_pos + n) % d->pre_period);
+  const DcNco nco = {d->d_nco_tab, d->d_nco_d, d->nco_pos};
+  if (d->nco_on)
+    d->nco_pos += n; // mod 2^32: phi_start of the next call is nco_pos * d, i.e. phi_start + n d mod 2^32
   switch (fmt)
   {
-    case kIqU8: shared ? LaunchChain<kIqU8, true>(d, p, st) : LaunchChain<kIqU8, false>(d, p, st); break;
-    case kIqS8: shared ? LaunchChain<kIqS8, true>(d, p, st) : LaunchChain<kIqS8, false>(d, p, st); break;
-    case kIqS16: shared ? LaunchChain<kIqS16, true>(d, p, st) : LaunchChain<kIqS16, false>(d, p, st); break;
-    default: LaunchChain<kIqCF32, false>(d, p, st); break;
+    case kIqU8: shared ? LaunchChain<kIqU8, true>(d, p, nco, st) : LaunchChain<kIqU8, false>(d, p, nco, st); break;
+    case kIqS8: shared ? LaunchChain<kIqS8, true>(d, p, nco, st) : LaunchChain<kIqS8, false>(d, p, nco, st); break;
+    case kIqS16: shared ? LaunchChain<kIqS16, true>(d, p, nco, st) : LaunchChain<kIqS16, false>(d, p, nco, st); break;
+    default: LaunchChain<kIqCF32, false>(d, p, nco, st); break;
   }
   d->tails_cur ^= 1;
   rfm::g_launches += 3;
@@ -804,6 +860,7 @@ void rfm_downconvert_destroy(rfm_downconvert* d)
   cudaFree(d->d_cos); cudaFree(d->d_sin); cudaFree(d->d_osc1); cudaFree(d->d_osc); cudaFree(d->d_cyc);
   cudaFree(d->d_tails[0]); cudaFree(d->d_tails[1]);
   cudaFree(d->d_in); cudaFree(d->d_out); cudaFree(d->d_raw);
+  cudaFree(d->d_nco_d); cudaFree(d->d_nco_tab);
   for (auto* t : d->d_taps)
     cudaFree(t);
   delete d;
@@ -853,6 +910,7 @@ int rfm_downconvert_reset(rfm_downconvert* d)
     return DcFail(RFM_ERR_INVALID, "rfm_downconvert_reset: null handle");
   cudaSetDevice(d->device);
   d->pre_pos = 0;
+  d->nco_pos = 0;
   return ResetState(d);
 }
 
@@ -860,6 +918,8 @@ int rfm_downconvert_set_premix(rfm_downconvert* d, const float* d_table, size_t 
 {
   if (!d || (d_table && (period == 0 || row_stride < period)))
     return DcFail(RFM_ERR_INVALID, "rfm_downconvert_set_premix: invalid argument");
+  if (d_table && d->nco_on)
+    return DcFail(RFM_ERR_INVALID, "rfm_downconvert_set_premix: the phasor NCO is set (one pre-mixer at a time)");
   d->pre = reinterpret_cast<const float2*>(d_table);
   d->pre_stride = row_stride;
   d->pre_period = d_table ? period : 0;
@@ -875,6 +935,52 @@ int rfm_downconvert_set_iq_correction(rfm_downconvert* d, const rfm_iq_correctio
     return DcFail(RFM_ERR_INVALID, "rfm_downconvert_set_iq_correction: coefficients must be finite");
   d->corr_on = c != nullptr;
   d->corr = c ? IqCorr{c->dc_i, c->dc_q, c->a, c->b} : IqCorr{0.f, 0.f, 1.f, 0.f};
+  return RFM_OK;
+}
+
+int rfm_downconvert_set_nco(rfm_downconvert* d, const double* nco_freq)
+{
+  if (!d)
+    return DcFail(RFM_ERR_INVALID, "rfm_downconvert_set_nco: null handle");
+  if (!nco_freq)
+  {
+    d->nco_on = false;
+    d->nco_pos = 0;
+    return RFM_OK;
+  }
+  if (d->pre)
+    return DcFail(RFM_ERR_INVALID, "rfm_downconvert_set_nco: a pre-mix table is set (one pre-mixer at a time)");
+  const double rate = (double)d->in_rate;
+  std::vector<unsigned> w(d->rows);
+  for (unsigned r = 0; r < d->rows; ++r)
+  {
+    if (!(isfinite(nco_freq[r]) && fabs(nco_freq[r]) <= rate / 2))
+      return DcFail(RFM_ERR_INVALID, "rfm_downconvert_set_nco: every frequency must be finite and within +-in_rate / 2");
+    w[r] = (uint32_t)(int64_t)llround(nco_freq[r] / rate * 4294967296.0);
+  }
+  cudaSetDevice(d->device);
+  if (!d->d_nco_tab)
+  {
+    // T0, T1, T2: exp(j 2 pi k / 2^8), exp(j 2 pi k / 2^16), exp(j 2 pi k / 2^24), double cos / sin rounded once.  No
+    // entry's double value lies within 2^-40 (relative) of a float rounding midpoint (tests/test_nco.py), so any
+    // faithfully rounded libm gives these floats.
+    std::vector<float2> t(kNcoTab);
+    const unsigned bits[3] = {8, 16, 24};
+    for (unsigned m = 0; m < 3; ++m)
+      for (unsigned k = 0; k < 256; ++k)
+      {
+        const double a = 2.0 * M_PI * k / (double)(1u << bits[m]);
+        t[m * 256 + k] = make_float2((float)cos(a), (float)sin(a));
+      }
+    if (DevAlloc(&d->d_nco_tab, kNcoTab) != cudaSuccess ||
+        cudaMemcpy(d->d_nco_tab, t.data(), kNcoSmem, cudaMemcpyHostToDevice) != cudaSuccess)
+      return DcFail(RFM_ERR_CUDA, "rfm_downconvert_set_nco: table upload failed");
+  }
+  if ((!d->d_nco_d && DevAlloc(&d->d_nco_d, d->rows) != cudaSuccess) ||
+      cudaMemcpy(d->d_nco_d, w.data(), d->rows * sizeof(unsigned), cudaMemcpyHostToDevice) != cudaSuccess)
+    return DcFail(RFM_ERR_CUDA, "rfm_downconvert_set_nco: upload of the frequency words failed");
+  d->nco_on = true;
+  d->nco_pos = 0;
   return RFM_OK;
 }
 

@@ -12,6 +12,7 @@
 //      "osc" mixer -- rfm_downconvert (CRDSDownConvert::SetFrequency(-f) + SetWfmDataRate, shared capture) feeding one
 //      rfm_decoder (cFmDecoder(rate, 0, 48000, 15000, 1)) per call of 16000 baseband samples, the front end of call
 //      k+1 overlapping the demodulator of call k; then status, RDS groups, PI and the name cRDSGroupDecoder publishes.
+//      rfm_scan_set_mixer(RFM_SCAN_MIXER_NCO) composes the "nco" receiver instead: rows at 0 Hz behind the phasor NCO.
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
@@ -237,6 +238,7 @@ struct rfm_scan
   int corr_mode = 0;                      // rfm_scan_set_iq_correction
   rfm_iq_correction corr_fixed = {0.f, 0.f, 1.f, 0.f, 0};
   rfm_iq_correction corr_applied = {0.f, 0.f, 1.f, 0.f, 0};
+  int mixer = RFM_SCAN_MIXER_OSC;         // rfm_scan_set_mixer
 };
 
 namespace
@@ -247,9 +249,15 @@ int Confirm(rfm_scan* s, int fmt, const uint8_t* d_cap, uint64_t calls, const st
             const rfm_iq_correction* corr)
 {
   const uint32_t M = (uint32_t)cand.size();
-  std::vector<float> nco(M);
+  const bool pnco = s->mixer == RFM_SCAN_MIXER_NCO;
+  std::vector<float> nco(M, 0.0f);
+  std::vector<double> pnco_freq(M);
   for (uint32_t m = 0; m < M; ++m)
-    nco[m] = (float)(-RasterFreq(s->cfg, cand[m]));
+  {
+    pnco_freq[m] = -RasterFreq(s->cfg, cand[m]);
+    if (!pnco)
+      nco[m] = (float)pnco_freq[m];
+  }
   rfm_downconvert* dc = nullptr;
   rfm_decoder* dec = nullptr;
   cudaStream_t s_dec = nullptr, s_done = nullptr;
@@ -259,6 +267,8 @@ int Confirm(rfm_scan* s, int fmt, const uint8_t* d_cap, uint64_t calls, const st
   int rc = rfm_downconvert_create(M, nco.data(), (float)s->cfg.sample_rate, kScanMaxBw, 1, s->n_call, s->device, &dc);
   if (rc == RFM_OK)
     rc = rfm_downconvert_set_iq_correction(dc, corr);
+  if (rc == RFM_OK && pnco)
+    rc = rfm_downconvert_set_nco(dc, pnco_freq.data());
   size_t stride = 0;
   void* front = nullptr;
   if (rc == RFM_OK)
@@ -715,6 +725,16 @@ int rfm_scan_set_iq_correction(rfm_scan* s, int mode, const rfm_iq_correction* f
   s->corr_mode = mode;
   if (mode == 2)
     s->corr_fixed = *fixed;
+  return RFM_OK;
+}
+
+int rfm_scan_set_mixer(rfm_scan* s, int mixer)
+{
+  if (!s)
+    return ScanFail(RFM_ERR_INVALID, "rfm_scan_set_mixer: null handle");
+  if (mixer != RFM_SCAN_MIXER_OSC && mixer != RFM_SCAN_MIXER_NCO)
+    return ScanFail(RFM_ERR_INVALID, "rfm_scan_set_mixer: unknown mixer (0 osc, 1 nco)");
+  s->mixer = mixer;
   return RFM_OK;
 }
 

@@ -15,6 +15,11 @@ Two mixers, both reference classes:
               one fused kernel per call, nothing intermediate in HBM.
   "freqshift_unfused"  the same arithmetic as separate primitive calls (64 x rfm_freqshift + one rfm_downconvert over
               an S x 2 M complex buffer); kept as a cross-check of the primitives' device entry points.
+And one mixer the project defines itself (DESIGN.md section 15):
+  "nco"       the phase-accumulator NCO (rfm_downconvert_set_nco(-f_k)) in front of CRDSDownConvert at 0 Hz: a 32-bit
+              phase per sample from its index, a phasor from three 256-entry tables (about -133 dBc).  Any frequency
+              within +-fs / 2, no phase-coherence condition, the phase continuous across calls, and the cost of the
+              freqshift table.
 
 The capture is u8 (RTL-SDR) by default; input_format = "s8" (HackRF), "s16" (the SoapySDR / UHD host format) or "cf32"
 takes the other rfm_iq_format formats, converted inside the first kernel that reads the capture.  iq_correction (an
@@ -32,7 +37,8 @@ class WidebandReceiver:
     def __init__(self, torch, station_freqs, fs: float = 50.0e6, front_block: int = 32000, blocks_per_call: int = 64,
                  mixer: str = "osc", max_bw: float = 100000.0, device: int = 0, lanes_sms: int = 8, n_slots: int = 3,
                  input_format="u8", iq_correction=None):
-        assert mixer in ("osc", "freqshift", "freqshift_unfused")
+        if mixer not in ("osc", "freqshift", "freqshift_unfused", "nco"):
+            raise ValueError(f"unknown mixer {mixer!r}: use \"osc\", \"freqshift\", \"freqshift_unfused\" or \"nco\"")
         self.torch, self.mixer, self.fs = torch, mixer, fs
         self._fmt = iq_format(input_format)
         self._esz = iq_format_bytes(self._fmt)
@@ -41,9 +47,12 @@ class WidebandReceiver:
         self.front_block, self.blocks_per_call = front_block, blocks_per_call
         self.n_call = front_block * blocks_per_call
         dev = torch.device("cuda", device)
-        if mixer == "osc":
+        if mixer in ("osc", "nco"):
             self.shift = None
-            self.dc = DownConvertBatch(-self.freqs, fs, max_bw, wfm=True, max_len=self.n_call, device=device)
+            self.dc = DownConvertBatch(-self.freqs if mixer == "osc" else np.zeros(S), fs, max_bw, wfm=True,
+                                       max_len=self.n_call, device=device)
+            if mixer == "nco":
+                self.dc.set_nco(-self.freqs)
         else:
             for f in self.freqs:
                 assert abs(f * front_block / fs - round(f * front_block / fs)) < 1e-9, "blocks must be phase-coherent"
@@ -100,7 +109,7 @@ class WidebandReceiver:
         if self.ev[slot] is not None:
             self.s_front.wait_event(self.ev[slot])            # the slot's previous call has left the demodulator
         bb, audio = self.bbs[slot], self.audios[slot]
-        if self.mixer in ("osc", "freqshift"):
+        if self.mixer in ("osc", "freqshift", "nco"):
             m = self.dc.process_iq_device(self._fmt, True, d_capture_ptr, self.n_call, bb.data_ptr(), self.n_bb,
                                           self.n_call, sf)
         else:
