@@ -47,7 +47,15 @@ typedef enum rfm_status
  *   RFM_IQ_CF32  float32 complex, taken as is
  * The s8 / s16 conversions are exact in float32: an s8 / s16 input gives bit for bit what the cf32 path gives for the
  * converted samples.  Full scale is the container's: a stream that uses fewer bits (bladeRF SC16_Q11: 12 bits in 16)
- * reads 2^(16-12) = 24 dB low; levels and the scan's dBFS values are relative to the container. */
+ * reads 2^(16-12) = 24 dB low; levels and the scan's dBFS values are relative to the container.
+ * Value domain: every code of every format and every finite float (zeros of either sign, subnormals, magnitudes up to
+ * FLT_MAX) gives the reference's outputs bit for bit.  Where the reference's arithmetic itself makes a NaN (a NaN or
+ * Inf sample, or an overflow inside the chain), the outputs are NaN-equivalent to it: NaN at the same places, every
+ * other value bit-equal (the NaN bit patterns are the device's).  The calls return RFM_OK; a NaN stays in its stream
+ * as in the reference (rfm_decoder_reset, like cFmDecoder::Reset, leaves the filters' delay lines and the de-emphasis
+ * state as they are: only a new decoder starts clean), and the band scan refuses a non-finite spectrum
+ * (rfm_scan_run).  rfm_iq_estimate on a non-finite cf32 capture returns a non-finite dc, a = 1, b = 0 and
+ * imbalance_valid = 0. */
 typedef enum rfm_iq_format { RFM_IQ_U8 = 0, RFM_IQ_S8 = 1, RFM_IQ_S16 = 2, RFM_IQ_CF32 = 3 } rfm_iq_format;
 /* bytes per complex sample: 2, 2, 4, 8; 0 for an unknown format */
 RFM_API uint32_t rfm_iq_format_bytes(int format);
@@ -112,7 +120,8 @@ typedef struct rfm_config
                             * the fractional resamplers and the rotating FIRs use fused multiply-adds (half the
                             * instructions).  Audio then differs from the reference by ~1e-4 of full scale (typical
                             * streams stay inside BASELINE.json's 1e-4; the worst of 4096 reached 1.75e-4: DESIGN.md
-                            * section 11), RDS bits normally still agree; not covered by the bit-exact parity tests. */
+                            * section 11), RDS bits normally still agree; not covered by the bit-exact parity tests.
+                            * After a NaN or Inf sample the resamplers may also place NaN up to 3 outputs early. */
 } rfm_config;
 
 RFM_API void rfm_config_default(rfm_config* cfg);
@@ -590,7 +599,10 @@ RFM_API void rfm_scan_destroy(rfm_scan* s);
 /* Whole capture of n samples of `format` (rfm_iq_format) in host memory (copied with cudaMemcpyAsync) or device memory
  * (complete before the call, aligned to the sample size: 2 / 2 / 4 / 8 bytes); n >= one call (RFM_ERR_INVALID
  * otherwise, as for an unknown format).  Blocking.  Zero candidates: no receiver is created and the scan has 0
- * stations. */
+ * stations.  A spectrum with a non-finite bin -- a NaN or Inf sample, a NaN dc from the mode-1 estimate, or a capture
+ * large enough to overflow the float32 FFT (a coherent tone from |x| of about 1e15: 32 segments of |X|^2 per sum) --
+ * has no floor and no candidates: RFM_ERR_INVALID, the bin in rfm_last_error(), before any decision; the handle keeps
+ * no result and stays usable. */
 RFM_API int rfm_scan_run(rfm_scan* s, int format, const void* iq, uint64_t n, int iq_on_device);
 /* rfm_scan_run(s, RFM_IQ_U8, iq, n, iq_on_device) */
 RFM_API int rfm_scan_run_u8(rfm_scan* s, const uint8_t* iq, uint64_t n, int iq_on_device);

@@ -6,6 +6,8 @@
     channel_powers   C_j = sum of its bins' P, in double, in bin order
     noise_floor      the sorted C at index (count - 1) // 4
     candidates       C_j >= floor * 10^(min_snr_db / 10), C_j > C_{j-1}, C_j >= C_{j+1} (where the neighbours exist)
+    check_spectrum   a spectrum with a NaN or Inf bin has no floor, no sort order and no candidates: ValueError, as
+                     rfm_scan_run returns RFM_ERR_INVALID before any decision (channel_powers and noise_floor apply it)
 
 The channel part takes the product's own float32 spectrum and evaluates the same double expressions as the product, so
 its channel powers and candidates are bit-for-bit the product's.  Only tests/ and bench scripts may import this.
@@ -60,8 +62,15 @@ def channel_bins(fs: float, first: float, step: float, count: int) -> list[np.nd
     return out
 
 
+def check_spectrum(p: np.ndarray) -> None:
+    bad = np.flatnonzero(~np.isfinite(np.asarray(p, dtype=np.float64)))
+    if bad.size:
+        raise ValueError(f"bin {int(bad[0])} of {np.asarray(p).size} is not finite: the scan makes no decision")
+
+
 def channel_powers(psd: np.ndarray, bins: list[np.ndarray]) -> np.ndarray:
     p = np.asarray(psd)
+    check_spectrum(p)
     out = np.zeros(len(bins), dtype=np.float64)
     for j, b in enumerate(bins):
         acc = 0.0
@@ -73,6 +82,7 @@ def channel_powers(psd: np.ndarray, bins: list[np.ndarray]) -> np.ndarray:
 
 def noise_floor(c: np.ndarray) -> float:
     c = np.asarray(c, dtype=np.float64)
+    check_spectrum(c)
     return float(np.sort(c)[(c.size - 1) // 4])
 
 

@@ -1480,7 +1480,8 @@ void launch_resample(const ResampleParams& p, cudaStream_t st)
 // formed once per block by k_res_taps (DownConvert.cpp:203-224, same float operations) and shared:
 //   * outputs are handled in groups of 4 consecutive ones; a group's taps are stored against a common time axis that
 //     starts at a multiple of 4 samples and is a multiple of 4 long (zero outside an output's own window: adding +-0
-//     leaves a running sum that started at +0 unchanged), 4 taps per time step as one float4;
+//     leaves a running sum that started at +0 unchanged; an output a NaN or Inf sample made non-finite is recomputed
+//     over its own window), 4 taps per time step as one float4;
 //   * k_resample_tiled: lane = stream, warp = group.  The [32 streams][span] input tiles of both channels and the
 //     groups' taps travel to shared memory with 16-byte cp.async copies (no registers, no per-element stores); rows
 //     keep a 16-byte aligned pitch of 4 * odd floats, so a lane's LDS.128 of four consecutive samples is
@@ -1617,6 +1618,14 @@ __global__ void __launch_bounds__(32 * GB) k_resample_tiled(ResampleParams p, un
   RS_STEP(k0, m.x, sv.x)
 #undef RS_STEP
   const unsigned i = 4 * (g0 + warp);
+  // The zero taps outside an output's own window add 0 * x, which is +-0 only for finite x: one NaN or Inf sample
+  // anywhere on the group's axis would make all four outputs NaN, where the reference (which reads each output's own
+  // window) makes NaN from the first output whose window holds it.  So when any of the eight sums is not finite (their
+  // sum is not: an overflow of finite sums also lands here), the outputs are recomputed over their own windows only,
+  // in the same order with the same taps, after the stores, when the accumulators are dead.  For a finite output that
+  // is exactly the sum the loop made.
+  const float sum8 = addf(addf(addf(a[0], a[1]), addf(a[2], a[3])), addf(addf(b[0], b[1]), addf(b[2], b[3])));
+  const bool redo = !isfinite(sum8);
   const bool vec = i + 4 <= p.na && ((p.lp_hist | p.lp_stride) & 3u) == 0;
   float* oM = p.lpM + (size_t)(s0 + lane) * p.lp_stride + p.lp_hist + i;
   float* oS = p.lpS + (size_t)(s0 + lane) * p.lp_stride + p.lp_hist + i;
@@ -1631,6 +1640,26 @@ __global__ void __launch_bounds__(32 * GB) k_resample_tiled(ResampleParams p, un
       oM[r] = a[r];
       oS[r] = b[r];
     }
+  if (!FUSED && redo)   // the tolerance mode (fir_fused) promises no NaN placement
+  {
+    const float* km = reinterpret_cast<const float*>(kk);
+    const float* xm = X + (size_t)lane * pitch + off;
+    const float* xs = X + (size_t)(32 + lane) * pitch + off;
+    const int vlo = s_meta[2 * warp];
+    for (unsigned r = 0; r < 4 && i + r < p.na; ++r)
+    {
+      const int pi = __float2int_rz(res_pos(p.pos_frac, p.pstep, i + r));
+      float ym = 0.0f, ys = 0.0f;
+      for (int j = 0; j <= (int)p.order; ++j)
+      {
+        const int t = (int)p.order + pi - j - vlo; // the axis position k_res_taps gave tap j of output r
+        ym = macf<FUSED>(ym, km[4 * t + r], xm[t]);
+        ys = macf<FUSED>(ys, km[4 * t + r], xs[t]);
+      }
+      oM[r] = ym;
+      oS[r] = ys;
+    }
+  }
 }
 
 template <int GB>

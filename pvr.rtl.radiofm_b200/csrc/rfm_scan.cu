@@ -637,6 +637,12 @@ int rfm_scan_run(rfm_scan* s, int format, const void* iq, uint64_t n, int iq_on_
   cudaEventElapsedTime(&ms, s->ev[0], s->ev[1]);
   s->spectrum_ms = ms;
   s->confirm_ms = 0.0;
+  // a NaN or Inf sample, a NaN dc from the estimate, or a capture large enough to overflow the float32 FFT leaves
+  // non-finite bins: no floor, candidate or sort order means anything then, so the run is refused before any decision
+  for (uint32_t k = 0; k < kScanN; ++k)
+    if (!isfinite(s->psd[k]))
+      return ScanFail(RFM_ERR_INVALID, "rfm_scan_run: spectrum bin " + std::to_string(k) + " is not finite (a NaN "
+                                       "or Inf sample, or a capture too large for the float32 FFT); no decision made");
 
   // 2. channels, floor, candidates
   const unsigned count = s->cfg.raster_count;

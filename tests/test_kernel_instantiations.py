@@ -415,7 +415,8 @@ def _as_format(u8: np.ndarray, fmt: str, seed: int = 0) -> np.ndarray:
     if fmt == "s8":
         return v.astype(np.int8)
     if fmt == "s16":
-        return (v * 256 + rng.integers(-128, 128, size=v.shape)).astype(np.int16)
+        # clipped: -128 * 256 + dither can fall below -32768, and a cast would wrap it to the other rail
+        return np.clip(v * 256 + rng.integers(-128, 128, size=v.shape), -32768, 32767).astype(np.int16)
     return (to_cf32(u8) + rng.standard_normal(u8.shape).astype(np.float32) * np.float32(1e-3)).astype(np.float32)
 
 
